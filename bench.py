@@ -7,7 +7,7 @@ curve (BASELINE config 2).  With N GPUs every rank evaluates its own 65,536-row 
 scaling, no data-path collective).  The PT-MCMC secondary metric (ensemble-iterations/s, BASELINE
 config 3) is measured in the same run and reported under "pt_mcmc".
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 Prints ONE JSON line on rank 0.
@@ -229,6 +229,8 @@ def run_ours(args, rank, world, local_rank):
     if dist:
         dist.barrier()
     step_ms = [a.elapsed_time(b) for a, b in ev]
+    # what the last timed step handed its caller, copied out after its timing has been read
+    last_out = d_out.cpu().numpy() if args.dump_outputs and rank == 0 else None
     total_ms = float(sum(step_ms))
     if dist:
         tt = torch.tensor([total_ms], dtype=torch.float64, device="cuda")
@@ -603,6 +605,13 @@ def run_ours(args, rank, world, local_rank):
             "summary": {"max_logpost": summary[0], "finite_rows": summary[1], "checksum_rank0": checksum},
         }
         print(json.dumps(line))
+        if last_out is not None:
+            # rows outside the prior come back as -inf; store which rows are finite and their values, so every
+            # stored number is finite and the class of each row is still compared
+            fin = np.isfinite(last_out)
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "finite_rows.npy"), fin.astype(np.float64))
+            np.save(os.path.join(args.dump_outputs, "logdensity.npy"), last_out[fin])
     series.close()
     if dist:
         dist.destroy_process_group()
@@ -624,7 +633,16 @@ def main():
     ap.add_argument("--scan-ny", type=int, default=1000000)
     ap.add_argument("--pt-ensembles", type=int, default=4096)
     ap.add_argument("--pt-iters", type=int, default=400)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write what the last one returned for rank 0's 65,536 rows: "
+                         "DIR/finite_rows.npy (1.0 where the log-density is finite, 0.0 where it is -inf outside the "
+                         "prior) and DIR/logdensity.npy (the finite log-densities in row order), both float64; the "
+                         "inputs are seeded, so two builds can be compared")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

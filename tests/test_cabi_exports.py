@@ -4,6 +4,8 @@ a CPU path) when asked to compute without CUDA."""
 import ctypes
 import os
 import re
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -76,15 +78,19 @@ def test_log_prior_host_helper():
 
 
 def test_no_cpu_fallback():
-    """Without a CUDA device every compute entry point must raise, not silently compute on the CPU."""
-    import carma_pack_b200 as C
-    if C._lib.device_count() > 0:
-        pytest.skip("a GPU is visible; this check is for the CPU-only container")
-    t = np.arange(10.0)
-    with pytest.raises(C.CarmaError):
-        C.Series(t, np.sin(t), np.ones(10))
-    with pytest.raises(C.CarmaError):
-        C._lib.fp64_peak_tflops(0)
+    """Without a CUDA device every compute entry point must raise, not silently compute on the CPU.  Checked in a
+    child process that is shown no device, so that the check also runs on a machine with a GPU."""
+    code = ("import numpy as np, pytest\n"
+            "import carma_pack_b200 as C\n"
+            "assert C._lib.device_count() == 0\n"
+            "t = np.arange(10.0)\n"
+            "with pytest.raises(C.CarmaError):\n"
+            "    C.Series(t, np.sin(t), np.ones(10))\n"
+            "with pytest.raises(C.CarmaError):\n"
+            "    C._lib.fp64_peak_tflops(0)\n")
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300, cwd=ROOT, env=env)
+    assert out.returncode == 0, out.stderr[-2000:]
 
 
 def test_product_never_imports_oracle():

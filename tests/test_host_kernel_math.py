@@ -12,6 +12,7 @@ import subprocess
 import numpy as np
 import pytest
 
+import build_native
 from carma_pack_b200 import synth
 from oracle import oracle as O
 from parity_util import assert_logpost_parity, ulp_shift
@@ -27,7 +28,7 @@ def _build():
     deps = [SRC] + [os.path.join(CSRC, f) for f in ("kalman_real.cuh", "fast_math.cuh", "theta_transform.cuh", "device_math.cuh")]
     if os.path.exists(LIB) and all(os.path.getmtime(LIB) >= os.path.getmtime(d) for d in deps):
         return
-    subprocess.check_call(["nvcc", "-O2", "-std=c++17", "-Xcompiler", "-fPIC", "-shared", "--expt-relaxed-constexpr",
+    subprocess.check_call([build_native.NVCC, "-O2", "-std=c++17", "-Xcompiler", "-fPIC", "-shared", "--expt-relaxed-constexpr",
                            "-Wno-deprecated-gpu-targets", "-o", LIB, SRC], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
 
 

@@ -73,16 +73,3 @@ def test_fits_binary_table_light_curve(tmp_path):
     # and it packs into the ragged batch layout next to an ASCII curve
     tt, yy, ee, off, kept = cio.pack_ragged([(t, y, e), (np.arange(5.0), np.arange(5.0), np.ones(5))])
     assert list(off) == [0, n - 4, n + 1]
-
-
-def test_reads_the_reference_kepler_file_when_present():
-    """In the build container the real file is there: 4,375 cadences of Zw 229-15 (not shipped with the repo)."""
-    import os
-    import pytest
-    path = "/root/reference/src/paper/data/kepler_zw229_Q7.fits"
-    if not os.path.exists(path):
-        pytest.skip("reference tree not available on this box")
-    cols = cio.read_fits_table(path)
-    assert len(cols) == 20 and cols["TIME"].size == 4375
-    t, y, e = cio.read_fits(path)
-    assert 4000 < t.size <= 4375 and np.all(np.diff(t) > 0) and np.all(e > 0)
