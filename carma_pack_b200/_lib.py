@@ -52,7 +52,7 @@ EXPORTED_SYMBOLS = [
     "carma_fp64_peak_tflops", "carma_philox_dev", "carma_tdist_dev", "carma_fastmath_dev",
     "carma_simulate", "carma_starting_value", "carma_comm_unique_id", "carma_comm_init_rank", "carma_comm_destroy",
     "carma_gather_summaries", "carma_gather_summaries_dev", "carma_derived_params", "carma_derived_params_dev", "carma_mle_batch_device",
-    "carma_mle_grid_device",
+    "carma_mle_grid_device", "carma_multi_series_curve_stats", "carma_multi_mle_grid_device",
 ]
 
 
@@ -86,6 +86,15 @@ class MLEJob(ctypes.Structure):   # carma_mle_job_t
 
 
 MAX_DIM = 17   # CARMA_MAX_DIM
+
+
+class CurveStats(ctypes.Structure):   # carma_curve_stats_t
+    _fields_ = [("y_mean", ctypes.c_double), ("y_var_pop", ctypes.c_double), ("y_var_sample", ctypes.c_double),
+                ("min_dt", ctypes.c_double), ("median_dt", ctypes.c_double), ("tspan", ctypes.c_double),
+                ("dt_max", ctypes.c_double), ("ny", ctypes.c_int64)]
+
+
+CURVE_STATS_DTYPE = np.dtype([(name, "f8" if ct is ctypes.c_double else "i8") for name, ct in CurveStats._fields_])
 
 
 class MLEOpts(ctypes.Structure):
@@ -144,6 +153,10 @@ def _load():
     L.carma_mle_batch_device.argtypes = L.carma_mle_batch.argtypes
     L.carma_mle_grid_device.argtypes = [_vp, ctypes.c_int, ctypes.POINTER(MLEJob), _dp, _dp, _dp, ctypes.POINTER(MLEOpts),
                                         _dp, _dp, ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_longlong), ctypes.c_int]
+    L.carma_multi_series_curve_stats.argtypes = [_vp, _vp]
+    L.carma_multi_mle_grid_device.argtypes = [_vp, ctypes.c_int, ctypes.POINTER(MLEJob), _vp, _dp, _dp, _dp,
+                                              ctypes.POINTER(MLEOpts), _dp, _dp, ctypes.POINTER(ctypes.c_int),
+                                              ctypes.POINTER(ctypes.c_longlong)]
     L.carma_multi_loglik_dev.argtypes = [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp, _vp, _vp,
                                          ctypes.c_uint, _vp]
     L.carma_multi_loglik.argtypes = [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp, _vp, _vp, ctypes.c_uint]
@@ -533,6 +546,75 @@ class MultiSeries:
         check(lib.carma_multi_pt_run(self.handle, kind, p, q, pp, ctypes.byref(o), n_ensembles, samples.ctypes.data,
                                      logposts.ctypes.data, acc.ctypes.data, xr.ctypes.data), "carma_multi_pt_run")
         return dict(samples=samples, logposts=logposts, accept_rates=acc, exchange_rates=xr)
+
+    def curve_stats(self):
+        """Per-curve statistics (structured array, CURVE_STATS_DTYPE): y_mean, y_var_pop, y_var_sample, min_dt,
+        median_dt, tspan, dt_max, ny."""
+        out = np.empty(self.ncurves, dtype=CURVE_STATS_DTYPE)
+        check(lib.carma_multi_series_curve_stats(self.handle, out.ctypes.data), "carma_multi_series_curve_stats")
+        return out
+
+    def mle_grid(self, jobs, priors=None, maxiter=1000, history=8, gtol=1e-5, ftol=2.2e-9, fd_eps=1e-8):
+        """Every model of `jobs` fitted on every curve in one launch (carma_multi_mle_grid_device), the survey twin of
+        Series.mle_grid.  jobs: sequence of (kind, p, q, x0, lower, upper, flags) with x0 (ncurves, nstart, d) and
+        lower / upper (ncurves, d); priors: ncurves entries of PRIOR_DTYPE or None (population-variance defaults).
+        Returns a list of (x (ncurves, nstart, d), f (ncurves, nstart), nit (ncurves,), nfev (ncurves,)), one per job."""
+        nj, nc = len(jobs), self.ncurves
+        cj = (MLEJob * max(nj, 1))()
+        lo = np.zeros((max(nj, 1), nc, MAX_DIM))
+        hi = np.zeros((max(nj, 1), nc, MAX_DIM))
+        xs, shapes = [], []
+        for j, (kind, p, q, x0, lower, upper, flags) in enumerate(jobs):
+            d = model_dim(kind, p, q)
+            x0 = np.ascontiguousarray(x0, dtype=np.float64)
+            if x0.ndim != 3 or x0.shape[0] != nc or x0.shape[2] != d:
+                raise ValueError("x0 of job %d must be (%d, nstart, %d)" % (j, nc, d))
+            lo[j, :, :d] = np.broadcast_to(np.asarray(lower, dtype=np.float64), (nc, d))
+            hi[j, :, :d] = np.broadcast_to(np.asarray(upper, dtype=np.float64), (nc, d))
+            cj[j].kind, cj[j].p, cj[j].q, cj[j].flags, cj[j].nstart = kind, p, q, flags, x0.shape[1]
+            xs.append(x0.reshape(-1))
+            shapes.append((x0.shape[1], d))
+        pp = None
+        if priors is not None:
+            priors = np.ascontiguousarray(priors, dtype=PRIOR_DTYPE)
+            if priors.shape != (nc,):
+                raise ValueError("priors must have %d entries" % nc)
+            pp = priors.ctypes.data
+        xin = np.ascontiguousarray(np.concatenate(xs)) if xs else np.zeros(0)
+        xout = np.empty_like(xin)
+        fout = np.empty(nc * sum(n for n, _ in shapes))
+        nit = np.zeros((max(nj, 1), nc), dtype=np.intc)
+        nfev = np.zeros((max(nj, 1), nc), dtype=np.longlong)
+        o = MLEOpts()
+        lib.carma_mle_default_opts(ctypes.byref(o))
+        o.maxiter, o.history, o.gtol, o.ftol, o.fd_eps = int(maxiter), int(history), gtol, ftol, fd_eps
+        check(lib.carma_multi_mle_grid_device(self.handle, nj, cj, pp, _ptr(xin), _ptr(lo), _ptr(hi), ctypes.byref(o),
+                                              _ptr(xout), _ptr(fout), nit.ctypes.data_as(ctypes.POINTER(ctypes.c_int)),
+                                              nfev.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong))),
+              "carma_multi_mle_grid_device")
+        res, ox, of = [], 0, 0
+        for j, (n, d) in enumerate(shapes):
+            res.append((xout[ox:ox + nc * n * d].reshape(nc, n, d).copy(), fout[of:of + nc * n].reshape(nc, n).copy(),
+                        nit[j].copy(), nfev[j].copy()))
+            ox += nc * n * d
+            of += nc * n
+        return res
+
+    def get_mle(self, p, q, ntrials=100, seed=None, maxiter=1000, curve_offset=0, priors=None):
+        """CarmaModel.get_mle for every curve: one starting-value launch, then one fitting launch over all curves x
+        starts.  Curve c's trial j is global trial (curve_offset + c) * ntrials + j, exactly as CarmaModel(curve
+        c).get_mle(..., trial_offset=(curve_offset + c) * ntrials) numbers it, so a survey split into curve blocks gives
+        the same fits.  Returns an OptimizeResult of per-curve arrays (see carma_pack.survey_get_mle)."""
+        from .carma_pack import survey_get_mle
+        return survey_get_mle(self, p, q, ntrials=ntrials, seed=seed, maxiter=maxiter, curve_offset=curve_offset,
+                              priors=priors)
+
+    def choose_order(self, pmax, qmax=None, pqlist=None, ntrials=100, seed=None, curve_offset=0):
+        """CarmaModel.choose_order for every curve, all models x curves x starts in one fitting launch.  Returns
+        (best_pq (ncurves, 2), pqlist, aicc (ncurves, nmodels), mles) (see carma_pack.survey_choose_order)."""
+        from .carma_pack import survey_choose_order
+        return survey_choose_order(self, pmax, qmax=qmax, pqlist=pqlist, ntrials=ntrials, seed=seed,
+                                   curve_offset=curve_offset)
 
     def loglik_dev(self, kind, p, q, d_priors_ptr, d_theta_ptr, d_out_ptr, flags=0, stream=0):
         check(lib.carma_multi_loglik_dev(self.handle, kind, p, q, d_priors_ptr, d_theta_ptr, d_out_ptr, flags, stream),

@@ -36,6 +36,45 @@ class OptimizeResult(dict):
     __setattr__ = dict.__setitem__
 
 
+def mle_bounds(p, q, ysigma, min_dt, tspan):
+    """Box bounds of the optimiser (carma_pack.py:218-240) from the light curve's standard deviation, shortest gap and
+    time span.  Scalars give (d,) arrays; arrays of curves give (..., d)."""
+    ysigma, min_dt, tspan = np.broadcast_arrays(*(np.asarray(v, dtype=float) for v in (ysigma, min_dt, tspan)))
+    one = np.ones_like(ysigma)
+    max_freq = 0.9 / min_dt
+    min_freq = 1.0 / tspan
+    lo = [ysigma / 10.0, 0.9 * one, -np.inf * one]
+    hi = [10.0 * ysigma, 1.1 * one, np.inf * one]
+    if p == 1:
+        lo.append(np.log(min_freq)); hi.append(np.log(max_freq))
+    else:
+        lo += [np.log(np.minimum(min_freq ** 2, 2.0 * min_freq))] * p
+        hi += [np.log(np.maximum(max_freq ** 2, 2.0 * max_freq))] * p
+        lo += [-np.inf * one] * q
+        hi += [np.inf * one] * q
+    return np.stack(lo, axis=-1), np.stack(hi, axis=-1)
+
+
+def redraw_out_of_box(x0, lower, upper, seed, trials):
+    """carma_pack.py:244-248 in place: every component of a row of x0 (n, d) that lies outside a finite bound is
+    redrawn uniformly inside the box, by the generator of the row's global trial index, default_rng([seed % 2**63,
+    trials[i]]).  lower / upper: (d,) or (n, d).  Only rows with such a component construct a generator."""
+    lower = np.broadcast_to(lower, x0.shape)
+    upper = np.broadcast_to(upper, x0.shape)
+    out = np.isfinite(lower) & ((x0 < lower) | (x0 > upper))
+    for i in np.flatnonzero(out.any(axis=1)):
+        rng = np.random.default_rng([seed % (2 ** 63), int(trials[i])])
+        for j in np.flatnonzero(out[i]):
+            x0[i, j] = rng.uniform(lower[i, j], upper[i, j])
+    return x0
+
+
+def aicc(fun, p, q, ny):
+    """AICc of a fit with -loglik `fun` on `ny` points (carma_pack.py:176-180), nparams = 2 + p + q as there (SURVEY Q11)."""
+    nparams = 2 + p + q  # sic, carma_pack.py:178
+    return 2.0 * nparams + 2.0 * fun + 2.0 * nparams * (nparams + 1.0) / (ny - nparams - 1.0)
+
+
 def batched_lbfgs(fun_batch, x0, lower, upper, maxiter=1000, m=8, gtol=1e-5, ftol=2.2e-9, fd_eps=1e-8):
     """Minimise fun over a box for every row of x0 simultaneously.
 
@@ -223,20 +262,7 @@ class CarmaModel(object):
 
     def _mle_bounds(self, p, q):
         """Box bounds of the optimiser (carma_pack.py:218-240)."""
-        ysigma = self.y.std()
-        dt = np.diff(self.time)
-        max_freq = 0.9 / dt.min()
-        min_freq = 1.0 / (self.time.max() - self.time.min())
-        lo = [ysigma / 10.0, 0.9, -np.inf]
-        hi = [10.0 * ysigma, 1.1, np.inf]
-        if p == 1:
-            lo.append(np.log(min_freq)); hi.append(np.log(max_freq))
-        else:
-            lo += [np.log(min(min_freq ** 2, 2.0 * min_freq))] * p
-            hi += [np.log(max(max_freq ** 2, 2.0 * max_freq))] * p
-            lo += [-np.inf] * q
-            hi += [np.inf] * q
-        return np.array(lo), np.array(hi)
+        return mle_bounds(p, q, self.y.std(), np.diff(self.time).min(), self.time.max() - self.time.min())
 
     def mle_starts(self, p, q, ntrials, seed, trial_offset=0, series=None):
         """The `ntrials` starting points of get_mle and everything that defines the fits: (kind, x0, lower, upper,
@@ -252,11 +278,7 @@ class CarmaModel(object):
         x0 = res["samples"][:, 0, :].copy()
         x0[:, 1] = 1.0  # carma_pack.py:216
         lo, hi = self._mle_bounds(p, q)
-        for i in range(ntrials):  # carma_pack.py:244-248, one generator per global trial index
-            rng = np.random.default_rng([seed % (2 ** 63), trial_offset + i])
-            for j in range(d):
-                if np.isfinite(lo[j]) and ((x0[i, j] < lo[j]) or (x0[i, j] > hi[j])):
-                    x0[i, j] = rng.uniform(lo[j], hi[j])
+        redraw_out_of_box(x0, lo, hi, seed, trial_offset + np.arange(ntrials))
         flags = 0 if p == 1 else IGNORE_BOUNDS  # SetMLE(True) only for p > 1 (carma_pack.py:242)
         return kind, x0, lo, hi, prior, flags
 
@@ -390,8 +412,7 @@ class CarmaModel(object):
         if verbose:
             print("p, q, AICc:")
         for MLE, (p, q) in zip(MLEs, pqlist):
-            nparams = 2 + p + q  # sic, carma_pack.py:178 (SURVEY Q11)
-            this_AICc = 2.0 * nparams + 2.0 * MLE.fun + 2.0 * nparams * (nparams + 1.0) / (self.time.size - nparams - 1.0)
+            this_AICc = aicc(MLE.fun, p, q, self.time.size)
             if verbose:
                 print(p, q, this_AICc)
             AICc.append(this_AICc)
@@ -401,6 +422,79 @@ class CarmaModel(object):
         if verbose:
             print("Model with best AICc has p =", self.p, " and q = ", self.q)
         return best_MLE, pqlist, AICc
+
+
+def _survey_starts(ms, p, q, ntrials, seed, curve_offset, priors, stats):
+    """CarmaModel.mle_starts for every curve of the multi-series `ms`: one multi-curve PT launch (ensemble of curve c,
+    trial j = global trial (curve_offset + c) * ntrials + j), measerr_scale := 1, out-of-box components redrawn.
+    Returns (kind, x0 (ncurves, ntrials, d), lower (ncurves, d), upper (ncurves, d), flags)."""
+    kind = _kind_for(p, q)
+    d = model_dim(kind, p, q)
+    nc = ms.ncurves
+    res = ms.pt_run(kind, p, q, 1, 25, ntemps=1 if p == 1 else 10, n_ensembles=ntrials, seed=seed,
+                    ensemble_offset=curve_offset * ntrials, priors=priors)
+    x0 = np.ascontiguousarray(res["samples"][:, :, 0, :])
+    x0[:, :, 1] = 1.0  # carma_pack.py:216
+    lo, hi = mle_bounds(p, q, np.sqrt(stats["y_var_pop"]), stats["min_dt"], stats["tspan"])
+    trials = (curve_offset + np.arange(nc))[:, None] * ntrials + np.arange(ntrials)[None, :]
+    redraw_out_of_box(x0.reshape(nc * ntrials, d), np.repeat(lo, ntrials, axis=0), np.repeat(hi, ntrials, axis=0), seed,
+                      trials.reshape(-1))
+    flags = 0 if p == 1 else IGNORE_BOUNDS  # SetMLE(True) only for p > 1 (carma_pack.py:242)
+    return kind, x0, lo, hi, flags
+
+
+def _survey_result(x, f, nit, nfev, x0, lo, hi):
+    best = np.argmin(f, axis=1)
+    rows = np.arange(f.shape[0])
+    fun = f[rows, best]
+    return OptimizeResult(x=x[rows, best], fun=fun, nit=nit, nfev=nfev, success=np.isfinite(fun),
+                          message="batched projected L-BFGS, best of %d starts per curve" % f.shape[1],
+                          all_x=x, all_fun=f, x0=x0, lower=lo, upper=hi)
+
+
+def _random_seed():
+    return int(np.random.SeedSequence().generate_state(1, dtype=np.uint64)[0]) % (2 ** 62)
+
+
+def survey_get_mle(ms, p, q, ntrials=100, seed=None, maxiter=1000, curve_offset=0, priors=None):
+    """CarmaModel.get_mle for every light curve of the multi-series `ms` (MultiSeries.get_mle): starting values of all
+    curves from one PT launch, then the fits of all curves x starts in one launch.  Returns an OptimizeResult of
+    per-curve arrays: x (ncurves, d) best of the starts, fun, nit, nfev, success, all_x (ncurves, ntrials, d), all_fun,
+    and the x0 / lower / upper rows the fits used."""
+    if not p > q:
+        raise ValueError("Order of AR polynomial, p, must be larger than order of MA polynomial, q.")
+    if seed is None:
+        seed = _random_seed()
+    stats = ms.curve_stats()
+    kind, x0, lo, hi, flags = _survey_starts(ms, p, q, ntrials, seed, curve_offset, priors, stats)
+    (x, f, nit, nfev), = ms.mle_grid([(kind, p, q, x0, lo, hi, flags)], priors=priors, maxiter=maxiter)
+    return _survey_result(x, f, nit, nfev, x0, lo, hi)
+
+
+def survey_choose_order(ms, pmax, qmax=None, pqlist=None, ntrials=100, seed=None, curve_offset=0):
+    """CarmaModel.choose_order for every light curve of the multi-series `ms` (MultiSeries.choose_order): the same
+    default grid and seeds (model k uses seed + k), one starting-value launch per model, then ONE launch fitting every
+    model on every curve from every start.  Per-curve AICc with the reference's formula and each curve's own ny.
+    Returns (best_pq (ncurves, 2), pqlist, aicc (ncurves, nmodels), mles) with mles[k] model k's per-curve result."""
+    if not pmax > 0:
+        raise ValueError("Order of AR polynomial must be at least 1.")
+    if qmax is None:
+        qmax = pmax - 1
+    if not pmax > qmax:
+        raise ValueError("Order of AR polynomial, p, must be larger than order of MA polynimial, q.")
+    if pqlist is None:
+        pqlist = [(p, q) for p in range(1, pmax + 1) for q in range(min(p, qmax + 1))]
+    if seed is None:
+        seed = _random_seed()
+    stats = ms.curve_stats()
+    starts = [_survey_starts(ms, p, q, ntrials, seed + k, curve_offset, None, stats) for k, (p, q) in enumerate(pqlist)]
+    fits = ms.mle_grid([(kind, p, q, x0, lo, hi, flags)
+                        for (kind, x0, lo, hi, flags), (p, q) in zip(starts, pqlist)])
+    mles = [_survey_result(x, f, nit, nfev, st[1], st[2], st[3]) for (x, f, nit, nfev), st in zip(fits, starts)]
+    table = np.stack([aicc(mle.fun, p, q, stats["ny"]) for mle, (p, q) in zip(mles, pqlist)], axis=1)
+    best = np.argmin(table, axis=1)
+    best_pq = np.asarray(pqlist, dtype=int)[best]
+    return best_pq, pqlist, table, mles
 
 
 class MCMCSample(object):

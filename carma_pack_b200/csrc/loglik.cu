@@ -975,10 +975,12 @@ int carma_multi_series_create(const double* time, const double* y, const double*
         size_t o0 = (size_t)offsets[c], o1 = (size_t)offsets[c + 1];
         if (o1 < o0 + 2) { set_error("carma_multi_series_create: every curve needs >= 2 points"); delete m; return CARMA_ERR_ARG; }
         m->max_ny = std::max(m->max_ny, (int)(o1 - o0));
+        double curve_dt_max = 0.0;
         for (size_t i = o0; i < o1; i++) {
             if (i + 1 < o1) {
                 dt[i] = time[i + 1] - time[i];
                 m->dt_max = std::max(m->dt_max, dt[i]);
+                curve_dt_max = std::max(curve_dt_max, dt[i]);
                 if (!(dt[i] > 0)) { set_error("carma_multi_series_create: times must be strictly increasing within a curve"); delete m; return CARMA_ERR_ARG; }
             }
             e2[i] = yerr[i] * yerr[i];
@@ -990,6 +992,7 @@ int carma_multi_series_create(const double* time, const double* y, const double*
         ci.prior = m->priors_pop[c];
         ci.y_mean = st.mean; ci.y_var_sample = st.var_sample; ci.y_var_pop = st.var_pop;
         ci.median_dt = st.median_dt; ci.tspan = st.tmax - st.tmin;
+        ci.min_dt = st.min_dt; ci.dt_max = curve_dt_max;
         m->info.push_back(ci);
     }
     bool ok = cuda_ok(cudaMalloc((void**)&m->d_dt, (total + 1) * sizeof(double)), "cudaMalloc(multi dt)") &&
@@ -1021,6 +1024,18 @@ int carma_multi_series_default_priors(carma_multi_series_t m, int population_var
     if (!m || !out) return CARMA_ERR_ARG;
     const std::vector<carma_prior_t>& src = population_var ? m->priors_pop : m->priors_sample;
     std::memcpy(out, src.data(), src.size() * sizeof(carma_prior_t));
+    return CARMA_OK;
+}
+
+int carma_multi_series_curve_stats(carma_multi_series_t m, carma_curve_stats_t* out) {
+    if (!m || !out) { set_error("carma_multi_series_curve_stats: null argument"); return CARMA_ERR_ARG; }
+    for (size_t c = 0; c < m->ncurves; c++) {
+        const CurveInfo& ci = m->info[c];
+        carma_curve_stats_t& o = out[c];
+        o.y_mean = ci.y_mean; o.y_var_pop = ci.y_var_pop; o.y_var_sample = ci.y_var_sample;
+        o.min_dt = ci.min_dt; o.median_dt = ci.median_dt; o.tspan = ci.tspan; o.dt_max = ci.dt_max;
+        o.ny = m->off[c + 1] - m->off[c];
+    }
     return CARMA_OK;
 }
 

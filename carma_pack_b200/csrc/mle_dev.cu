@@ -76,6 +76,22 @@ struct MleJob {           // one model: its starts are rows [first, first + nsta
 constexpr int ML_AREA = 32 * ML_D /*pts*/ + 32 /*fv*/ + 7 * ML_D /*x g xn gn pg qv dir*/ + 2 * ML_M * ML_D /*S Y*/ +
                         2 * ML_M /*rho alpha*/ + 2 * ML_D /*blocked, retry (ints, one double slot each)*/;
 
+// Multi-curve mode (carma_multi_mle_grid_device): the queue runs over (job, curve, start).  Within a job the rows
+// are curve-major in the order of `order` (curve indices, longest curve first); x0 / x_out / f_out / bounds / nit /
+// nfev keep the caller's curve order.
+struct MleCurve {         // what a fit needs of its curve beside the data: the prior and the curve's own longest gap
+    carma_prior_t prior;
+    double dt_max;
+};
+struct MleMulti {
+    const double *dt, *y, *e2;          // CSR arrays of the multi-series
+    const long long* off;               // ncurves + 1
+    const int* order;                   // ncurves: curve indices, longest first
+    const MleCurve* curve;              // ncurves
+    const unsigned long long* per_curve;   // njobs: starts per curve of each job (device job order)
+    unsigned long long ncurves;
+};
+
 // IEEE operations that the compiler may not contract into FMAs (see the header comment)
 __device__ __forceinline__ double mul(double a, double b) { return __dmul_rn(a, b); }
 __device__ __forceinline__ double add(double a, double b) { return __dadd_rn(a, b); }
@@ -383,14 +399,69 @@ __device__ __noinline__ void fit_start(const MleDevParams& mp, const MleJob& job
     }
 }
 
+__device__ __forceinline__ void fit_start_p(int p, const MleDevParams& mp, const MleJob& job, const SeriesView& sv, const MathTab& tb,
+                                            const double* sdt, const double* sy, const double* se, const double* lo,
+                                            const double* hi, double* area, int lane, const double* xs, double* xo,
+                                            double* fo, int* nit, unsigned long long* nfev) {
+    switch (p) {
+        case 1: fit_start<1>(mp, job, sv, tb, sdt, sy, se, lo, hi, area, lane, xs, xo, fo, nit, nfev); break;
+        case 2: fit_start<2>(mp, job, sv, tb, sdt, sy, se, lo, hi, area, lane, xs, xo, fo, nit, nfev); break;
+        case 3: fit_start<3>(mp, job, sv, tb, sdt, sy, se, lo, hi, area, lane, xs, xo, fo, nit, nfev); break;
+        case 4: fit_start<4>(mp, job, sv, tb, sdt, sy, se, lo, hi, area, lane, xs, xo, fo, nit, nfev); break;
+        case 5: fit_start<5>(mp, job, sv, tb, sdt, sy, se, lo, hi, area, lane, xs, xo, fo, nit, nfev); break;
+        case 6: fit_start<6>(mp, job, sv, tb, sdt, sy, se, lo, hi, area, lane, xs, xo, fo, nit, nfev); break;
+        default: fit_start<7>(mp, job, sv, tb, sdt, sy, se, lo, hi, area, lane, xs, xo, fo, nit, nfev); break;
+    }
+}
+
+// MULTI = false: one series (sv), staged once per block when it fits.  MULTI = true: every row names its curve of
+// the multi-series `mm` (sv is unused) and the fit reads the curve from global memory: staging it into the warp's own
+// shared-memory slice was measured slower (DESIGN.md, lbfgs_kernel).
+template <bool MULTI>
 __global__ void __launch_bounds__(ML_WARPS * 32, ML_BLOCKS_PER_SM) lbfgs_kernel(SeriesView sv, MleDevParams mp, const MleJob* __restrict__ jobs,
                                                               const double* __restrict__ x0, const double* __restrict__ bounds,
                                                               double* __restrict__ x_out, double* __restrict__ f_out,
                                                               int* __restrict__ nit_out, unsigned long long* __restrict__ nfev_out,
-                                                              unsigned long long* __restrict__ next_row) {
+                                                              unsigned long long* __restrict__ next_row, MleMulti mm) {
     extern __shared__ __align__(16) double smem[];
     MathTab tb;
     tb.load();
+    if constexpr (MULTI) {
+        const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+        double* area = smem + (size_t)warp * (ML_AREA + ML_LU);
+        for (;;) {
+            unsigned long long row = 0;
+            if (lane == 0) row = atomicAdd(next_row, 1ull);
+            row = __shfl_sync(0xffffffffu, row, 0);
+            if (row >= mp.total) break;
+            int j = 0;
+            while (j + 1 < mp.njobs && row >= jobs[j].first + jobs[j].nstart) j++;
+            const unsigned long long ns = mm.per_curve[j], r = row - jobs[j].first;
+            const int c = mm.order[r / ns];
+            const unsigned long long idx = (unsigned long long)c * ns + r % ns;   // the row's place in the caller's layout
+            const long long o0 = mm.off[c];
+            const int ny = (int)(mm.off[c + 1] - o0);
+            // the curve as a Series built from it would hold it: gaps to the next point, the next point's yerr^2
+            SeriesView cv;
+            cv.dt = mm.dt + o0;
+            cv.y = mm.y + o0;
+            cv.e2n = mm.e2 + o0 + 1;
+            cv.t = nullptr;
+            cv.e2_0 = mm.e2[o0];
+            cv.dt_max = mm.curve[c].dt_max;
+            cv.ny = ny;
+            cv.nyp = ny;
+            MleJob job = jobs[j];
+            job.prior = mm.curve[c].prior;
+            const unsigned long long pc = (unsigned long long)j * mm.ncurves + c;
+            const double *lo = bounds + pc * 2 * MAX_D, *hi = lo + MAX_D;
+            fit_start_p(job.p, mp, job, cv, tb, nullptr, nullptr, nullptr, lo, hi, area, lane,
+                           x0 + job.x_off + idx * job.d, x_out + job.x_off + idx * job.d, f_out + job.first + idx,
+                           nit_out + pc, nfev_out + pc);
+            __syncwarp();
+        }
+        return;
+    }
     const int nyp = mp.series_in_smem ? sv.nyp : 0;
     double *sdt = smem, *sy = smem + nyp, *se = smem + 2 * (size_t)nyp;
     if (mp.series_in_smem) {
@@ -430,23 +501,42 @@ __global__ void __launch_bounds__(ML_WARPS * 32, ML_BLOCKS_PER_SM) lbfgs_kernel(
     }
 }
 
+template <bool MULTI>
 cudaError_t lbfgs_attrs() {
     static OncePerDevice once;
-    return once.run([] { return cudaFuncSetAttribute(lbfgs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ML_SMEM_MAX); });
+    return once.run([] { return cudaFuncSetAttribute(lbfgs_kernel<MULTI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ML_SMEM_MAX); });
 }
 
+// smem: dynamic shared memory of a block, bytes
+template <bool MULTI>
 cudaError_t launch_lbfgs(const SeriesView& sv, const MleDevParams& mp, const MleJob* jobs, const double* x0, const double* bounds,
                          double* x_out, double* f_out, int* nit, unsigned long long* nfev, unsigned long long* next_row,
-                         cudaStream_t st) {
-    const size_t smem = ((mp.series_in_smem ? 3 * (size_t)sv.nyp : 0) + (size_t)ML_WARPS * (ML_AREA + ML_LU)) * sizeof(double);
-    const cudaError_t attr_err = lbfgs_attrs();
+                         const MleMulti& mm, size_t smem, cudaStream_t st) {
+    const cudaError_t attr_err = lbfgs_attrs<MULTI>();
     if (attr_err != cudaSuccess) return attr_err;
     int nsm = 148, dev = 0;
     if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
     const size_t want = ((size_t)mp.total + ML_WARPS - 1) / ML_WARPS, cap = (size_t)nsm * ML_BLOCKS_PER_SM;
     const unsigned grid = (unsigned)std::min(want, cap);
-    lbfgs_kernel<<<grid, ML_WARPS * 32, smem, st>>>(sv, mp, jobs, x0, bounds, x_out, f_out, nit, nfev, next_row);
+    lbfgs_kernel<MULTI><<<grid, ML_WARPS * 32, smem, st>>>(sv, mp, jobs, x0, bounds, x_out, f_out, nit, nfev, next_row, mm);
     return cudaGetLastError();
+}
+
+// heaviest job first (the long fits start first); stable, so equal weights keep the caller's order
+std::vector<int> jobs_heaviest_first(int njobs, const carma_mle_job_t* jobs) {
+    std::vector<int> order(njobs);
+    for (int j = 0; j < njobs; j++) order[j] = j;
+    auto weight = [&](int j) {
+        const int d = model_dim(jobs[j].kind, jobs[j].p, jobs[j].q);
+        return (double)jobs[j].p * jobs[j].p * (d + 1);
+    };
+    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return weight(a) > weight(b); });
+    return order;
+}
+
+bool valid_job(const carma_mle_job_t& jb) {
+    return !(jb.kind < CARMA_KIND_CAR1 || jb.kind > CARMA_KIND_ZCARMA || jb.p < 1 || jb.p > MAX_P ||
+             (jb.kind == CARMA_KIND_CAR1 && jb.p != 1) || (jb.kind == CARMA_KIND_CARMA && !(jb.q >= 0 && jb.q < jb.p)));
 }
 
 }  // namespace
@@ -467,16 +557,12 @@ extern "C" int carma_mle_grid_device(carma_series_t s, int njobs, const carma_ml
         set_error("carma_mle_grid_device: invalid options (1 <= history <= 8)");
         return CARMA_ERR_ARG;
     }
-    // the queue serves the jobs in the order given here: heaviest first, so that the long fits start first
-    std::vector<int> order(njobs);
-    for (int j = 0; j < njobs; j++) order[j] = j;
     std::vector<MleJob> dj(njobs);
     std::vector<size_t> f_first(njobs), x_first(njobs);
     size_t total = 0, xdoubles = 0;
     for (int j = 0; j < njobs; j++) {
         const carma_mle_job_t& jb = jobs[j];
-        if (jb.kind < CARMA_KIND_CAR1 || jb.kind > CARMA_KIND_ZCARMA || jb.p < 1 || jb.p > MAX_P ||
-            (jb.kind == CARMA_KIND_CAR1 && jb.p != 1) || (jb.kind == CARMA_KIND_CARMA && !(jb.q >= 0 && jb.q < jb.p))) {
+        if (!valid_job(jb)) {
             set_error("carma_mle_grid_device: invalid (kind,p,q) in job " + std::to_string(j));
             return CARMA_ERR_ARG;
         }
@@ -490,11 +576,8 @@ extern "C" int carma_mle_grid_device(carma_series_t s, int njobs, const carma_ml
         if (nfev_out) nfev_out[j] = 0;
     }
     if (total == 0) return CARMA_OK;
-    auto weight = [&](int j) {
-        const int d = model_dim(jobs[j].kind, jobs[j].p, jobs[j].q);
-        return (double)jobs[j].p * jobs[j].p * (d + 1);
-    };
-    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return weight(a) > weight(b); });
+    // the queue serves the jobs in this order
+    const std::vector<int> order = jobs_heaviest_first(njobs, jobs);
     // device order: rows of job order[k] follow those of order[k-1] in the queue, in x and in f
     std::vector<double> hx(xdoubles), hb((size_t)njobs * 2 * MAX_D, 0.0);
     size_t qrow = 0, qx = 0;
@@ -542,7 +625,9 @@ extern "C" int carma_mle_grid_device(carma_series_t s, int njobs, const carma_ml
     mp.njobs = njobs;
     mp.total = total;
     mp.series_in_smem = ((3 * (size_t)sv.nyp + (size_t)ML_WARPS * (ML_AREA + ML_LU)) * sizeof(double) <= ML_SMEM_MAX) ? 1 : 0;
-    if (!cuda_ok(launch_lbfgs(sv, mp, d_jobs, din, d_b, dout, d_f, d_nit, d_nfev, d_next, st), "lbfgs_kernel launch")) return CARMA_ERR_CUDA;
+    const size_t smem = ((mp.series_in_smem ? 3 * (size_t)sv.nyp : 0) + (size_t)ML_WARPS * (ML_AREA + ML_LU)) * sizeof(double);
+    if (!cuda_ok(launch_lbfgs<false>(sv, mp, d_jobs, din, d_b, dout, d_f, d_nit, d_nfev, d_next, MleMulti{}, smem, st), "lbfgs_kernel launch"))
+        return CARMA_ERR_CUDA;
     std::vector<double> rx(xdoubles), rf(total);
     std::vector<int> rnit(njobs);
     std::vector<unsigned long long> rnfev(njobs);
@@ -585,4 +670,132 @@ extern "C" int carma_mle_batch_device(carma_series_t s, int kind, int p, int q, 
     std::copy(lower, lower + d, lo);
     std::copy(upper, upper + d, hi);
     return carma_mle_grid_device(s, 1, &jb, x0, lo, hi, opts, x_out, f_out, nit_out, nfev_out, slot);
+}
+
+extern "C" int carma_multi_mle_grid_device(carma_multi_series_t m, int njobs, const carma_mle_job_t* jobs,
+                                           const carma_prior_t* priors, const double* x0, const double* lower,
+                                           const double* upper, const carma_mle_opts_t* opts, double* x_out,
+                                           double* f_out, int* nit_out, long long* nfev_out) {
+    if (!m || njobs < 0 || (njobs > 0 && (!jobs || !x0 || !lower || !upper || !x_out || !f_out))) {
+        set_error("carma_multi_mle_grid_device: bad argument");
+        return CARMA_ERR_ARG;
+    }
+    carma_mle_opts_t o;
+    if (opts) o = *opts; else carma_mle_default_opts(&o);
+    if (o.maxiter < 0 || o.history < 1 || o.history > ML_M || o.max_backtrack < 1 || !(o.fd_eps > 0)) {
+        set_error("carma_multi_mle_grid_device: invalid options (1 <= history <= 8)");
+        return CARMA_ERR_ARG;
+    }
+    const size_t nc = m->ncurves;
+    std::vector<size_t> f_first(njobs), x_first(njobs);
+    size_t total = 0, xdoubles = 0;
+    for (int j = 0; j < njobs; j++) {
+        if (!valid_job(jobs[j])) {
+            set_error("carma_multi_mle_grid_device: invalid (kind,p,q) in job " + std::to_string(j));
+            return CARMA_ERR_ARG;
+        }
+        f_first[j] = total;
+        x_first[j] = xdoubles;
+        total += nc * jobs[j].nstart;
+        xdoubles += nc * jobs[j].nstart * (size_t)model_dim(jobs[j].kind, jobs[j].p, jobs[j].q);
+    }
+    for (size_t k = 0; k < (size_t)njobs * nc; k++) {
+        if (nit_out) nit_out[k] = 0;
+        if (nfev_out) nfev_out[k] = 0;
+    }
+    if (total == 0) return CARMA_OK;
+    const std::vector<int> order = jobs_heaviest_first(njobs, jobs);
+    // within a job the longest curves first: a fit's latency scales with ny and the launch lasts as long as its slowest fit
+    std::vector<int> corder(nc);
+    for (size_t c = 0; c < nc; c++) corder[c] = (int)c;
+    std::stable_sort(corder.begin(), corder.end(), [&](int a, int b) { return m->off[a + 1] - m->off[a] > m->off[b + 1] - m->off[b]; });
+    std::vector<MleCurve> hc(nc);
+    for (size_t c = 0; c < nc; c++) {
+        hc[c].prior = priors ? priors[c] : m->info[c].prior;
+        hc[c].dt_max = m->info[c].dt_max;
+    }
+    // device job order; per job the rows keep the caller's (curve-major) layout, bounds are (job, curve) rows
+    std::vector<MleJob> dj(njobs);
+    std::vector<unsigned long long> per_curve(njobs);
+    std::vector<double> hx(xdoubles), hb((size_t)njobs * nc * 2 * MAX_D, 0.0);
+    size_t qrow = 0, qx = 0;
+    for (int k = 0; k < njobs; k++) {
+        const int j = order[k];
+        const carma_mle_job_t& jb = jobs[j];
+        const int d = model_dim(jb.kind, jb.p, jb.q);
+        MleJob& mj = dj[k];
+        mj.kind = jb.kind; mj.p = jb.p; mj.q = jb.q; mj.d = d; mj.flags = jb.flags; mj.prior = jb.prior;
+        mj.first = qrow; mj.nstart = nc * jb.nstart; mj.x_off = qx;
+        per_curve[k] = jb.nstart;
+        std::copy(x0 + x_first[j], x0 + x_first[j] + nc * jb.nstart * d, hx.begin() + qx);
+        for (size_t c = 0; c < nc; c++) {
+            const double* lo = lower + ((size_t)j * nc + c) * CARMA_MAX_DIM;
+            const double* hi = upper + ((size_t)j * nc + c) * CARMA_MAX_DIM;
+            double* b = hb.data() + ((size_t)k * nc + c) * 2 * MAX_D;
+            std::copy(lo, lo + d, b);
+            std::copy(hi, hi + d, b + MAX_D);
+        }
+        qrow += nc * jb.nstart;
+        qx += nc * jb.nstart * d;
+    }
+    if (!cuda_ok(cudaSetDevice(m->device), "cudaSetDevice")) return CARMA_ERR_CUDA;
+    // scratch_in: [ x0 | bounds | jobs | per_curve | curves | order ]   scratch_out: [ x | f | nfev | queue head | nit ]
+    const size_t nb = (size_t)njobs * nc;
+    const size_t in_bytes = (xdoubles + hb.size()) * sizeof(double) + (size_t)njobs * (sizeof(MleJob) + sizeof(unsigned long long)) +
+                            nc * (sizeof(MleCurve) + sizeof(int));
+    const size_t out_bytes = (xdoubles + total + nb + 1) * sizeof(double) + nb * sizeof(int);
+    if (!m->scratch_in.reserve(in_bytes) || !m->scratch_out.reserve(out_bytes)) return CARMA_ERR_CUDA;
+    double* din = (double*)m->scratch_in.p;
+    double* d_b = din + xdoubles;
+    MleJob* d_jobs = (MleJob*)(d_b + hb.size());
+    unsigned long long* d_pc = (unsigned long long*)(d_jobs + njobs);
+    MleCurve* d_curve = (MleCurve*)(d_pc + njobs);
+    int* d_order = (int*)(d_curve + nc);
+    double* dout = (double*)m->scratch_out.p;
+    double* d_f = dout + xdoubles;
+    unsigned long long* d_nfev = (unsigned long long*)(d_f + total);
+    unsigned long long* d_next = d_nfev + nb;
+    int* d_nit = (int*)(d_next + 1);
+    cudaStream_t st = 0;
+    if (!cuda_ok(cudaMemcpyAsync(din, hx.data(), xdoubles * sizeof(double), cudaMemcpyHostToDevice, st), "H2D x0") ||
+        !cuda_ok(cudaMemcpyAsync(d_b, hb.data(), hb.size() * sizeof(double), cudaMemcpyHostToDevice, st), "H2D bounds") ||
+        !cuda_ok(cudaMemcpyAsync(d_jobs, dj.data(), njobs * sizeof(MleJob), cudaMemcpyHostToDevice, st), "H2D jobs") ||
+        !cuda_ok(cudaMemcpyAsync(d_pc, per_curve.data(), njobs * sizeof(unsigned long long), cudaMemcpyHostToDevice, st), "H2D per_curve") ||
+        !cuda_ok(cudaMemcpyAsync(d_curve, hc.data(), nc * sizeof(MleCurve), cudaMemcpyHostToDevice, st), "H2D curves") ||
+        !cuda_ok(cudaMemcpyAsync(d_order, corder.data(), nc * sizeof(int), cudaMemcpyHostToDevice, st), "H2D curve order") ||
+        !cuda_ok(cudaMemsetAsync(d_nfev, 0, (nb + 1) * sizeof(double) + nb * sizeof(int), st), "memset counters"))
+        return CARMA_ERR_CUDA;
+    MleDevParams mp{};
+    mp.maxiter = o.maxiter; mp.history = o.history; mp.max_backtrack = o.max_backtrack;
+    mp.gtol = o.gtol; mp.ftol = o.ftol; mp.fd_eps = o.fd_eps;
+    mp.series_in_smem = 0;
+    mp.njobs = njobs;
+    mp.total = total;
+    MleMulti mm{};
+    mm.dt = m->d_dt; mm.y = m->d_y; mm.e2 = m->d_e2; mm.off = m->d_off;
+    mm.order = d_order; mm.curve = d_curve; mm.per_curve = d_pc; mm.ncurves = nc;
+    const size_t smem = (size_t)ML_WARPS * (ML_AREA + ML_LU) * sizeof(double);
+    if (!cuda_ok(launch_lbfgs<true>(SeriesView{}, mp, d_jobs, din, d_b, dout, d_f, d_nit, d_nfev, d_next, mm, smem, st),
+                 "lbfgs_kernel launch"))
+        return CARMA_ERR_CUDA;
+    std::vector<double> rx(xdoubles), rf(total);
+    std::vector<int> rnit(nb);
+    std::vector<unsigned long long> rnfev(nb);
+    if (!cuda_ok(cudaMemcpyAsync(rx.data(), dout, xdoubles * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H x") ||
+        !cuda_ok(cudaMemcpyAsync(rf.data(), d_f, total * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H f") ||
+        !cuda_ok(cudaMemcpyAsync(rnit.data(), d_nit, nb * sizeof(int), cudaMemcpyDeviceToHost, st), "D2H nit") ||
+        !cuda_ok(cudaMemcpyAsync(rnfev.data(), d_nfev, nb * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st), "D2H nfev") ||
+        !cuda_ok(cudaStreamSynchronize(st), "multi mle sync"))
+        return CARMA_ERR_CUDA;
+    for (int k = 0; k < njobs; k++) {
+        const int j = order[k];
+        const MleJob& mj = dj[k];
+        std::copy(rx.begin() + mj.x_off, rx.begin() + mj.x_off + mj.nstart * mj.d, x_out + x_first[j]);
+        std::copy(rf.begin() + mj.first, rf.begin() + mj.first + mj.nstart, f_out + f_first[j]);
+        for (size_t c = 0; c < nc; c++) {
+            if (nit_out) nit_out[(size_t)j * nc + c] = rnit[(size_t)k * nc + c];
+            if (nfev_out) nfev_out[(size_t)j * nc + c] = (long long)rnfev[(size_t)k * nc + c];
+        }
+    }
+    return CARMA_OK;
 }

@@ -82,6 +82,7 @@ namespace carma {
 struct CurveInfo {
     carma_prior_t prior;
     double y_mean, y_var_sample, y_var_pop, median_dt, tspan;
+    double min_dt, dt_max;   // shortest and longest gap of the curve (the optimiser's box, its rate clamp)
 };
 }  // namespace carma
 

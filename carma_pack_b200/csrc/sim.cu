@@ -48,7 +48,7 @@ simulate_kernel(size_t ncurves, int ny, int kind, int q, int d, const double* __
     double* py = y_out + c * (size_t)ny;
     double* pe = e2_out + c * (size_t)ny;
     const double e2 = yerr * yerr;
-    double sum = 0.0, sumsq = 0.0, tspan = 0.0, dmin = 1e300;
+    double sum = 0.0, sumsq = 0.0, tspan = 0.0, dmin = 1e300, dmax = 0.0;
     for (int i = 0; i < ny; i++) {
         double u0, u1, u2, u3;
         uniforms2(seed, chain, STREAM_SIMULATE, (uint32_t)i, 0u, &u0, &u1);
@@ -68,6 +68,7 @@ simulate_kernel(size_t ncurves, int ny, int kind, int q, int d, const double* __
             pdt[i] = dt;
             tspan += dt;
             dmin = fmin(dmin, dt);
+            dmax = fmax(dmax, dt);
             const double inv = kf.var > 0.0 ? 1.0 / kf.var : 0.0;
             kf.measurement_update(innov, inv);
             kf.template predict_observe<false>(prm, tb, dt, 0.0);
@@ -102,6 +103,8 @@ simulate_kernel(size_t ncurves, int ny, int kind, int q, int d, const double* __
     ci.y_var_sample = ny > 1 ? ci.y_var_pop * (double)ny / (double)(ny - 1) : 0.0;
     ci.median_dt = med_lo;
     ci.tspan = tspan;
+    ci.min_dt = dmin;
+    ci.dt_max = dmax;
     ci.prior.max_stdev = 10.0 * sqrt(fmax(ci.y_var_pop, 0.0));
     ci.prior.max_freq = 1.0 / dmin;
     ci.prior.min_freq = 1.0 / tspan;

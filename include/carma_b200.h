@@ -186,6 +186,19 @@ int carma_mle_grid_device(carma_series_t s, int njobs, const carma_mle_job_t* jo
                           const double* lower, const double* upper, const carma_mle_opts_t* opts, double* x_out,
                           double* f_out, int* nit_out, long long* nfev_out, int slot);
 
+/* carma_mle_grid_device over every curve of a multi-series, in ONE launch (survey-scale get_mle / choose_order): job j
+ * fits jobs[j].nstart starts PER CURVE.  jobs[j].prior is ignored; the per-curve priors come from `priors` (ncurves
+ * entries, or NULL = the population-variance defaults).  Per job, curve-major: x0 / x_out ncurves*nstart_j rows of d_j
+ * doubles, f_out ncurves*nstart_j values, lower / upper ncurves rows of CARMA_MAX_DIM doubles; the jobs one after the
+ * other.  nit_out / nfev_out: njobs*ncurves entries (largest iteration count / total evaluations of that curve's starts;
+ * may be NULL).  A fit reads its curve as a carma_series_t built from that curve would hold it (its own longest gap
+ * included), so a start's result depends only on (job, curve, x0 row, bounds row, prior): it equals what
+ * carma_mle_batch_device returns for that curve alone.  Blocking; uses the multi-series' own scratch buffers. */
+int carma_multi_mle_grid_device(carma_multi_series_t m, int njobs, const carma_mle_job_t* jobs,
+                                const carma_prior_t* priors, const double* x0, const double* lower,
+                                const double* upper, const carma_mle_opts_t* opts, double* x_out,
+                                double* f_out, int* nit_out, long long* nfev_out);
+
 /* ---- multi light-curve batch (one theta per curve) ----------------------------------------
  * The reference loops over objects in Python; this is the survey-scale form of the same
  * LogDensity call.  offsets: ncurves+1 (CSR), host pointers. priors: ncurves or NULL (defaults). */
@@ -206,6 +219,13 @@ int carma_multi_series_simulate(size_t ncurves, size_t ny, int kind, int p, int 
 /* Copy curve `curve` back to the host (time measured from 0). capacity: length of the three arrays. */
 int carma_multi_series_get_curve(carma_multi_series_t m, size_t curve, double* time, double* y, double* yerr,
                                  size_t capacity, size_t* ny_out);
+/* Per-curve statistics of a multi-series (what the optimiser's box and the default priors are built from): mean and
+ * population / N-1 variance of y, shortest, median and longest sampling gap, time span, number of points. */
+typedef struct carma_curve_stats {
+    double y_mean, y_var_pop, y_var_sample, min_dt, median_dt, tspan, dt_max;
+    int64_t ny;
+} carma_curve_stats_t;
+int carma_multi_series_curve_stats(carma_multi_series_t m, carma_curve_stats_t* out /* ncurves */);
 int carma_multi_loglik_dev(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* d_priors,
                            const double* d_theta /* ncurves x d */, double* d_logpost, unsigned flags, void* stream);
 int carma_multi_loglik(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* priors,
