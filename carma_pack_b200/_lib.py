@@ -53,6 +53,7 @@ EXPORTED_SYMBOLS = [
     "carma_simulate", "carma_starting_value", "carma_comm_unique_id", "carma_comm_init_rank", "carma_comm_destroy",
     "carma_gather_summaries", "carma_gather_summaries_dev", "carma_derived_params", "carma_derived_params_dev", "carma_mle_batch_device",
     "carma_mle_grid_device", "carma_multi_series_curve_stats", "carma_multi_mle_grid_device",
+    "carma_multi_filter_dev", "carma_multi_filter", "carma_multi_assess_fit", "carma_multi_predict",
 ]
 
 
@@ -160,6 +161,13 @@ def _load():
     L.carma_multi_loglik_dev.argtypes = [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp, _vp, _vp,
                                          ctypes.c_uint, _vp]
     L.carma_multi_loglik.argtypes = [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp, _vp, _vp, ctypes.c_uint]
+    L.carma_multi_filter_dev.argtypes = [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp, _vp, ctypes.c_uint, _vp, _vp,
+                                         _vp, _vp]
+    L.carma_multi_filter.argtypes = [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp, _vp, ctypes.c_uint, _vp, _vp, _vp]
+    L.carma_multi_assess_fit.argtypes = [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp, _vp, ctypes.c_uint,
+                                         ctypes.c_int, _vp]
+    L.carma_multi_predict.argtypes = [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp, _vp, ctypes.c_uint, _vp, _vp,
+                                      _vp, _vp]
     L.carma_filter.argtypes = [_vp, ctypes.c_double, _dp, _dp, ctypes.c_int, ctypes.c_double, ctypes.c_double, _dp, _dp]
     L.carma_predict.argtypes = [_vp, ctypes.c_double, _dp, _dp, ctypes.c_int, ctypes.c_double, ctypes.c_double,
                                 _dp, _sz, _dp, _dp]
@@ -619,6 +627,75 @@ class MultiSeries:
     def loglik_dev(self, kind, p, q, d_priors_ptr, d_theta_ptr, d_out_ptr, flags=0, stream=0):
         check(lib.carma_multi_loglik_dev(self.handle, kind, p, q, d_priors_ptr, d_theta_ptr, d_out_ptr, flags, stream),
               "carma_multi_loglik_dev")
+
+    def _rows(self, kind, p, q, theta, priors):
+        """theta (ncurves, d) and priors (ncurves entries or None) as contiguous arrays for the survey calls."""
+        th = np.ascontiguousarray(theta, dtype=np.float64)
+        d = model_dim(kind, p, q)
+        if th.shape != (self.ncurves, d):
+            raise ValueError("theta must be (%d, %d)" % (self.ncurves, d))
+        if priors is not None:
+            priors = np.ascontiguousarray(priors, dtype=PRIOR_DTYPE)
+            if priors.shape != (self.ncurves,):
+                raise ValueError("priors must have %d entries" % self.ncurves)
+        return th, priors
+
+    @staticmethod
+    def _default_flags(p, flags):
+        # the rule the survey fits use: SetMLE(True) only for p > 1 (carma_pack.py:242)
+        return (0 if p == 1 else IGNORE_BOUNDS) if flags is None else flags
+
+    def kalman_filter(self, kind, p, q, theta, priors=None, flags=None):
+        """One-step predictive mean and variance of every point of every curve, one theta row per curve
+        (carma_multi_filter, the survey form of CarmaSample.kalman_filter).  Returns (mean + mu, var, loglik): mean and
+        var flat in the CSR order of the curves, loglik per curve (bitwise MultiSeries.loglik with the same arguments).
+        flags: None = the survey fits' rule (0 for p == 1, else IGNORE_BOUNDS)."""
+        th, priors = self._rows(kind, p, q, theta, priors)
+        flags = self._default_flags(p, flags)
+        total = int(self.offsets[-1])
+        mean, var, ll = np.empty(total), np.empty(total), np.empty(self.ncurves)
+        check(lib.carma_multi_filter(self.handle, kind, p, q, None if priors is None else priors.ctypes.data, th.ctypes.data,
+                                     flags, mean.ctypes.data, var.ctypes.data, ll.ctypes.data), "carma_multi_filter")
+        mean += np.repeat(th[:, 2], np.diff(self.offsets))
+        return mean, var, ll
+
+    def filter_dev(self, kind, p, q, d_priors_ptr, d_theta_ptr, d_mean_ptr, d_var_ptr, d_loglik_ptr=None, flags=None,
+                   stream=0):
+        """Device-resident kalman_filter (carma_multi_filter_dev): raw device pointers, mean without mu, no sync."""
+        check(lib.carma_multi_filter_dev(self.handle, kind, p, q, d_priors_ptr, d_theta_ptr, self._default_flags(p, flags),
+                                         d_mean_ptr, d_var_ptr, d_loglik_ptr, stream), "carma_multi_filter_dev")
+
+    def assess_fit_values(self, kind, p, q, theta, nlags=20, priors=None, flags=None):
+        """CarmaSample.assess_fit_values for every curve (carma_multi_assess_fit): moments and autocorrelation of the
+        standardised one-step residuals, computed on the device.  Returns an OptimizeResult-style dict of per-curve arrays:
+        loglik, resid_mean, resid_std, acf (ncurves, nlags), acf_sq (ncurves, nlags) -- lags 1..nlags -- and
+        bound = 1.96 / sqrt(ny), the band a white residual stays in."""
+        from .carma_pack import OptimizeResult
+        th, priors = self._rows(kind, p, q, theta, priors)
+        nlags = int(nlags)
+        out = np.empty((self.ncurves, 3 + 2 * max(nlags, 0)))
+        check(lib.carma_multi_assess_fit(self.handle, kind, p, q, None if priors is None else priors.ctypes.data,
+                                         th.ctypes.data, self._default_flags(p, flags), nlags, out.ctypes.data),
+              "carma_multi_assess_fit")
+        return OptimizeResult(loglik=out[:, 0].copy(), resid_mean=out[:, 1].copy(), resid_std=out[:, 2].copy(),
+                              acf=out[:, 3:3 + nlags].copy(), acf_sq=out[:, 3 + nlags:].copy(),
+                              bound=1.96 / np.sqrt(np.diff(self.offsets).astype(np.float64)))
+
+    def predict(self, kind, p, q, theta, tq, q_offsets, priors=None, flags=None):
+        """Expected value and variance of every curve at its own query times given its data (carma_multi_predict, the
+        survey form of CarmaSample.predict).  tq: absolute times, curve c's at tq[q_offsets[c]:q_offsets[c+1]], any
+        order.  Returns (qmean + mu, qvar) in the order of tq."""
+        th, priors = self._rows(kind, p, q, theta, priors)
+        t = _c(np.atleast_1d(tq))
+        qo = np.ascontiguousarray(q_offsets, dtype=np.int64)
+        if qo.shape != (self.ncurves + 1,) or qo[-1] != t.size:
+            raise ValueError("q_offsets must have %d entries and end at len(tq) = %d" % (self.ncurves + 1, t.size))
+        qm, qv = np.empty(t.size), np.empty(t.size)
+        check(lib.carma_multi_predict(self.handle, kind, p, q, None if priors is None else priors.ctypes.data, th.ctypes.data,
+                                      self._default_flags(p, flags), qo.ctypes.data, t.ctypes.data, qm.ctypes.data,
+                                      qv.ctypes.data), "carma_multi_predict")
+        qm += np.repeat(th[:, 2], np.diff(qo))
+        return qm, qv
 
 
 def lbfgs_batch(fun_batch, x0, lower, upper, maxiter=1000, history=8, gtol=1e-5, ftol=2.2e-9, fd_eps=1e-8):

@@ -455,6 +455,68 @@ __device__ void filter_span_blocks_any(KalmanReal<P>& kf, LogLikAcc& acc, const 
 }
 #endif
 
+// KalmanFilterp::Predict (kfilter.cpp:218-337) of one query time t*, resumed from the forward filter's state.
+// ip: number of data times strictly before t*; st_z / st_D: the state (z, D) predicted at point ip - 1 (not read when
+// ip == 0); gap_before = t* - t[ip-1], gap_after = t[ip] - t* (each only read where it exists).  The curve is read
+// through y(i), dt(i) (gap from point i to i + 1) and e2(i) (yerr^2 of point i).  The linear-coefficient pass runs over
+// the ny - ip points behind the query.  Outputs: predictive mean (without mu) and variance.
+template <int P, class Tab, class Y, class DT, class E2>
+__device__ __forceinline__ void predict_resume(const RealParams<P>& prm, const Tab& tb, const double* st_z,
+                                               const double* st_D, int ip, int ny, double gap_before, double gap_after,
+                                               Y y, DT dt, E2 e2, double* qmean, double* qvar) {
+    constexpr int NS = P / 2, NT = P * (P + 1) / 2;
+    KalmanReal<P> kf;
+    double fa[NS > 0 ? NS : 1], fb[NS > 0 ? NS : 1], fsb[NS > 0 ? NS : 1], fo;
+    double pmean, pvar;
+    if (ip == 0) {
+        kf.reset(prm, 0.0);       // stationary law: mean 0, variance Re(b V b^H), g = V b^H
+        pmean = 0.0;
+        pvar = prm.v0;
+    } else {
+#pragma unroll
+        for (int i = 0; i < P; i++) kf.z[i] = st_z[i];
+#pragma unroll
+        for (int i = 0; i < NT; i++) kf.D[i] = st_D[i];
+        kf.observe(prm, e2(ip - 1));
+        const double innov = (y(ip - 1) - prm.mu) - kf.mean;
+        kf.template advance<false>(prm, tb, innov, 1.0 / kf.var, gap_before, 0.0);  // no noise at t*
+        pmean = kf.mean;
+        pvar = kf.var;
+    }
+    if (ip == ny) { *qmean = pmean; *qvar = pvar; return; }   // forecast: nothing behind the query
+    // InitializeCoefs (kfilter.cpp:290-312): y* enters as a noiseless pseudo-observation with the predictive law
+    double prec = 1.0 / pvar, pm = pmean * prec;
+    double zs[P];
+    {
+        const double inv = 1.0 / pvar;
+#pragma unroll
+        for (int i = 0; i < P; i++) zs[i] = kf.g[i] * inv;            // state_slope = K
+        kf.measurement_update(-pmean, inv);                           // state_const = x - K ymean ; P -= yvar K K^H
+        KalmanReal<P>::template transition<false>(prm, tb, gap_after, fa, fb, fsb, &fo);
+        KalmanReal<P>::propagate_vec(fa, fb, fsb, fo, zs);
+        kf.propagate(prm, fa, fb, fsb, fo, e2(ip));                   // kf.mean = yconst, kf.var = var[ip]
+    }
+    double yslope = KalmanReal<P>::observe_vec(zs);
+    prec += yslope * yslope / kf.var;
+    pm += yslope * ((y(ip) - prm.mu) - kf.mean) / kf.var;
+    for (int i = ip + 1; i < ny; i++) {                               // UpdateCoefs (kfilter.cpp:316-337)
+        const double inv = 1.0 / kf.var;
+        const double sl = yslope * inv;
+#pragma unroll
+        for (int j = 0; j < P; j++) zs[j] = fma(-kf.g[j], sl, zs[j]);  // state_slope -= K yslope
+        kf.measurement_update((y(i - 1) - prm.mu) - kf.mean, inv);     // state_const += K (y - yconst) ; P -= var K K^H
+        KalmanReal<P>::template transition<false>(prm, tb, dt(i - 1), fa, fb, fsb, &fo);
+        KalmanReal<P>::propagate_vec(fa, fb, fsb, fo, zs);
+        kf.propagate(prm, fa, fb, fsb, fo, e2(i));
+        yslope = KalmanReal<P>::observe_vec(zs);
+        prec += yslope * yslope / kf.var;
+        pm += yslope * ((y(i) - prm.mu) - kf.mean) / kf.var;
+    }
+    pvar = 1.0 / prec;
+    *qmean = pm * pvar;
+    *qvar = pvar;
+}
+
 // Exact (slow) evaluation of the log-likelihood of one theta: the same recursion with one log() per point.
 // Only reached when LogLikAcc::bad was raised (var not a positive normal number somewhere).
 template <int P, class Src, class Tab>

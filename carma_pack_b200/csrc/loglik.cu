@@ -341,7 +341,7 @@ template <int P>
 __global__ void __launch_bounds__(64)
 predict_real_kernel(SeriesView sv, ExplicitModel ex, const double* __restrict__ state, const double* __restrict__ tq, size_t nq,
                     double* __restrict__ qmean, double* __restrict__ qvar /* may be null */) {
-    constexpr int NS = P / 2, NT = P * (P + 1) / 2, SD = P + NT;
+    constexpr int SD = P + P * (P + 1) / 2;
     MathTab tb;
     tb.load();
     const size_t k = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -356,57 +356,14 @@ predict_real_kernel(SeriesView sv, ExplicitModel ex, const double* __restrict__ 
         if (sv.t[mid] < time) lo = mid + 1; else hi = mid;
     }
     const int ip = lo;
-    auto e2_at = [&](int i) { return i == 0 ? sv.e2_0 : sv.e2n[i - 1]; };
-    KalmanReal<P> kf;
-    double fa[NS > 0 ? NS : 1], fb[NS > 0 ? NS : 1], fsb[NS > 0 ? NS : 1], fo;
+    const double* st = state + (size_t)(ip > 0 ? ip - 1 : 0) * SD;
+    const double gap_before = ip > 0 ? fabs(time - sv.t[ip - 1]) : 0.0;
+    const double gap_after = ip < ny ? fabs(sv.t[ip] - time) : 0.0;
     double pmean, pvar;
-    if (ip == 0) {
-        kf.reset(prm, 0.0);       // stationary law: mean 0, variance Re(b V b^H), g = V b^H
-        pmean = 0.0;
-        pvar = prm.v0;
-    } else {
-        const double* st = state + (size_t)(ip - 1) * SD;
-#pragma unroll
-        for (int i = 0; i < P; i++) kf.z[i] = st[i];
-#pragma unroll
-        for (int i = 0; i < NT; i++) kf.D[i] = st[P + i];
-        kf.observe(prm, e2_at(ip - 1));
-        const double innov = (sv.y[ip - 1] - prm.mu) - kf.mean;
-        kf.template advance<false>(prm, tb, innov, 1.0 / kf.var, fabs(time - sv.t[ip - 1]), 0.0);  // no noise at t*
-        pmean = kf.mean;
-        pvar = kf.var;
-    }
-    if (ip == ny) { qmean[k] = pmean; if (qvar) qvar[k] = pvar; return; }   // forecast: nothing behind the query
-    // InitializeCoefs (kfilter.cpp:290-312): y* enters as a noiseless pseudo-observation with the predictive law
-    double prec = 1.0 / pvar, pm = pmean * prec;
-    double zs[P];
-    {
-        const double inv = 1.0 / pvar;
-#pragma unroll
-        for (int i = 0; i < P; i++) zs[i] = kf.g[i] * inv;            // state_slope = K
-        kf.measurement_update(-pmean, inv);                           // state_const = x - K ymean ; P -= yvar K K^H
-        KalmanReal<P>::template transition<false>(prm, tb, fabs(sv.t[ip] - time), fa, fb, fsb, &fo);
-        KalmanReal<P>::propagate_vec(fa, fb, fsb, fo, zs);
-        kf.propagate(prm, fa, fb, fsb, fo, e2_at(ip));                // kf.mean = yconst, kf.var = var[ip]
-    }
-    double yslope = KalmanReal<P>::observe_vec(zs);
-    prec += yslope * yslope / kf.var;
-    pm += yslope * ((sv.y[ip] - prm.mu) - kf.mean) / kf.var;
-    for (int i = ip + 1; i < ny; i++) {                               // UpdateCoefs (kfilter.cpp:316-337)
-        const double inv = 1.0 / kf.var;
-        const double sl = yslope * inv;
-#pragma unroll
-        for (int j = 0; j < P; j++) zs[j] = fma(-kf.g[j], sl, zs[j]);  // state_slope -= K yslope
-        kf.measurement_update((sv.y[i - 1] - prm.mu) - kf.mean, inv);  // state_const += K (y - yconst) ; P -= var K K^H
-        KalmanReal<P>::template transition<false>(prm, tb, sv.dt[i - 1], fa, fb, fsb, &fo);
-        KalmanReal<P>::propagate_vec(fa, fb, fsb, fo, zs);
-        kf.propagate(prm, fa, fb, fsb, fo, e2_at(i));
-        yslope = KalmanReal<P>::observe_vec(zs);
-        prec += yslope * yslope / kf.var;
-        pm += yslope * ((sv.y[i] - prm.mu) - kf.mean) / kf.var;
-    }
-    pvar = 1.0 / prec;
-    qmean[k] = pm * pvar;
+    predict_resume<P>(prm, tb, st, st + P, ip, ny, gap_before, gap_after, [&](int i) { return sv.y[i]; },
+                      [&](int i) { return sv.dt[i]; }, [&](int i) { return i == 0 ? sv.e2_0 : sv.e2n[i - 1]; },
+                      &pmean, &pvar);
+    qmean[k] = pmean;
     if (qvar) qvar[k] = pvar;
 }
 
@@ -738,7 +695,7 @@ void prior_from_stats(const SeriesStats& st, int population_var, carma_prior_t* 
     out->measerr_dof = 50.0;
 }
 
-static bool valid_model(int kind, int p, int q) {
+bool valid_model(int kind, int p, int q) {
     if (kind < CARMA_KIND_CAR1 || kind > CARMA_KIND_ZCARMA) return false;
     if (kind == CARMA_KIND_CAR1) return p == 1;
     if (p < 1 || p > MAX_P) return false;
@@ -970,11 +927,13 @@ int carma_multi_series_create(const double* time, const double* y, const double*
     m->device = device; m->ncurves = ncurves; m->total = total; m->dt_max = 0.0;
     m->off.assign(offsets, offsets + ncurves + 1);
     m->priors_pop.resize(ncurves); m->priors_sample.resize(ncurves);
+    m->t0.resize(ncurves);
     std::vector<double> dt(total + 1, 0.0), e2(total + 1, 0.0);
     for (size_t c = 0; c < ncurves; c++) {
         size_t o0 = (size_t)offsets[c], o1 = (size_t)offsets[c + 1];
         if (o1 < o0 + 2) { set_error("carma_multi_series_create: every curve needs >= 2 points"); delete m; return CARMA_ERR_ARG; }
         m->max_ny = std::max(m->max_ny, (int)(o1 - o0));
+        m->t0[c] = time[o0];
         double curve_dt_max = 0.0;
         for (size_t i = o0; i < o1; i++) {
             if (i + 1 < o1) {
@@ -1016,6 +975,7 @@ int carma_multi_series_destroy(carma_multi_series_t m) {
     if (m->d_e2) cudaFree(m->d_e2);
     if (m->d_off) cudaFree(m->d_off);
     m->scratch_in.release(); m->scratch_out.release(); m->scratch_pr.release(); m->scratch_misc.release();
+    m->scratch_pts.release(); m->scratch_q.release();
     delete m;
     return CARMA_OK;
 }

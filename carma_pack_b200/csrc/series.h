@@ -99,7 +99,9 @@ struct carma_multi_series {
     std::vector<long long> off;
     std::vector<carma_prior_t> priors_pop, priors_sample;
     std::vector<carma::CurveInfo> info;  // default (population-variance) priors + statistics
+    std::vector<double> t0;  // first time of every curve: the device holds gaps only, each curve's axis starts at 0
     carma::DevBuf scratch_in, scratch_out, scratch_pr, scratch_misc;
+    carma::DevBuf scratch_pts, scratch_q;  // per-point filter outputs and per-query records (survey.cu)
     int max_ny = 0;
     double dt_max = 1.0;  // longest sampling gap over all curves
 };
@@ -113,4 +115,5 @@ int scan_explicit(carma_series* s, int p, const ExplicitModel& ex, double* d_mea
                   double* d_loglik, cudaStream_t st, const double* d_y_override = nullptr);
 SeriesStats compute_stats(const double* t, const double* y, size_t n);
 void prior_from_stats(const SeriesStats& st, int population_var, carma_prior_t* out);
+bool valid_model(int kind, int p, int q);   // (kind, p, q) names a model the library evaluates
 }  // namespace carma

@@ -139,6 +139,7 @@ extern "C" int carma_multi_series_simulate(size_t ncurves, size_t ny, int kind, 
     m->max_ny = (int)ny;
     m->off.resize(ncurves + 1);
     for (size_t c = 0; c <= ncurves; c++) m->off[c] = (long long)(c * ny);
+    m->t0.assign(ncurves, 0.0);
     const int d = model_dim(kind, p, q);
     carma_prior_t pr;
     if (prior) {

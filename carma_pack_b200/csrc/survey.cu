@@ -1,0 +1,510 @@
+// survey.cu -- the KalmanFilterp outputs for every light curve of a multi-series, taking one theta row per curve the
+// way carma_multi_loglik does:
+//   multi_filter_kernel<P>     one thread = one curve: K4's recursion (same operations, so the log-density is bitwise
+//                              K4's) that also stores the one-step predictive mean and variance of every point;
+//   residual_acf_kernel        one warp = one curve: moments and autocorrelation of the standardised residuals
+//                              (the numeric part of CarmaSample.assess_fit_values) without sending them to the host;
+//   predict_forward_kernel<P>  one thread = one curve: the same recursion with a cursor over the curve's (time-sorted)
+//   predict_query_kernel<P>    queries, parking the state in front of each; then one thread = one query resumes from it
+//                              (predict_resume, shared with the single-series predict_real_kernel).
+#include <algorithm>
+#include <cmath>
+#include <cstdlib>
+#include <cstring>
+#include <numeric>
+#include <string>
+#include <vector>
+
+#include "kalman_real.cuh"
+#include "series.h"
+
+namespace carma {
+
+constexpr int SF_BLOCK = 64;
+
+__device__ __forceinline__ void stg4(double* q, double a, double b, double c, double d) {   // q 32-byte aligned
+    asm volatile("st.global.v4.f64 [%0], {%1, %2, %3, %4};" ::"l"(q), "d"(a), "d"(b), "d"(c), "d"(d) : "memory");
+}
+
+// filter_span_blocks (kalman_real.cuh) with the predictive mean / variance of every point stored to mo / vo.  The same
+// loads and the same steps in the same order, so the accumulated log-density is bitwise K4's.  Each thread writes its
+// own curve: with one 8-byte store per point a warp store touches 32 sectors.  BLKST: the four points of a block are
+// written with one 32-byte store per array (mo / vo sit like dt within a sector; the head and tail peel with scalar
+// stores); otherwise one scalar store per point and array.
+template <int P, bool ALLC, bool BLKST, class Tab>
+__device__ void filter_span_emit(KalmanReal<P>& kf, LogLikAcc& acc, const RealParams<P>& prm, const Tab& tb,
+                                 const double* __restrict__ dt, const double* __restrict__ y,
+                                 const double* __restrict__ E, int len, double* __restrict__ mo,
+                                 double* __restrict__ vo) {
+    const int nadv = len - 1;
+    int since = 0;
+    auto step = [&](double dt_i, double y_i, double e_i) {
+        const double innov = (y_i - prm.mu) - kf.mean;
+        const double inv = rcp_fast(kf.var);
+        acc.add(kf.var, innov, inv);
+        kf.template advance<ALLC>(prm, tb, innov, inv, dt_i, e_i);
+    };
+    int i = 0;
+    const int head = min(nadv, (int)((4u - (unsigned)(((size_t)dt >> 3) & 3u)) & 3u));
+    for (; i < head; i++) {
+        mo[i] = kf.mean; vo[i] = kf.var;
+        step(dt[i], y[i], E[i + 1]);
+    }
+    since = head;
+    if (i + 4 <= nadv) {
+        Dbl4 cdt = ldg4(dt + i), cy = ldg4(y + i), cE = ldg4(E + i);
+        for (;;) {
+            const bool nx = i + 8 <= len;   // the next block lies inside this curve
+            Dbl4 ndt = cdt, ny_ = cy, nE = cE;
+            double e_last;
+            if (nx) {
+                ndt = ldg4(dt + i + 4); ny_ = ldg4(y + i + 4); nE = ldg4(E + i + 4);
+                e_last = nE.a;
+            } else {
+                e_last = E[i + 4];          // i + 4 <= nadv = len - 1
+            }
+            const double m0 = kf.mean, v0 = kf.var;
+            step(cdt.a, cy.a, cE.b);
+            const double m1 = kf.mean, v1 = kf.var;
+            step(cdt.b, cy.b, cE.c);
+            const double m2 = kf.mean, v2 = kf.var;
+            step(cdt.c, cy.c, cE.d);
+            const double m3 = kf.mean, v3 = kf.var;
+            step(cdt.d, cy.d, e_last);
+            if (BLKST) {
+                stg4(mo + i, m0, m1, m2, m3);
+                stg4(vo + i, v0, v1, v2, v3);
+            } else {
+                mo[i] = m0; mo[i + 1] = m1; mo[i + 2] = m2; mo[i + 3] = m3;
+                vo[i] = v0; vo[i + 1] = v1; vo[i + 2] = v2; vo[i + 3] = v3;
+            }
+            i += 4;
+            since += 4;
+            if (since >= RENORM_EVERY - 8) { acc.renorm(since); since = 0; }
+            if (!nx || i + 4 > nadv) break;
+            cdt = ndt; cy = ny_; cE = nE;
+        }
+    }
+    for (; i < nadv; i++, since++) {
+        mo[i] = kf.mean; vo[i] = kf.var;
+        step(dt[i], y[i], E[i + 1]);
+    }
+    if (since) acc.renorm(since);
+    {   // the last point is only scored
+        mo[len - 1] = kf.mean; vo[len - 1] = kf.var;
+        const double innov = (y[len - 1] - prm.mu) - kf.mean;
+        const double inv = rcp_fast(kf.var);
+        acc.add(kf.var, innov, inv);
+        acc.renorm(1);
+    }
+}
+
+template <int P, bool BLKST>
+__global__ void __launch_bounds__(SF_BLOCK, P <= 3 ? 8 : 1)   // K4's bounds
+multi_filter_kernel(const double* __restrict__ dt, const double* __restrict__ y, const double* __restrict__ e2,
+                    const long long* __restrict__ off, size_t ncurves, double dt_max, int kind, int q, int d,
+                    unsigned flags, const carma_prior_t* __restrict__ priors, const double* __restrict__ theta,
+                    double* __restrict__ mean, double* __restrict__ var, double* __restrict__ out /* may be null */) {
+    MathTab tb;
+    tb.load();
+    const size_t c = (size_t)blockIdx.x * SF_BLOCK + threadIdx.x;
+    if (c >= ncurves) return;
+    const long long o0 = off[c], o1 = off[c + 1];
+    const int ny = (int)(o1 - o0);
+    double th[MAX_D];
+#pragma unroll
+    for (int j = 0; j < MAX_D; j++) th[j] = (j < d) ? theta[c * (size_t)d + j] : 0.0;
+    RealParams<P> prm;
+    carma_prior_t pr = priors[c];
+    if (transform_theta<P>(kind, q, flags, pr, th, dt_max, prm) != TT_OK) {
+        for (int i = 0; i < ny; i++) { mean[o0 + i] = NAN; var[o0 + i] = NAN; }
+        if (out) out[c] = -INFINITY;
+        return;
+    }
+    KalmanReal<P> kf;
+    LogLikAcc acc;
+    kf.reset(prm, e2[o0]);
+    acc.init();
+    constexpr unsigned ALL = (P / 2 > 0) ? ((1u << (P / 2)) - 1u) : 0u;
+    if (__all_sync(__activemask(), prm.cmask == ALL))   // warp-uniform, as filter_span_blocks_any
+        filter_span_emit<P, true, BLKST>(kf, acc, prm, tb, dt + o0, y + o0, e2 + o0, ny, mean + o0, var + o0);
+    else
+        filter_span_emit<P, false, BLKST>(kf, acc, prm, tb, dt + o0, y + o0, e2 + o0, ny, mean + o0, var + o0);
+    if (out) {
+        const SeriesPtr src{dt + o0, y + o0, e2 + o0 + 1};
+        out[c] = (acc.bad() ? loglik_exact_slow<P>(prm, tb, src, ny, e2[o0]) : acc.value()) + prm.logprior;
+    }
+}
+
+// One warp per curve.  Pass 1 turns mean into the standardised residuals r = (y - (mean + mu)) / sqrt(var) in place and
+// sums r and r^2; pass 2: lane k sums (r_i - rbar)(r_{i+L} - rbar) over i in index order for its lags L = k, k + 32, ...
+// (r and r^2), with r_i read by every lane and r_{i+L} adjacent across lanes.  Fixed summation order: deterministic.
+// out row (3 + 2 nlags): loglik, mean(r), population std(r), acf(r)[1..nlags], acf(r^2)[1..nlags] (mean-subtracted,
+// normalised by lag 0).
+constexpr int ACF_BLOCK = 128;
+__global__ void __launch_bounds__(ACF_BLOCK)
+residual_acf_kernel(const double* __restrict__ y, const long long* __restrict__ off, size_t ncurves,
+                    const double* __restrict__ theta, int d, const double* __restrict__ loglik, double* mean,
+                    const double* __restrict__ var, int nlags, double* __restrict__ out) {
+    const size_t c = ((size_t)blockIdx.x * ACF_BLOCK + threadIdx.x) / 32;
+    const int lane = threadIdx.x & 31;
+    if (c >= ncurves) return;   // uniform over the warp
+    const long long o0 = off[c];
+    const int ny = (int)(off[c + 1] - o0);
+    const double mu = theta[c * (size_t)d + 2];
+    double* r = mean + o0;
+    double s1 = 0.0, s2 = 0.0;
+    for (int i = lane; i < ny; i += 32) {
+        const double ri = (y[o0 + i] - (r[i] + mu)) / sqrt(var[o0 + i]);
+        r[i] = ri;
+        s1 += ri;
+        s2 += ri * ri;
+    }
+#pragma unroll
+    for (int k = 16; k >= 1; k >>= 1) {
+        s1 += __shfl_xor_sync(0xffffffffu, s1, k);
+        s2 += __shfl_xor_sync(0xffffffffu, s2, k);
+    }
+    __syncwarp();   // the residuals of every lane are visible to the warp
+    const double rbar = s1 / ny, qbar = s2 / ny;
+    const int w = 3 + 2 * nlags;
+    double* o = out + c * (size_t)w;
+    double c0r = 0.0, c0q = 0.0;
+    for (int L = lane; L <= nlags; L += 32) {
+        double ar = 0.0, aq = 0.0;
+        for (int i = 0; i + L < ny; i++) {
+            const double a = r[i], b = r[i + L];
+            ar += (a - rbar) * (b - rbar);
+            aq += (a * a - qbar) * (b * b - qbar);
+        }
+        if (L == 0) { c0r = ar; c0q = aq; }
+        else { o[2 + L] = ar; o[2 + nlags + L] = aq; }
+    }
+    c0r = __shfl_sync(0xffffffffu, c0r, 0);
+    c0q = __shfl_sync(0xffffffffu, c0q, 0);
+    for (int L = lane; L <= nlags; L += 32) {
+        if (L == 0) continue;
+        o[2 + L] /= c0r;
+        o[2 + nlags + L] /= c0q;
+    }
+    if (lane == 0) {
+        o[0] = loglik[c];
+        o[1] = rbar;
+        o[2] = sqrt(c0r / ny);
+    }
+}
+
+// Predict, forward part.  Curve c's queries are qtq[qoff[c] .. qoff[c+1]), sorted by time, on the curve's own axis (the
+// running sum of its gaps from 0, as carma_multi_series_get_curve forms it).  For every query the record holds the state
+// (z, D) predicted at point ip - 1 (ip = number of data times strictly before t*), then t* - t[ip-1], t[ip] - t* and ip.
+template <int P>
+struct PredictRec {
+    static constexpr int NT = P * (P + 1) / 2, SD = P + NT, R = SD + 3;
+};
+
+template <int P>
+__global__ void __launch_bounds__(SF_BLOCK)
+predict_forward_kernel(const double* __restrict__ dt, const double* __restrict__ y, const double* __restrict__ e2,
+                       const long long* __restrict__ off, size_t ncurves, double dt_max, int kind, int q, int d,
+                       unsigned flags, const carma_prior_t* __restrict__ priors, const double* __restrict__ theta,
+                       const long long* __restrict__ qoff, const double* __restrict__ qtq, double* __restrict__ rec,
+                       RealParams<P>* __restrict__ prm_out, int* __restrict__ status_out) {
+    using PR = PredictRec<P>;
+    MathTab tb;
+    tb.load();
+    const size_t c = (size_t)blockIdx.x * SF_BLOCK + threadIdx.x;
+    if (c >= ncurves) return;
+    long long k = qoff[c];
+    const long long k1 = qoff[c + 1];
+    double th[MAX_D];
+#pragma unroll
+    for (int j = 0; j < MAX_D; j++) th[j] = (j < d) ? theta[c * (size_t)d + j] : 0.0;
+    RealParams<P> prm;
+    carma_prior_t pr = priors[c];
+    const int status = transform_theta<P>(kind, q, flags, pr, th, dt_max, prm);
+    prm_out[c] = prm;        // the query threads of this curve read the constants from here
+    status_out[c] = status;
+    if (status != TT_OK || k == k1) return;
+    const long long o0 = off[c];
+    const int ny = (int)(off[c + 1] - o0);
+    const double *cdt = dt + o0, *cy = y + o0, *cE = e2 + o0;
+    double t = 0.0;
+    for (; k < k1 && !(qtq[k] > t); k++) {   // at or before the first point: ip = 0
+        double* r = rec + (size_t)k * PR::R;
+        r[PR::SD] = 0.0;
+        r[PR::SD + 1] = fabs(t - qtq[k]);
+        r[PR::SD + 2] = 0.0;
+    }
+    KalmanReal<P> kf;
+    kf.reset(prm, cE[0]);
+    for (int i = 0; i < ny && k < k1; i++) {
+        const bool last = i + 1 == ny;
+        const double tn = last ? 0.0 : t + cdt[i];
+        for (; k < k1 && (last || !(qtq[k] > tn)); k++) {   // t[i] < t* <= t[i+1], or past the last point
+            double* r = rec + (size_t)k * PR::R;
+#pragma unroll
+            for (int j = 0; j < P; j++) r[j] = kf.z[j];
+#pragma unroll
+            for (int j = 0; j < PR::NT; j++) r[P + j] = kf.D[j];
+            r[PR::SD] = fabs(qtq[k] - t);
+            r[PR::SD + 1] = last ? 0.0 : fabs(tn - qtq[k]);
+            r[PR::SD + 2] = (double)(i + 1);
+        }
+        if (last || k == k1) break;
+        const double innov = (cy[i] - prm.mu) - kf.mean;
+        kf.template advance<false>(prm, tb, innov, 1.0 / kf.var, cdt[i], cE[i + 1]);
+        t = tn;
+    }
+}
+
+// Predict, query part: one thread per query (sorted curve-major, then by time, so a warp walks one curve), result
+// written to the caller's position perm[k].
+template <int P>
+__global__ void __launch_bounds__(SF_BLOCK)
+predict_query_kernel(const double* __restrict__ dt, const double* __restrict__ y, const double* __restrict__ e2,
+                     const long long* __restrict__ off, const int* __restrict__ qcurve, const long long* __restrict__ perm,
+                     size_t nq, const double* __restrict__ rec, const RealParams<P>* __restrict__ prms,
+                     const int* __restrict__ status, double* __restrict__ qmean, double* __restrict__ qvar) {
+    using PR = PredictRec<P>;
+    MathTab tb;
+    tb.load();
+    const size_t k = (size_t)blockIdx.x * SF_BLOCK + threadIdx.x;
+    if (k >= nq) return;
+    const int c = qcurve[k];
+    const long long dst = perm[k];
+    if (status[c] != TT_OK) { qmean[dst] = NAN; qvar[dst] = NAN; return; }
+    const RealParams<P> prm = prms[c];
+    const double* r = rec + k * PR::R;
+    const long long o0 = off[c];
+    const int ny = (int)(off[c + 1] - o0);
+    double pm, pv;
+    predict_resume<P>(prm, tb, r, r + P, (int)r[PR::SD + 2], ny, r[PR::SD], r[PR::SD + 1],
+                      [&](int i) { return y[o0 + i]; }, [&](int i) { return dt[o0 + i]; },
+                      [&](int i) { return e2[o0 + i]; }, &pm, &pv);
+    qmean[dst] = pm;
+    qvar[dst] = pv;
+}
+
+// ---- launchers ---------------------------------------------------------------------------------------------------
+static bool alike32(const void* a, const void* b) { return (((size_t)a ^ (size_t)b) & 31u) == 0; }
+
+static cudaError_t launch_multi_filter(const carma_multi_series* m, int kind, int p, int q, unsigned flags,
+                                       const carma_prior_t* d_priors, const double* d_theta, double* d_mean,
+                                       double* d_var, double* d_out, cudaStream_t st) {
+    const int d = model_dim(kind, p, q);
+    const unsigned grid = (unsigned)((m->ncurves + SF_BLOCK - 1) / SF_BLOCK);
+    // block stores need mean / var to sit like the curve arrays within a 32-byte sector; CARMA_MULTI_FILTER_STORES=scalar
+    // selects one store per point (kept for comparison; read at every call so both can be timed in one process)
+    const char* env = getenv("CARMA_MULTI_FILTER_STORES");
+    const bool blk = !(env && !strcmp(env, "scalar")) && alike32(m->d_dt, d_mean) && alike32(m->d_dt, d_var);
+#define LAUNCH_SF(PP)                                                                                                  \
+    if (blk) multi_filter_kernel<PP, true><<<grid, SF_BLOCK, 0, st>>>(m->d_dt, m->d_y, m->d_e2, m->d_off, m->ncurves,   \
+                                                                     m->dt_max, kind, q, d, flags, d_priors, d_theta,  \
+                                                                     d_mean, d_var, d_out);                            \
+    else multi_filter_kernel<PP, false><<<grid, SF_BLOCK, 0, st>>>(m->d_dt, m->d_y, m->d_e2, m->d_off, m->ncurves,      \
+                                                                  m->dt_max, kind, q, d, flags, d_priors, d_theta,     \
+                                                                  d_mean, d_var, d_out)
+    switch (p) {
+        case 1: LAUNCH_SF(1); break;
+        case 2: LAUNCH_SF(2); break;
+        case 3: LAUNCH_SF(3); break;
+        case 4: LAUNCH_SF(4); break;
+        case 5: LAUNCH_SF(5); break;
+        case 6: LAUNCH_SF(6); break;
+        case 7: LAUNCH_SF(7); break;
+        default: return cudaErrorInvalidValue;
+    }
+#undef LAUNCH_SF
+    return cudaGetLastError();
+}
+
+template <int P>
+static cudaError_t launch_predict_p(const carma_multi_series* m, int kind, int q, unsigned flags, double dt_max,
+                                    const carma_prior_t* d_priors, const double* d_theta, const long long* d_qoff,
+                                    const double* d_qtq, const int* d_qcurve, const long long* d_perm, size_t nq,
+                                    double* d_rec, void* d_prm, int* d_status, double* d_qm, double* d_qv,
+                                    cudaStream_t st) {
+    const int d = model_dim(kind, P, q);
+    predict_forward_kernel<P><<<(unsigned)((m->ncurves + SF_BLOCK - 1) / SF_BLOCK), SF_BLOCK, 0, st>>>(
+        m->d_dt, m->d_y, m->d_e2, m->d_off, m->ncurves, dt_max, kind, q, d, flags, d_priors, d_theta, d_qoff, d_qtq,
+        d_rec, (RealParams<P>*)d_prm, d_status);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    predict_query_kernel<P><<<(unsigned)((nq + SF_BLOCK - 1) / SF_BLOCK), SF_BLOCK, 0, st>>>(
+        m->d_dt, m->d_y, m->d_e2, m->d_off, d_qcurve, d_perm, nq, d_rec, (const RealParams<P>*)d_prm, d_status, d_qm,
+        d_qv);
+    return cudaGetLastError();
+}
+
+// upload the priors (NULL: the population-variance defaults) and theta rows into the multi-series' scratch
+static int upload_rows(carma_multi_series* m, int kind, int p, int q, const carma_prior_t* priors, const double* theta,
+                       cudaStream_t st) {
+    const size_t d = (size_t)model_dim(kind, p, q), n = m->ncurves;
+    if (!m->scratch_in.reserve(n * d * sizeof(double)) || !m->scratch_pr.reserve(n * sizeof(carma_prior_t)))
+        return CARMA_ERR_CUDA;
+    const carma_prior_t* hp = priors ? priors : m->priors_pop.data();
+    if (!cuda_ok(cudaMemcpyAsync(m->scratch_pr.p, hp, n * sizeof(carma_prior_t), cudaMemcpyHostToDevice, st), "H2D priors") ||
+        !cuda_ok(cudaMemcpyAsync(m->scratch_in.p, theta, n * d * sizeof(double), cudaMemcpyHostToDevice, st), "H2D theta"))
+        return CARMA_ERR_CUDA;
+    return CARMA_OK;
+}
+
+static size_t round32(size_t n) { return (n + 31) & ~(size_t)31; }   // doubles: keeps 256-byte alignment
+
+}  // namespace carma
+
+using namespace carma;
+
+extern "C" {
+
+int carma_multi_filter_dev(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* d_priors,
+                           const double* d_theta, unsigned flags, double* d_mean, double* d_var, double* d_loglik,
+                           void* stream) {
+    if (!m || !d_priors || !d_theta || !d_mean || !d_var) { set_error("carma_multi_filter_dev: null argument"); return CARMA_ERR_ARG; }
+    if (!valid_model(kind, p, q)) { set_error("carma_multi_filter_dev: invalid (kind,p,q)"); return CARMA_ERR_ARG; }
+    if (!alike32(m->d_dt, m->d_y) || !alike32(m->d_dt, m->d_e2)) { set_error("carma_multi_filter_dev: curve arrays not sector-aligned"); return CARMA_ERR_ARG; }
+    if (!cuda_ok(launch_multi_filter(m, kind, p, q, flags, d_priors, d_theta, d_mean, d_var, d_loglik, (cudaStream_t)stream),
+                 "multi_filter_kernel launch"))
+        return CARMA_ERR_CUDA;
+    return CARMA_OK;
+}
+
+// the filter of every curve into the multi-series' scratch: mean at scratch_pts, var behind it, loglik in scratch_out
+static int multi_filter_to_scratch(carma_multi_series* m, int kind, int p, int q, const carma_prior_t* priors,
+                                   const double* theta, unsigned flags, cudaStream_t st, double** d_mean, double** d_var) {
+    if (!cuda_ok(cudaSetDevice(m->device), "cudaSetDevice")) return CARMA_ERR_CUDA;
+    const size_t stride = round32(m->total);
+    if (!m->scratch_pts.reserve(2 * stride * sizeof(double)) || !m->scratch_out.reserve(m->ncurves * sizeof(double)))
+        return CARMA_ERR_CUDA;
+    int rc = upload_rows(m, kind, p, q, priors, theta, st);
+    if (rc) return rc;
+    *d_mean = (double*)m->scratch_pts.p;
+    *d_var = *d_mean + stride;
+    return carma_multi_filter_dev(m, kind, p, q, (const carma_prior_t*)m->scratch_pr.p, (const double*)m->scratch_in.p,
+                                  flags, *d_mean, *d_var, (double*)m->scratch_out.p, st);
+}
+
+int carma_multi_filter(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* priors, const double* theta,
+                       unsigned flags, double* mean, double* var, double* loglik) {
+    if (!m || !theta || !mean || !var) { set_error("carma_multi_filter: null argument"); return CARMA_ERR_ARG; }
+    if (!valid_model(kind, p, q)) { set_error("carma_multi_filter: invalid (kind,p,q)"); return CARMA_ERR_ARG; }
+    cudaStream_t st = 0;
+    double *d_mean = nullptr, *d_var = nullptr;
+    int rc = multi_filter_to_scratch(m, kind, p, q, priors, theta, flags, st, &d_mean, &d_var);
+    if (rc) return rc;
+    const size_t n = m->total;
+    if (!cuda_ok(cudaMemcpyAsync(mean, d_mean, n * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H mean") ||
+        !cuda_ok(cudaMemcpyAsync(var, d_var, n * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H var"))
+        return CARMA_ERR_CUDA;
+    if (loglik && !cuda_ok(cudaMemcpyAsync(loglik, m->scratch_out.p, m->ncurves * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H loglik"))
+        return CARMA_ERR_CUDA;
+    if (!cuda_ok(cudaStreamSynchronize(st), "multi_filter sync")) return CARMA_ERR_CUDA;
+    return CARMA_OK;
+}
+
+int carma_multi_assess_fit(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* priors,
+                           const double* theta, unsigned flags, int nlags, double* out) {
+    if (nlags < 1) { set_error("carma_multi_assess_fit: nlags must be >= 1"); return CARMA_ERR_ARG; }
+    if (!m || !theta || !out) { set_error("carma_multi_assess_fit: null argument"); return CARMA_ERR_ARG; }
+    if (!valid_model(kind, p, q)) { set_error("carma_multi_assess_fit: invalid (kind,p,q)"); return CARMA_ERR_ARG; }
+    long long min_ny = m->off[1] - m->off[0];
+    for (size_t c = 1; c < m->ncurves; c++) min_ny = std::min(min_ny, m->off[c + 1] - m->off[c]);
+    if ((long long)nlags >= min_ny) {
+        set_error("carma_multi_assess_fit: nlags must be below the shortest curve's length (" + std::to_string(min_ny) + ")");
+        return CARMA_ERR_ARG;
+    }
+    cudaStream_t st = 0;
+    double *d_mean = nullptr, *d_var = nullptr;
+    int rc = multi_filter_to_scratch(m, kind, p, q, priors, theta, flags, st, &d_mean, &d_var);
+    if (rc) return rc;
+    const size_t w = 3 + 2 * (size_t)nlags, n = m->ncurves;
+    if (!m->scratch_misc.reserve(n * w * sizeof(double))) return CARMA_ERR_CUDA;
+    const unsigned grid = (unsigned)((n * 32 + ACF_BLOCK - 1) / ACF_BLOCK);
+    residual_acf_kernel<<<grid, ACF_BLOCK, 0, st>>>(m->d_y, m->d_off, n, (const double*)m->scratch_in.p,
+                                                    model_dim(kind, p, q), (const double*)m->scratch_out.p, d_mean,
+                                                    d_var, nlags, (double*)m->scratch_misc.p);
+    if (!cuda_ok(cudaGetLastError(), "residual_acf_kernel launch")) return CARMA_ERR_CUDA;
+    if (!cuda_ok(cudaMemcpyAsync(out, m->scratch_misc.p, n * w * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H assess_fit") ||
+        !cuda_ok(cudaStreamSynchronize(st), "multi_assess_fit sync"))
+        return CARMA_ERR_CUDA;
+    return CARMA_OK;
+}
+
+int carma_multi_predict(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* priors,
+                        const double* theta, unsigned flags, const int64_t* q_offsets, const double* tq, double* qmean,
+                        double* qvar) {
+    if (q_offsets && q_offsets[0] != 0) { set_error("carma_multi_predict: q_offsets must start at 0"); return CARMA_ERR_ARG; }
+    if (!m || !theta || !q_offsets) { set_error("carma_multi_predict: null argument"); return CARMA_ERR_ARG; }
+    if (!valid_model(kind, p, q)) { set_error("carma_multi_predict: invalid (kind,p,q)"); return CARMA_ERR_ARG; }
+    const size_t nc = m->ncurves;
+    for (size_t c = 0; c < nc; c++)
+        if (q_offsets[c + 1] < q_offsets[c]) { set_error("carma_multi_predict: q_offsets must be non-decreasing"); return CARMA_ERR_ARG; }
+    const size_t nq = (size_t)q_offsets[nc];
+    if (nq == 0) return CARMA_OK;
+    if (!tq || !qmean || !qvar) { set_error("carma_multi_predict: null argument"); return CARMA_ERR_ARG; }
+    for (size_t k = 0; k < nq; k++)
+        if (!std::isfinite(tq[k])) { set_error("carma_multi_predict: non-finite query time"); return CARMA_ERR_ARG; }
+    // sort every curve's queries by time, on the curve's own axis (t - t0[c]); the rate clamp must cover the longest
+    // transition of the call: the data gaps, forecasts past the last point and backcasts before the first
+    std::vector<long long> perm(nq);
+    std::vector<double> qtq(nq);
+    std::vector<int> qcurve(nq);
+    double dt_max = m->dt_max;
+    for (size_t c = 0; c < nc; c++) {
+        const size_t k0 = (size_t)q_offsets[c], k1 = (size_t)q_offsets[c + 1];
+        std::iota(perm.begin() + k0, perm.begin() + k1, (long long)k0);
+        std::stable_sort(perm.begin() + k0, perm.begin() + k1, [&](long long a, long long b) { return tq[a] < tq[b]; });
+        const double tspan = m->info[c].tspan;
+        for (size_t k = k0; k < k1; k++) {
+            qtq[k] = tq[perm[k]] - m->t0[c];
+            qcurve[k] = (int)c;
+            dt_max = std::max(dt_max, std::max(qtq[k] - tspan, -qtq[k]));
+        }
+    }
+    if (!cuda_ok(cudaSetDevice(m->device), "cudaSetDevice")) return CARMA_ERR_CUDA;
+    cudaStream_t st = 0;
+    int rc = upload_rows(m, kind, p, q, priors, theta, st);
+    if (rc) return rc;
+    // scratch_q: records | qtq | qm | qv | perm | qoff | prm | status | qcurve, each on a 256-byte boundary
+    const size_t R = (size_t)(p + p * (p + 1) / 2 + 3);
+    const size_t b_rec = round32(nq * R), b_q = round32(nq), b_off = round32(nc + 1),
+                 b_prm = round32((nc * sizeof(RealParams<MAX_P>) + 7) / 8), b_st = round32((nc + 1) / 2), b_qc = round32((nq + 1) / 2);
+    if (!m->scratch_q.reserve((b_rec + 4 * b_q + b_off + b_prm + b_st + b_qc) * sizeof(double))) return CARMA_ERR_CUDA;
+    double* d_rec = (double*)m->scratch_q.p;
+    double* d_qtq = d_rec + b_rec;
+    double* d_qm = d_qtq + b_q;
+    double* d_qv = d_qm + b_q;
+    long long* d_perm = (long long*)(d_qv + b_q);
+    long long* d_qoff = (long long*)((double*)d_perm + b_q);
+    void* d_prm = (double*)d_qoff + b_off;
+    int* d_status = (int*)((double*)d_prm + b_prm);
+    int* d_qcurve = (int*)((double*)d_status + b_st);
+    bool ok = cuda_ok(cudaMemcpyAsync(d_qtq, qtq.data(), nq * sizeof(double), cudaMemcpyHostToDevice, st), "H2D tq") &&
+              cuda_ok(cudaMemcpyAsync(d_perm, perm.data(), nq * sizeof(long long), cudaMemcpyHostToDevice, st), "H2D perm") &&
+              cuda_ok(cudaMemcpyAsync(d_qoff, q_offsets, (nc + 1) * sizeof(long long), cudaMemcpyHostToDevice, st), "H2D q_offsets") &&
+              cuda_ok(cudaMemcpyAsync(d_qcurve, qcurve.data(), nq * sizeof(int), cudaMemcpyHostToDevice, st), "H2D qcurve");
+    if (!ok) return CARMA_ERR_CUDA;
+    const carma_prior_t* d_pr = (const carma_prior_t*)m->scratch_pr.p;
+    const double* d_th = (const double*)m->scratch_in.p;
+    cudaError_t e;
+#define LAUNCH_PQ(PP) e = launch_predict_p<PP>(m, kind, q, flags, dt_max, d_pr, d_th, d_qoff, d_qtq, d_qcurve, d_perm, nq, \
+                                                d_rec, d_prm, d_status, d_qm, d_qv, st)
+    switch (p) {
+        case 1: LAUNCH_PQ(1); break;
+        case 2: LAUNCH_PQ(2); break;
+        case 3: LAUNCH_PQ(3); break;
+        case 4: LAUNCH_PQ(4); break;
+        case 5: LAUNCH_PQ(5); break;
+        case 6: LAUNCH_PQ(6); break;
+        default: LAUNCH_PQ(7); break;
+    }
+#undef LAUNCH_PQ
+    if (!cuda_ok(e, "predict kernels launch")) return CARMA_ERR_CUDA;
+    if (!cuda_ok(cudaMemcpyAsync(qmean, d_qm, nq * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H qmean") ||
+        !cuda_ok(cudaMemcpyAsync(qvar, d_qv, nq * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H qvar") ||
+        !cuda_ok(cudaStreamSynchronize(st), "multi_predict sync"))
+        return CARMA_ERR_CUDA;
+    return CARMA_OK;
+}
+
+}  // extern "C"

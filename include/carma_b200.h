@@ -230,6 +230,31 @@ int carma_multi_loglik_dev(carma_multi_series_t m, int kind, int p, int q, const
                            const double* d_theta /* ncurves x d */, double* d_logpost, unsigned flags, void* stream);
 int carma_multi_loglik(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* priors,
                        const double* theta, double* logpost, unsigned flags);
+/* KalmanFilterp::Filter + GetMean()/GetVar() (src/kfilter.cpp:138-215) of every curve with its own theta row, in one
+ * launch: theta ncurves x d, priors ncurves entries or NULL (population-variance defaults), as carma_multi_loglik.
+ * mean / var: the one-step predictive mean (without mu) and variance (with measerr_scale * yerr^2) at every point, in the
+ * CSR order of the multi-series (total points); mean[first] = 0 and var[first] = Var(y) + scale * yerr_first^2 for every
+ * curve, as carma_filter.  loglik (ncurves, may be NULL): bitwise what carma_multi_loglik returns for the same
+ * arguments.  A row the transform rejects gives NaN mean / var for its curve and -inf loglik.  _dev: device pointers and
+ * a stream, no synchronisation. */
+int carma_multi_filter_dev(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* d_priors,
+                           const double* d_theta, unsigned flags, double* d_mean, double* d_var, double* d_loglik,
+                           void* stream);
+int carma_multi_filter(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* priors, const double* theta,
+                       unsigned flags, double* mean, double* var, double* loglik);
+/* The numeric part of assess_fit (CarmaSample.assess_fit_values) for every curve, without the per-point outputs crossing
+ * PCIe: with r = (y - mu - mean) / sqrt(var) the standardised one-step residuals, out holds per curve 3 + 2 nlags
+ * doubles: loglik, mean(r), population std(r), acf(r)[1..nlags], acf(r^2)[1..nlags] (mean-subtracted, normalised by
+ * lag 0).  1 <= nlags < the shortest curve's length. */
+int carma_multi_assess_fit(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* priors,
+                           const double* theta, unsigned flags, int nlags, double* out);
+/* KalmanFilterp::Predict (src/kfilter.cpp:218-337) of every curve at its own query times: q_offsets ncurves+1 (CSR)
+ * into tq, times absolute (on the axis the curves were created with), in any order, possibly equal to data times.
+ * qmean (without mu) / qvar come back in the caller's order.  Forecasts, backcasts and interpolation as carma_predict;
+ * a curve's queries cost O(ny - ip) filter steps each (ip: data points before the query). */
+int carma_multi_predict(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* priors,
+                        const double* theta, unsigned flags, const int64_t* q_offsets, const double* tq, double* qmean,
+                        double* qvar);
 
 /* ---- one very long light curve: temporally parallel (associative-scan) form of the same LogDensity ----
  * Replaces the strictly sequential Filter() loop (src/include/kfilter.hpp:126-132) when there is a single
