@@ -54,6 +54,7 @@ EXPORTED_SYMBOLS = [
     "carma_gather_summaries", "carma_gather_summaries_dev", "carma_derived_params", "carma_derived_params_dev", "carma_mle_batch_device",
     "carma_mle_grid_device", "carma_multi_series_curve_stats", "carma_multi_mle_grid_device",
     "carma_multi_filter_dev", "carma_multi_filter", "carma_multi_assess_fit", "carma_multi_predict",
+    "carma_multi_simulate",
 ]
 
 
@@ -168,6 +169,8 @@ def _load():
                                          ctypes.c_int, _vp]
     L.carma_multi_predict.argtypes = [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp, _vp, ctypes.c_uint, _vp, _vp,
                                       _vp, _vp]
+    L.carma_multi_simulate.argtypes = [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp, _vp, _sz, ctypes.c_uint, _vp,
+                                       _vp, _sz, ctypes.c_uint64, ctypes.c_uint32, _vp]
     L.carma_filter.argtypes = [_vp, ctypes.c_double, _dp, _dp, ctypes.c_int, ctypes.c_double, ctypes.c_double, _dp, _dp]
     L.carma_predict.argtypes = [_vp, ctypes.c_double, _dp, _dp, ctypes.c_int, ctypes.c_double, ctypes.c_double,
                                 _dp, _sz, _dp, _dp]
@@ -696,6 +699,36 @@ class MultiSeries:
                                       qv.ctypes.data), "carma_multi_predict")
         qm += np.repeat(th[:, 2], np.diff(qo))
         return qm, qv
+
+    def conditional_simulate(self, kind, p, q, theta, tsim, s_offsets, npaths=1, seed=None, curve_offset=0, priors=None,
+                             flags=None):
+        """Draws of every curve at its own times given its data (carma_multi_simulate, the survey form of
+        CarmaSample.simulate).  tsim: absolute times, curve c's at tsim[s_offsets[c]:s_offsets[c+1]], any order.
+        theta: (ncurves, d), one row for all paths of a curve, or (ncurves, npaths, d), one row per path (posterior
+        predictive).  Path j of curve c depends only on (seed, j, curve_offset + c) and its theta row.  Returns
+        (npaths, len(tsim)) in the order of tsim, mu included.  flags: None = the survey fits' rule."""
+        d = model_dim(kind, p, q)
+        npaths = int(npaths)
+        if npaths < 1:
+            raise ValueError("npaths must be >= 1")
+        th = np.ascontiguousarray(theta, dtype=np.float64)
+        if th.shape == (self.ncurves, npaths, d):
+            th = th.reshape(self.ncurves * npaths, d)
+        elif th.shape != (self.ncurves, d):
+            raise ValueError("theta must be (%d, %d) or (%d, %d, %d)" % (self.ncurves, d, self.ncurves, npaths, d))
+        _, priors = self._rows(kind, p, q, th[:self.ncurves], priors)
+        t = _c(np.atleast_1d(tsim))
+        so = np.ascontiguousarray(s_offsets, dtype=np.int64)
+        if so.shape != (self.ncurves + 1,) or so[0] != 0 or so[-1] != t.size:
+            raise ValueError("s_offsets must have %d entries from 0 to len(tsim) = %d" % (self.ncurves + 1, t.size))
+        if seed is None:
+            seed = int(np.random.SeedSequence().generate_state(1, dtype=np.uint64)[0] >> 1)
+        out = np.empty((npaths, t.size))
+        check(lib.carma_multi_simulate(self.handle, kind, p, q, None if priors is None else priors.ctypes.data,
+                                       th.ctypes.data, th.shape[0], self._default_flags(p, flags), so.ctypes.data,
+                                       t.ctypes.data, npaths, int(seed), int(curve_offset), out.ctypes.data),
+              "carma_multi_simulate")
+        return out
 
 
 def lbfgs_batch(fun_batch, x0, lower, upper, maxiter=1000, history=8, gtol=1e-5, ftol=2.2e-9, fd_eps=1e-8):

@@ -517,6 +517,37 @@ __device__ __forceinline__ void predict_resume(const RealParams<P>& prm, const T
     *qvar = pvar;
 }
 
+// Conditional simulation, prior part (carma_simulate's sim_prior_kernel, the survey's condsim_prior_kernel): an
+// unconditional path of the noise-free process on the merged grid of data and requested times, drawn point by point
+// from the innovations form of the filter (kf built with prm.scale = 0).  Merged point k of path `path` uses the Philox
+// counters (seed, path, STREAM_CONDSIM, k, block).
+enum { STREAM_CONDSIM = 5 };
+
+// Draw f at the current merged point: returns f = mean + innov; rr * sn is a second, independent normal (the
+// measurement noise of a data point).
+template <int P>
+__device__ __forceinline__ double condsim_draw(const KalmanReal<P>& kf, unsigned long long seed, uint32_t path, uint32_t k,
+                                               uint32_t block, double* innov, double* rr, double* sn) {
+    double u0, u1;
+    uniforms2(seed, path, STREAM_CONDSIM, k, block, &u0, &u1);
+    *rr = sqrt(-2.0 * log(u0));
+    double cs;
+    sincos(6.283185307179586476925286766559 * u1, sn, &cs);
+    const double var = fmax(kf.var, 0.0);
+    *innov = sqrt(var) * *rr * cs;
+    return kf.mean + *innov;
+}
+
+// Condition on the drawn value and move to the next merged point, dt ahead.
+template <int P, class Tab>
+__device__ __forceinline__ void condsim_next(KalmanReal<P>& kf, const RealParams<P>& prm, const Tab& tb, double innov,
+                                             double dt) {
+    // a point that coincides with the previous one (var = 0) carries no new information
+    const double inv = kf.var > 1e-300 ? 1.0 / kf.var : 0.0;
+    kf.measurement_update(innov, inv);
+    kf.template predict_observe<false>(prm, tb, dt, 0.0);
+}
+
 // Exact (slow) evaluation of the log-likelihood of one theta: the same recursion with one log() per point.
 // Only reached when LogLikAcc::bad was raised (var not a positive normal number somewhere).
 template <int P, class Src, class Tab>

@@ -375,8 +375,6 @@ predict_real_kernel(SeriesView sv, ExplicitModel ex, const double* __restrict__ 
 // (O(nsim (ny + nsim))), and every path of a call is independent: one thread draws one prior path (innovations form
 // of the noise-free filter, as simulate_kernel), the conditional mean comes from the fast Predict above.
 // ---------------------------------------------------------------------------------------------
-enum { STREAM_CONDSIM = 5 };
-
 template <int P>
 __global__ void __launch_bounds__(64)
 sim_prior_kernel(ExplicitModel ex, double dt_max, int nm, const double* __restrict__ dtm /* nm: gap to next merged point */,
@@ -397,23 +395,12 @@ sim_prior_kernel(ExplicitModel ex, double dt_max, int nm, const double* __restri
     KalmanReal<P> kf;
     kf.reset(prm, 0.0);
     for (int k = 0; k < nm; k++) {
-        double u0, u1;
-        uniforms2(seed, (uint32_t)path, STREAM_CONDSIM, (uint32_t)k, 0u, &u0, &u1);
-        const double rr = sqrt(-2.0 * log(u0));
-        double sn, cs;
-        sincos(6.283185307179586476925286766559 * u1, &sn, &cs);
-        const double var = fmax(kf.var, 0.0);
-        const double innov = sqrt(var) * rr * cs;
-        const double f = kf.mean + innov;
+        double innov, rr, sn;
+        const double f = condsim_draw(kf, seed, (uint32_t)path, (uint32_t)k, 0u, &innov, &rr, &sn);
         const int id = idx[k];
         if (id >= 0) yres[(size_t)path * nyp + id] = (y[id] - mu) - f - sscale * yerr[id] * rr * sn;   // second normal: eps
         else fsim[(size_t)path * nsim + (-id - 1)] = f;
-        if (k + 1 < nm) {
-            // a point that coincides with the previous one (var = 0) carries no new information
-            const double inv = kf.var > 1e-300 ? 1.0 / kf.var : 0.0;
-            kf.measurement_update(innov, inv);
-            kf.template predict_observe<false>(prm, tb, dtm[k], 0.0);
-        }
+        if (k + 1 < nm) condsim_next(kf, prm, tb, innov, dtm[k]);
     }
 }
 

@@ -6,7 +6,9 @@
 //                              (the numeric part of CarmaSample.assess_fit_values) without sending them to the host;
 //   predict_forward_kernel<P>  one thread = one curve: the same recursion with a cursor over the curve's (time-sorted)
 //   predict_query_kernel<P>    queries, parking the state in front of each; then one thread = one query resumes from it
-//                              (predict_resume, shared with the single-series predict_real_kernel).
+//                              (predict_resume, shared with the single-series predict_real_kernel);
+//   condsim_prior_kernel<P>    one thread = one (curve, path): the prior draw of conditional simulation (Matheron's rule,
+//                              as carma_simulate); the two predict kernels then run on every path's residual data.
 #include <algorithm>
 #include <cmath>
 #include <cstdlib>
@@ -202,35 +204,53 @@ struct PredictRec {
     static constexpr int NT = P * (P + 1) / 2, SD = P + NT, R = SD + 3;
 };
 
-template <int P>
+// The paths one launch of the predict kernels serves when they are instantiated with PATHS = true, for conditional
+// simulation: paths j0 .. j0 + B - 1 of every curve; path jj filters its own residual-data row y + jj * ystride
+// (centred: mu = 0) with theta row c * rpc + j (rpc = npaths: one row per path) or c (rpc = 1), and the query pass adds
+// its mean to the prior draw already stored at path jj's destination jj * nq + perm[k].  Threads are path-minor (curve
+// c, path jj at c * B + jj; query k, path jj at k * B + jj), so the lanes of a warp walk the same curve and query and
+// share its trip counts.  PATHS = false is predict: one path, the curve's data, theta row c -- the index arithmetic
+// folds away and the kernels compile as they did before paths existed.
+struct PathSet {
+    unsigned B = 1, j0 = 0;
+    size_t ystride = 0, rpc = 1;
+    __device__ size_t theta_row(size_t c, unsigned jj) const { return c * rpc + (rpc > 1 ? j0 + jj : 0); }
+};
+
+template <int P, bool PATHS>
 __global__ void __launch_bounds__(SF_BLOCK)
 predict_forward_kernel(const double* __restrict__ dt, const double* __restrict__ y, const double* __restrict__ e2,
                        const long long* __restrict__ off, size_t ncurves, double dt_max, int kind, int q, int d,
                        unsigned flags, const carma_prior_t* __restrict__ priors, const double* __restrict__ theta,
-                       const long long* __restrict__ qoff, const double* __restrict__ qtq, double* __restrict__ rec,
-                       RealParams<P>* __restrict__ prm_out, int* __restrict__ status_out) {
+                       const long long* __restrict__ qoff, const double* __restrict__ qtq, PathSet ps,
+                       double* __restrict__ rec, RealParams<P>* __restrict__ prm_out, int* __restrict__ status_out) {
     using PR = PredictRec<P>;
     MathTab tb;
     tb.load();
-    const size_t c = (size_t)blockIdx.x * SF_BLOCK + threadIdx.x;
-    if (c >= ncurves) return;
+    const unsigned B = PATHS ? ps.B : 1u;
+    const size_t tid = (size_t)blockIdx.x * SF_BLOCK + threadIdx.x;
+    if (tid >= ncurves * B) return;
+    const size_t c = tid / B;
+    const unsigned jj = (unsigned)(tid - c * B);
     long long k = qoff[c];
     const long long k1 = qoff[c + 1];
     double th[MAX_D];
+    const size_t row = PATHS ? ps.theta_row(c, jj) : c;
 #pragma unroll
-    for (int j = 0; j < MAX_D; j++) th[j] = (j < d) ? theta[c * (size_t)d + j] : 0.0;
+    for (int j = 0; j < MAX_D; j++) th[j] = (j < d) ? theta[row * d + j] : 0.0;
     RealParams<P> prm;
     carma_prior_t pr = priors[c];
     const int status = transform_theta<P>(kind, q, flags, pr, th, dt_max, prm);
-    prm_out[c] = prm;        // the query threads of this curve read the constants from here
-    status_out[c] = status;
+    if (PATHS) prm.mu = 0.0;   // the residual data are centred
+    prm_out[tid] = prm;      // the query threads of this curve and path read the constants from here
+    status_out[tid] = status;
     if (status != TT_OK || k == k1) return;
     const long long o0 = off[c];
     const int ny = (int)(off[c + 1] - o0);
-    const double *cdt = dt + o0, *cy = y + o0, *cE = e2 + o0;
+    const double *cdt = dt + o0, *cy = y + (PATHS ? jj * ps.ystride : 0) + o0, *cE = e2 + o0;
     double t = 0.0;
     for (; k < k1 && !(qtq[k] > t); k++) {   // at or before the first point: ip = 0
-        double* r = rec + (size_t)k * PR::R;
+        double* r = rec + ((size_t)k * B + jj) * PR::R;
         r[PR::SD] = 0.0;
         r[PR::SD + 1] = fabs(t - qtq[k]);
         r[PR::SD + 2] = 0.0;
@@ -241,7 +261,7 @@ predict_forward_kernel(const double* __restrict__ dt, const double* __restrict__
         const bool last = i + 1 == ny;
         const double tn = last ? 0.0 : t + cdt[i];
         for (; k < k1 && (last || !(qtq[k] > tn)); k++) {   // t[i] < t* <= t[i+1], or past the last point
-            double* r = rec + (size_t)k * PR::R;
+            double* r = rec + ((size_t)k * B + jj) * PR::R;
 #pragma unroll
             for (int j = 0; j < P; j++) r[j] = kf.z[j];
 #pragma unroll
@@ -257,32 +277,99 @@ predict_forward_kernel(const double* __restrict__ dt, const double* __restrict__
     }
 }
 
-// Predict, query part: one thread per query (sorted curve-major, then by time, so a warp walks one curve), result
-// written to the caller's position perm[k].
-template <int P>
+// Predict, query part: one thread per query and path (queries sorted curve-major, then by time, so a warp walks one
+// curve), result written to the caller's position perm[k] of the path's row.
+template <int P, bool PATHS>
 __global__ void __launch_bounds__(SF_BLOCK)
 predict_query_kernel(const double* __restrict__ dt, const double* __restrict__ y, const double* __restrict__ e2,
                      const long long* __restrict__ off, const int* __restrict__ qcurve, const long long* __restrict__ perm,
-                     size_t nq, const double* __restrict__ rec, const RealParams<P>* __restrict__ prms,
-                     const int* __restrict__ status, double* __restrict__ qmean, double* __restrict__ qvar) {
+                     size_t nq, PathSet ps, const double* __restrict__ rec, const RealParams<P>* __restrict__ prms,
+                     const int* __restrict__ status, double* __restrict__ qmean, double* __restrict__ qvar /* may be null */) {
     using PR = PredictRec<P>;
     MathTab tb;
     tb.load();
-    const size_t k = (size_t)blockIdx.x * SF_BLOCK + threadIdx.x;
-    if (k >= nq) return;
+    const unsigned B = PATHS ? ps.B : 1u;
+    const size_t u = (size_t)blockIdx.x * SF_BLOCK + threadIdx.x;
+    if (u >= nq * B) return;
+    const size_t k = u / B;
+    const unsigned jj = (unsigned)(u - k * B);
     const int c = qcurve[k];
-    const long long dst = perm[k];
-    if (status[c] != TT_OK) { qmean[dst] = NAN; qvar[dst] = NAN; return; }
-    const RealParams<P> prm = prms[c];
-    const double* r = rec + k * PR::R;
+    const size_t cp = (size_t)c * B + jj;
+    const size_t dst = jj * nq + (size_t)perm[k];
+    if (status[cp] != TT_OK) { qmean[dst] = NAN; if (qvar) qvar[dst] = NAN; return; }
+    const RealParams<P> prm = prms[cp];
+    const double* r = rec + u * PR::R;
     const long long o0 = off[c];
     const int ny = (int)(off[c + 1] - o0);
+    const double* cy = y + (PATHS ? jj * ps.ystride : 0) + o0;
     double pm, pv;
     predict_resume<P>(prm, tb, r, r + P, (int)r[PR::SD + 2], ny, r[PR::SD], r[PR::SD + 1],
-                      [&](int i) { return y[o0 + i]; }, [&](int i) { return dt[o0 + i]; },
+                      [&](int i) { return cy[i]; }, [&](int i) { return dt[o0 + i]; },
                       [&](int i) { return e2[o0 + i]; }, &pm, &pv);
-    qmean[dst] = pm;
-    qvar[dst] = pv;
+    qmean[dst] = PATHS ? qmean[dst] + pm : pm;
+    if (qvar) qvar[dst] = pv;
+}
+
+// Conditional simulation, prior part: one thread per curve and path (path-minor, as PathSet).  The noise-free
+// innovations filter (condsim_draw / condsim_next, shared with carma_simulate's sim_prior_kernel) walks the curve's
+// merged grid: its data points and its time-sorted queries, a query equal to a data time after it, all on the curve's
+// own axis.  Merged point k of global path j uses the Philox counters (seed, j, STREAM_CONDSIM, k, curve_offset + c).
+// Writes the residual data (y - mu) - f - sqrt(scale) yerr eps of every point to the path's row yres + jj * ystride
+// (CSR layout) and f + mu of every query to out[jj * nq + perm[k]].  A rejected theta row gives NaN queries.
+template <int P>
+__global__ void __launch_bounds__(SF_BLOCK)
+condsim_prior_kernel(const double* __restrict__ dt, const double* __restrict__ y, const double* __restrict__ e2,
+                     const long long* __restrict__ off, size_t ncurves, double dt_max, int kind, int q, int d,
+                     unsigned flags, const carma_prior_t* __restrict__ priors, const double* __restrict__ theta,
+                     const long long* __restrict__ qoff, const double* __restrict__ qtq, const long long* __restrict__ perm,
+                     size_t nq, PathSet ps, unsigned long long seed, uint32_t curve_offset, double* __restrict__ yres,
+                     double* __restrict__ out) {
+    MathTab tb;
+    tb.load();
+    const size_t tid = (size_t)blockIdx.x * SF_BLOCK + threadIdx.x;
+    if (tid >= ncurves * ps.B) return;
+    const size_t c = tid / ps.B;
+    const unsigned jj = (unsigned)(tid - c * ps.B);
+    long long k = qoff[c];
+    const long long k1 = qoff[c + 1];
+    double* o = out + jj * nq;
+    double th[MAX_D];
+    const size_t row = ps.theta_row(c, jj);
+#pragma unroll
+    for (int j = 0; j < MAX_D; j++) th[j] = (j < d) ? theta[row * d + j] : 0.0;
+    RealParams<P> prm;
+    carma_prior_t pr = priors[c];
+    if (transform_theta<P>(kind, q, flags, pr, th, dt_max, prm) != TT_OK) {
+        for (; k < k1; k++) o[perm[k]] = NAN;
+        return;
+    }
+    const double mu = prm.mu, sscale = sqrt(prm.scale);
+    prm.scale = 0.0;   // the process itself carries no measurement noise
+    KalmanReal<P> kf;
+    kf.reset(prm, 0.0);
+    const long long o0 = off[c];
+    const int ny = (int)(off[c + 1] - o0);
+    const double *cdt = dt + o0, *cy = y + o0, *cE = e2 + o0;
+    double* res = yres + jj * ps.ystride + o0;
+    const uint32_t path = ps.j0 + jj, block = curve_offset + (uint32_t)c;
+    double td = 0.0, tprev = 0.0, innov = 0.0;   // time of data point i, of the previous merged point
+    int i = 0;
+    for (uint32_t km = 0; i < ny || k < k1; km++) {
+        const bool data = k == k1 || (i < ny && td <= qtq[k]);
+        const double tm = data ? td : qtq[k];
+        if (km > 0) condsim_next(kf, prm, tb, innov, tm - tprev);
+        double rr, sn;
+        const double f = condsim_draw(kf, seed, path, km, block, &innov, &rr, &sn);
+        if (data) {
+            res[i] = (cy[i] - mu) - f - sscale * sqrt(cE[i]) * rr * sn;   // second normal: the measurement noise
+            td += cdt[i];
+            i++;
+        } else {
+            o[perm[k]] = f + mu;
+            k++;
+        }
+        tprev = tm;
+    }
 }
 
 // ---- launchers ---------------------------------------------------------------------------------------------------
@@ -318,35 +405,77 @@ static cudaError_t launch_multi_filter(const carma_multi_series* m, int kind, in
     return cudaGetLastError();
 }
 
-template <int P>
+template <int P, bool PATHS>
 static cudaError_t launch_predict_p(const carma_multi_series* m, int kind, int q, unsigned flags, double dt_max,
-                                    const carma_prior_t* d_priors, const double* d_theta, const long long* d_qoff,
-                                    const double* d_qtq, const int* d_qcurve, const long long* d_perm, size_t nq,
-                                    double* d_rec, void* d_prm, int* d_status, double* d_qm, double* d_qv,
-                                    cudaStream_t st) {
+                                    const carma_prior_t* d_priors, const double* d_theta, const double* d_y,
+                                    const PathSet& ps, const long long* d_qoff, const double* d_qtq, const int* d_qcurve,
+                                    const long long* d_perm, size_t nq, double* d_rec, void* d_prm, int* d_status,
+                                    double* d_qm, double* d_qv, cudaStream_t st) {
     const int d = model_dim(kind, P, q);
-    predict_forward_kernel<P><<<(unsigned)((m->ncurves + SF_BLOCK - 1) / SF_BLOCK), SF_BLOCK, 0, st>>>(
-        m->d_dt, m->d_y, m->d_e2, m->d_off, m->ncurves, dt_max, kind, q, d, flags, d_priors, d_theta, d_qoff, d_qtq,
+    predict_forward_kernel<P, PATHS><<<(unsigned)((m->ncurves * ps.B + SF_BLOCK - 1) / SF_BLOCK), SF_BLOCK, 0, st>>>(
+        m->d_dt, d_y, m->d_e2, m->d_off, m->ncurves, dt_max, kind, q, d, flags, d_priors, d_theta, d_qoff, d_qtq, ps,
         d_rec, (RealParams<P>*)d_prm, d_status);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
-    predict_query_kernel<P><<<(unsigned)((nq + SF_BLOCK - 1) / SF_BLOCK), SF_BLOCK, 0, st>>>(
-        m->d_dt, m->d_y, m->d_e2, m->d_off, d_qcurve, d_perm, nq, d_rec, (const RealParams<P>*)d_prm, d_status, d_qm,
+    predict_query_kernel<P, PATHS><<<(unsigned)((nq * ps.B + SF_BLOCK - 1) / SF_BLOCK), SF_BLOCK, 0, st>>>(
+        m->d_dt, d_y, m->d_e2, m->d_off, d_qcurve, d_perm, nq, ps, d_rec, (const RealParams<P>*)d_prm, d_status, d_qm,
         d_qv);
     return cudaGetLastError();
 }
 
-// upload the priors (NULL: the population-variance defaults) and theta rows into the multi-series' scratch
+// one chunk of conditional-simulation paths: prior draws, then the predict kernels on their residual data
+template <int P>
+static cudaError_t launch_simulate_p(const carma_multi_series* m, int kind, int q, unsigned flags, double dt_max,
+                                     const carma_prior_t* d_priors, const double* d_theta, const PathSet& ps,
+                                     unsigned long long seed, uint32_t curve_offset, const long long* d_qoff,
+                                     const double* d_qtq, const int* d_qcurve, const long long* d_perm, size_t nq,
+                                     double* d_yres, double* d_rec, void* d_prm, int* d_status, double* d_out,
+                                     cudaStream_t st) {
+    const int d = model_dim(kind, P, q);
+    condsim_prior_kernel<P><<<(unsigned)((m->ncurves * ps.B + SF_BLOCK - 1) / SF_BLOCK), SF_BLOCK, 0, st>>>(
+        m->d_dt, m->d_y, m->d_e2, m->d_off, m->ncurves, dt_max, kind, q, d, flags, d_priors, d_theta, d_qoff, d_qtq,
+        d_perm, nq, ps, seed, curve_offset, d_yres, d_out);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    return launch_predict_p<P, true>(m, kind, q, flags, dt_max, d_priors, d_theta, d_yres, ps, d_qoff, d_qtq, d_qcurve, d_perm,
+                               nq, d_rec, d_prm, d_status, d_out, nullptr, st);
+}
+
+// upload the priors (NULL: the population-variance defaults) and `rows` theta rows into the multi-series' scratch
 static int upload_rows(carma_multi_series* m, int kind, int p, int q, const carma_prior_t* priors, const double* theta,
-                       cudaStream_t st) {
+                       size_t rows, cudaStream_t st) {
     const size_t d = (size_t)model_dim(kind, p, q), n = m->ncurves;
-    if (!m->scratch_in.reserve(n * d * sizeof(double)) || !m->scratch_pr.reserve(n * sizeof(carma_prior_t)))
+    if (!m->scratch_in.reserve(rows * d * sizeof(double)) || !m->scratch_pr.reserve(n * sizeof(carma_prior_t)))
         return CARMA_ERR_CUDA;
     const carma_prior_t* hp = priors ? priors : m->priors_pop.data();
     if (!cuda_ok(cudaMemcpyAsync(m->scratch_pr.p, hp, n * sizeof(carma_prior_t), cudaMemcpyHostToDevice, st), "H2D priors") ||
-        !cuda_ok(cudaMemcpyAsync(m->scratch_in.p, theta, n * d * sizeof(double), cudaMemcpyHostToDevice, st), "H2D theta"))
+        !cuda_ok(cudaMemcpyAsync(m->scratch_in.p, theta, rows * d * sizeof(double), cudaMemcpyHostToDevice, st), "H2D theta"))
         return CARMA_ERR_CUDA;
     return CARMA_OK;
+}
+
+// Sort every curve's queries by time, on the curve's own axis (t - t0[c]): perm[k] is the caller's position of sorted
+// query k, qtq its time on the axis, qcurve its curve.  Returns the rate clamp of the call, which must cover its longest
+// transition: the data gaps, forecasts past the last point and backcasts before the first.
+static double sort_queries(const carma_multi_series* m, const int64_t* q_offsets, const double* tq,
+                           std::vector<long long>& perm, std::vector<double>& qtq, std::vector<int>& qcurve) {
+    const size_t nc = m->ncurves, nq = (size_t)q_offsets[nc];
+    perm.resize(nq);
+    qtq.resize(nq);
+    qcurve.resize(nq);
+    double dt_max = m->dt_max;
+    for (size_t c = 0; c < nc; c++) {
+        const size_t k0 = (size_t)q_offsets[c], k1 = (size_t)q_offsets[c + 1];
+        std::iota(perm.begin() + k0, perm.begin() + k1, (long long)k0);
+        std::stable_sort(perm.begin() + k0, perm.begin() + k1, [&](long long a, long long b) { return tq[a] < tq[b]; });
+        const double tspan = m->info[c].tspan;
+        for (size_t k = k0; k < k1; k++) {
+            qtq[k] = tq[perm[k]] - m->t0[c];
+            qcurve[k] = (int)c;
+            dt_max = std::max(dt_max, std::max(qtq[k] - tspan, -qtq[k]));
+        }
+    }
+    return dt_max;
 }
 
 static size_t round32(size_t n) { return (n + 31) & ~(size_t)31; }   // doubles: keeps 256-byte alignment
@@ -376,7 +505,7 @@ static int multi_filter_to_scratch(carma_multi_series* m, int kind, int p, int q
     const size_t stride = round32(m->total);
     if (!m->scratch_pts.reserve(2 * stride * sizeof(double)) || !m->scratch_out.reserve(m->ncurves * sizeof(double)))
         return CARMA_ERR_CUDA;
-    int rc = upload_rows(m, kind, p, q, priors, theta, st);
+    int rc = upload_rows(m, kind, p, q, priors, theta, m->ncurves, st);
     if (rc) return rc;
     *d_mean = (double*)m->scratch_pts.p;
     *d_var = *d_mean + stride;
@@ -444,26 +573,13 @@ int carma_multi_predict(carma_multi_series_t m, int kind, int p, int q, const ca
     if (!tq || !qmean || !qvar) { set_error("carma_multi_predict: null argument"); return CARMA_ERR_ARG; }
     for (size_t k = 0; k < nq; k++)
         if (!std::isfinite(tq[k])) { set_error("carma_multi_predict: non-finite query time"); return CARMA_ERR_ARG; }
-    // sort every curve's queries by time, on the curve's own axis (t - t0[c]); the rate clamp must cover the longest
-    // transition of the call: the data gaps, forecasts past the last point and backcasts before the first
-    std::vector<long long> perm(nq);
-    std::vector<double> qtq(nq);
-    std::vector<int> qcurve(nq);
-    double dt_max = m->dt_max;
-    for (size_t c = 0; c < nc; c++) {
-        const size_t k0 = (size_t)q_offsets[c], k1 = (size_t)q_offsets[c + 1];
-        std::iota(perm.begin() + k0, perm.begin() + k1, (long long)k0);
-        std::stable_sort(perm.begin() + k0, perm.begin() + k1, [&](long long a, long long b) { return tq[a] < tq[b]; });
-        const double tspan = m->info[c].tspan;
-        for (size_t k = k0; k < k1; k++) {
-            qtq[k] = tq[perm[k]] - m->t0[c];
-            qcurve[k] = (int)c;
-            dt_max = std::max(dt_max, std::max(qtq[k] - tspan, -qtq[k]));
-        }
-    }
+    std::vector<long long> perm;
+    std::vector<double> qtq;
+    std::vector<int> qcurve;
+    const double dt_max = sort_queries(m, q_offsets, tq, perm, qtq, qcurve);
     if (!cuda_ok(cudaSetDevice(m->device), "cudaSetDevice")) return CARMA_ERR_CUDA;
     cudaStream_t st = 0;
-    int rc = upload_rows(m, kind, p, q, priors, theta, st);
+    int rc = upload_rows(m, kind, p, q, priors, theta, nc, st);
     if (rc) return rc;
     // scratch_q: records | qtq | qm | qv | perm | qoff | prm | status | qcurve, each on a 256-byte boundary
     const size_t R = (size_t)(p + p * (p + 1) / 2 + 3);
@@ -487,8 +603,8 @@ int carma_multi_predict(carma_multi_series_t m, int kind, int p, int q, const ca
     const carma_prior_t* d_pr = (const carma_prior_t*)m->scratch_pr.p;
     const double* d_th = (const double*)m->scratch_in.p;
     cudaError_t e;
-#define LAUNCH_PQ(PP) e = launch_predict_p<PP>(m, kind, q, flags, dt_max, d_pr, d_th, d_qoff, d_qtq, d_qcurve, d_perm, nq, \
-                                                d_rec, d_prm, d_status, d_qm, d_qv, st)
+#define LAUNCH_PQ(PP) e = launch_predict_p<PP, false>(m, kind, q, flags, dt_max, d_pr, d_th, m->d_y, PathSet{}, d_qoff, d_qtq, \
+                                                d_qcurve, d_perm, nq, d_rec, d_prm, d_status, d_qm, d_qv, st)
     switch (p) {
         case 1: LAUNCH_PQ(1); break;
         case 2: LAUNCH_PQ(2); break;
@@ -504,6 +620,94 @@ int carma_multi_predict(carma_multi_series_t m, int kind, int p, int q, const ca
         !cuda_ok(cudaMemcpyAsync(qvar, d_qv, nq * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H qvar") ||
         !cuda_ok(cudaStreamSynchronize(st), "multi_predict sync"))
         return CARMA_ERR_CUDA;
+    return CARMA_OK;
+}
+
+int carma_multi_simulate(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* priors,
+                         const double* theta, size_t theta_rows, unsigned flags, const int64_t* s_offsets,
+                         const double* tsim, size_t npaths, uint64_t seed, uint32_t curve_offset, double* ysim) {
+    if (s_offsets && s_offsets[0] != 0) { set_error("carma_multi_simulate: s_offsets must start at 0"); return CARMA_ERR_ARG; }
+    if (!m || !theta || !s_offsets) { set_error("carma_multi_simulate: null argument"); return CARMA_ERR_ARG; }
+    if (!valid_model(kind, p, q)) { set_error("carma_multi_simulate: invalid (kind,p,q)"); return CARMA_ERR_ARG; }
+    const size_t nc = m->ncurves;
+    for (size_t c = 0; c < nc; c++)
+        if (s_offsets[c + 1] < s_offsets[c]) { set_error("carma_multi_simulate: s_offsets must be non-decreasing"); return CARMA_ERR_ARG; }
+    const size_t nq = (size_t)s_offsets[nc];
+    if (npaths == 0 || nq == 0) return CARMA_OK;
+    if (!tsim || !ysim) { set_error("carma_multi_simulate: null argument"); return CARMA_ERR_ARG; }
+    if (theta_rows != nc && theta_rows != nc * npaths) {
+        set_error("carma_multi_simulate: theta_rows must be ncurves or ncurves * npaths");
+        return CARMA_ERR_ARG;
+    }
+    if ((uint64_t)curve_offset + nc > ((uint64_t)1 << 32) || (uint64_t)npaths > ((uint64_t)1 << 32)) {
+        set_error("carma_multi_simulate: curve_offset + ncurves and npaths must not exceed 2^32 (32-bit Philox counters)");
+        return CARMA_ERR_ARG;
+    }
+    for (size_t k = 0; k < nq; k++)
+        if (!std::isfinite(tsim[k])) { set_error("carma_multi_simulate: non-finite time"); return CARMA_ERR_ARG; }
+    std::vector<long long> perm;
+    std::vector<double> qtq;
+    std::vector<int> qcurve;
+    const double dt_max = sort_queries(m, s_offsets, tsim, perm, qtq, qcurve);
+    if (!cuda_ok(cudaSetDevice(m->device), "cudaSetDevice")) return CARMA_ERR_CUDA;
+    cudaStream_t st = 0;
+    int rc = upload_rows(m, kind, p, q, priors, theta, theta_rows, st);
+    if (rc) return rc;
+    // Paths go in chunks of B whose scratch fits the budget (CARMA_MULTI_SIMULATE_BUDGET bytes, read at every call so
+    // that a test can force several chunks): per path a residual-data row, the query records, the output row and the
+    // constants of every curve.  A draw depends only on its curve, path and theta row, so chunking changes no bit.
+    const size_t R = (size_t)(p + p * (p + 1) / 2 + 3), ystride = round32(m->total);
+    const size_t prm_d = (sizeof(RealParams<MAX_P>) + 7) / 8;
+    const size_t per_path = ystride + nq * (R + 1) + nc * (prm_d + 1);
+    size_t budget = (size_t)4 << 30;
+    if (const char* env = getenv("CARMA_MULTI_SIMULATE_BUDGET")) budget = (size_t)std::strtoull(env, nullptr, 10);
+    const size_t B = std::max<size_t>(1, std::min(npaths, budget / (per_path * sizeof(double))));
+    // scratch_pts: B residual-data rows; scratch_q: records | out | qtq | perm | qoff | prm | status | qcurve
+    const size_t b_rec = round32(nq * B * R), b_out = round32(nq * B), b_q = round32(nq), b_off = round32(nc + 1),
+                 b_prm = round32(nc * B * prm_d), b_st = round32((nc * B + 1) / 2), b_qc = round32((nq + 1) / 2);
+    if (!m->scratch_pts.reserve(B * ystride * sizeof(double)) ||
+        !m->scratch_q.reserve((b_rec + b_out + 2 * b_q + b_off + b_prm + b_st + b_qc) * sizeof(double)))
+        return CARMA_ERR_CUDA;
+    double* d_yres = (double*)m->scratch_pts.p;
+    double* d_rec = (double*)m->scratch_q.p;
+    double* d_out = d_rec + b_rec;
+    double* d_qtq = d_out + b_out;
+    long long* d_perm = (long long*)(d_qtq + b_q);
+    long long* d_qoff = (long long*)((double*)d_perm + b_q);
+    void* d_prm = (double*)d_qoff + b_off;
+    int* d_status = (int*)((double*)d_prm + b_prm);
+    int* d_qcurve = (int*)((double*)d_status + b_st);
+    bool ok = cuda_ok(cudaMemcpyAsync(d_qtq, qtq.data(), nq * sizeof(double), cudaMemcpyHostToDevice, st), "H2D tsim") &&
+              cuda_ok(cudaMemcpyAsync(d_perm, perm.data(), nq * sizeof(long long), cudaMemcpyHostToDevice, st), "H2D perm") &&
+              cuda_ok(cudaMemcpyAsync(d_qoff, s_offsets, (nc + 1) * sizeof(long long), cudaMemcpyHostToDevice, st), "H2D s_offsets") &&
+              cuda_ok(cudaMemcpyAsync(d_qcurve, qcurve.data(), nq * sizeof(int), cudaMemcpyHostToDevice, st), "H2D qcurve");
+    if (!ok) return CARMA_ERR_CUDA;
+    const carma_prior_t* d_pr = (const carma_prior_t*)m->scratch_pr.p;
+    const double* d_th = (const double*)m->scratch_in.p;
+    for (size_t j0 = 0; j0 < npaths; j0 += B) {
+        PathSet ps;
+        ps.B = (unsigned)std::min(B, npaths - j0);
+        ps.j0 = (unsigned)j0;
+        ps.ystride = ystride;
+        ps.rpc = theta_rows / nc;
+        cudaError_t e;
+#define LAUNCH_SIM(PP) e = launch_simulate_p<PP>(m, kind, q, flags, dt_max, d_pr, d_th, ps, seed, curve_offset, d_qoff, d_qtq, \
+                                                 d_qcurve, d_perm, nq, d_yres, d_rec, d_prm, d_status, d_out, st)
+        switch (p) {
+            case 1: LAUNCH_SIM(1); break;
+            case 2: LAUNCH_SIM(2); break;
+            case 3: LAUNCH_SIM(3); break;
+            case 4: LAUNCH_SIM(4); break;
+            case 5: LAUNCH_SIM(5); break;
+            case 6: LAUNCH_SIM(6); break;
+            default: LAUNCH_SIM(7); break;
+        }
+#undef LAUNCH_SIM
+        if (!cuda_ok(e, "simulate kernels launch")) return CARMA_ERR_CUDA;
+        if (!cuda_ok(cudaMemcpyAsync(ysim + j0 * nq, d_out, ps.B * nq * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H ysim"))
+            return CARMA_ERR_CUDA;
+    }
+    if (!cuda_ok(cudaStreamSynchronize(st), "multi_simulate sync")) return CARMA_ERR_CUDA;
     return CARMA_OK;
 }
 

@@ -255,6 +255,22 @@ int carma_multi_assess_fit(carma_multi_series_t m, int kind, int p, int q, const
 int carma_multi_predict(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* priors,
                         const double* theta, unsigned flags, const int64_t* q_offsets, const double* tq, double* qmean,
                         double* qvar);
+/* KalmanFilter<>::Simulate (src/include/kfilter.hpp:135-184) of every curve of a multi-series at its own times, npaths
+ * paths per curve, by Matheron's rule as carma_simulate: a draw of the noise-free process at the requested times given
+ * the curve's data.  s_offsets (ncurves+1, CSR) and tsim as carma_multi_predict: absolute times, any order, possibly
+ * repeated or equal to data times (a requested time equal to a data time follows it on the curve's own axis).
+ * theta_rows = ncurves: every path of curve c uses row c; theta_rows = ncurves * npaths: path j of curve c uses row
+ * c * npaths + j (posterior predictive: one posterior sample per path).  priors and flags as carma_multi_predict.
+ * ysim[path * nsim_total + k] in the caller's order of tsim, mu included.  Draw (curve c, path j) uses the Philox
+ * counters of carma_simulate's path j with block word curve_offset + c (0 in carma_simulate): curve c equals a one-curve
+ * multi-series of that curve called with curve_offset = c, and path j does not depend on npaths.  A theta row the
+ * transform rejects gives NaN for its curve (or path).  npaths == 0 or no times: a no-op.  Blocking; uses the
+ * multi-series' scratch (one call per handle at a time).  Paths run in chunks of B whose scratch stays within 4 GiB:
+ * peak scratch B * (8 round32(total) + 8 nsim_total (p + p(p+1)/2 + 4) + ncurves (sizeof constants + 4)) bytes plus
+ * 20 nsim_total + 8 (ncurves + 1) for the sorted times, plus the theta rows and priors. */
+int carma_multi_simulate(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* priors,
+                         const double* theta, size_t theta_rows, unsigned flags, const int64_t* s_offsets,
+                         const double* tsim, size_t npaths, uint64_t seed, uint32_t curve_offset, double* ysim);
 
 /* ---- one very long light curve: temporally parallel (associative-scan) form of the same LogDensity ----
  * Replaces the strictly sequential Filter() loop (src/include/kfilter.hpp:126-132) when there is a single
