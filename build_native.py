@@ -21,7 +21,7 @@ CSRC = os.path.join(HERE, "csrc")
 NVCC = os.environ.get("NVCC") or shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
 CXX = os.environ.get("CXX_HOST") or shutil.which("g++") or "g++"
 
-CUDA_SOURCES = ["loglik.cu", "mcmc.cu", "scan.cu", "sim.cu", "mle.cu", "mle_dev.cu", "comm.cu", "survey.cu"]
+CUDA_SOURCES = ["loglik.cu", "mcmc.cu", "scan.cu", "sim.cu", "mle.cu", "mle_dev.cu", "comm.cu", "survey.cu", "posterior.cu"]
 CUDA_HEADERS = ["device_math.cuh", "fast_math.cuh", "theta_transform.cuh", "kalman_real.cuh", "kalman_cplx.cuh", "series.h",
                 os.path.join(ROOT, "include", "carma_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

@@ -8,9 +8,9 @@ from . import _lib
 from ._lib import (CarmaError, Series, MultiSeries, Prior, PTOpts, KIND_CAR1, KIND_CARP, KIND_CARMA, KIND_ZCAR,
                    KIND_ZCARMA, IGNORE_BOUNDS, LOGLIK_ONLY, model_dim)
 from .synth import get_ar_roots, carma_variance, carma_process, car1_process, power_spectrum
-from .carma_pack import CarmaModel, CarmaSample, Car1Sample, MCMCSample, batched_lbfgs
+from .carma_pack import CarmaModel, CarmaSample, Car1Sample, MCMCSample, SurveySample, batched_lbfgs
 
 __all__ = ["CarmaError", "Series", "MultiSeries", "Prior", "PTOpts", "KIND_CAR1", "KIND_CARP", "KIND_CARMA",
            "KIND_ZCAR", "KIND_ZCARMA", "IGNORE_BOUNDS", "LOGLIK_ONLY", "model_dim", "get_ar_roots",
            "carma_variance", "carma_process", "car1_process", "power_spectrum", "CarmaModel", "CarmaSample",
-           "Car1Sample", "MCMCSample", "batched_lbfgs"]
+           "Car1Sample", "MCMCSample", "SurveySample", "batched_lbfgs"]

@@ -54,7 +54,8 @@ EXPORTED_SYMBOLS = [
     "carma_gather_summaries", "carma_gather_summaries_dev", "carma_derived_params", "carma_derived_params_dev", "carma_mle_batch_device",
     "carma_mle_grid_device", "carma_multi_series_curve_stats", "carma_multi_mle_grid_device",
     "carma_multi_filter_dev", "carma_multi_filter", "carma_multi_assess_fit", "carma_multi_predict",
-    "carma_multi_simulate",
+    "carma_multi_simulate", "carma_psd_quantiles", "carma_psd_quantiles_dev", "carma_effective_samples",
+    "carma_effective_samples_dev",
 ]
 
 
@@ -191,6 +192,12 @@ def _load():
                                        ctypes.c_uint32, ctypes.c_int, _dp, _dp]
     L.carma_derived_params.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_void_p, _sz, _dp, _dp, ctypes.c_int]
     L.carma_derived_params_dev.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_void_p, _sz, _vp, _vp, _vp]
+    L.carma_psd_quantiles.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp, _sz, _sz, _vp, _vp, _sz, _sz, _vp, _sz,
+                                      _vp, _vp, ctypes.c_int]
+    L.carma_psd_quantiles_dev.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp, _sz, _sz, _vp, _vp, _sz, _sz, _vp,
+                                          _sz, _vp, _vp, _vp]
+    L.carma_effective_samples.argtypes = [_sz, _sz, _sz, _vp, _vp, ctypes.c_int]
+    L.carma_effective_samples_dev.argtypes = [_sz, _sz, _sz, _vp, _vp, _vp]
     L.carma_comm_unique_id.argtypes = [ctypes.c_char_p]
     L.carma_comm_init_rank.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_char_p, ctypes.c_int, ctypes.POINTER(ctypes.c_void_p)]
     L.carma_comm_destroy.argtypes = [_vp]
@@ -248,6 +255,54 @@ def derived_params(kind, p, q, theta, prior=None, device=0):
     return {"ar_roots": out[:, 0:2 * p:2] + 1j * out[:, 1:2 * p:2], "ar_coefs": out[:, 2 * p:3 * p + 1].copy(),
             "ma_coefs": out[:, 3 * p + 1:4 * p + 1].copy(), "sigma": out[:, 4 * p + 1].copy(),
             "psd_width": out[:, 4 * p + 2:5 * p + 2].copy(), "psd_centroid": out[:, 5 * p + 2:6 * p + 2].copy()}
+
+
+def psd_quantiles(kind, p, q, theta, freq, percentiles, priors=None, return_psd=False, device=0):
+    """Pointwise percentiles of the power spectrum over each curve's samples (carma_psd_quantiles).  theta (ncurves,
+    nsamples, d); freq (nfreq,) shared by every curve or (ncurves, nfreq); percentiles in [0, 100]; priors: ncurves
+    entries of PRIOR_DTYPE (only the kappa bounds are read; required for ZCARMA).  Returns out (ncurves, npct, nfreq),
+    bitwise np.percentile(psd, percentiles, axis=1) of the kernel's PSD values, and with return_psd=True also those
+    values, psd (ncurves, nsamples, nfreq)."""
+    th = np.ascontiguousarray(theta, dtype=np.float64)
+    d = model_dim(kind, p, q)
+    if th.ndim != 3 or th.shape[2] != d:
+        raise ValueError("theta must be (ncurves, nsamples, %d)" % d)
+    nc, ns = th.shape[0], th.shape[1]
+    fr = _c(freq)
+    if fr.ndim == 1:
+        rows = 1
+    elif fr.ndim == 2 and fr.shape[0] == nc:
+        rows = nc
+    else:
+        raise ValueError("freq must be (nfreq,) or (%d, nfreq)" % nc)
+    nf = fr.shape[-1]
+    pct = _c(np.atleast_1d(percentiles))
+    if pct.ndim != 1:
+        raise ValueError("percentiles must be a scalar or a 1-d sequence")
+    pp = None
+    if priors is not None:
+        priors = np.ascontiguousarray(priors, dtype=PRIOR_DTYPE)
+        if priors.shape != (nc,):
+            raise ValueError("priors must have %d entries" % nc)
+        pp = priors.ctypes.data
+    out = np.empty((nc, pct.size, nf))
+    psd = np.empty((nc, ns, nf)) if return_psd else None
+    check(lib.carma_psd_quantiles(kind, p, q, pp, nc, ns, th.ctypes.data, fr.ctypes.data, rows, nf, pct.ctypes.data,
+                                  pct.size, out.ctypes.data, psd.ctypes.data if return_psd else None, device),
+          "carma_psd_quantiles")
+    return (out, psd) if return_psd else out
+
+
+def effective_samples(x, device=0):
+    """MCMCSample.effective_samples for every column of every series (carma_effective_samples): x (nseries, n, k) ->
+    ess (nseries, k)."""
+    xs = np.ascontiguousarray(x, dtype=np.float64)
+    if xs.ndim != 3:
+        raise ValueError("x must be (nseries, n, k)")
+    ns, n, k = xs.shape
+    ess = np.empty((ns, k))
+    check(lib.carma_effective_samples(ns, n, k, xs.ctypes.data, ess.ctypes.data, device), "carma_effective_samples")
+    return ess
 
 
 class Series:
@@ -557,6 +612,14 @@ class MultiSeries:
         check(lib.carma_multi_pt_run(self.handle, kind, p, q, pp, ctypes.byref(o), n_ensembles, samples.ctypes.data,
                                      logposts.ctypes.data, acc.ctypes.data, xr.ctypes.data), "carma_multi_pt_run")
         return dict(samples=samples, logposts=logposts, accept_rates=acc, exchange_rates=xr)
+
+    def run_mcmc(self, p, q, nsamples, nburnin=None, ntemperatures=None, nthin=1, seed=None, n_ensembles=1, priors=None):
+        """CarmaModel.run_mcmc for every curve in one launch (carma_multi_pt_run), with the same defaults: curve c with
+        the same seed gives what CarmaModel(curve c).run_mcmc gives when it is curve 0.  Returns a SurveySample (see
+        carma_pack.survey_run_mcmc)."""
+        from .carma_pack import survey_run_mcmc
+        return survey_run_mcmc(self, p, q, nsamples, nburnin=nburnin, ntemperatures=ntemperatures, nthin=nthin, seed=seed,
+                               n_ensembles=n_ensembles, priors=priors)
 
     def curve_stats(self):
         """Per-curve statistics (structured array, CURVE_STATS_DTYPE): y_mean, y_var_pop, y_var_sample, min_dt,

@@ -497,6 +497,147 @@ def survey_choose_order(ms, pmax, qmax=None, pqlist=None, ntrials=100, seed=None
     return best_pq, pqlist, table, mles
 
 
+def survey_run_mcmc(ms, p, q, nsamples, nburnin=None, ntemperatures=None, nthin=1, seed=None, n_ensembles=1, priors=None):
+    """CarmaModel.run_mcmc for every light curve of the multi-series `ms` (MultiSeries.run_mcmc): the same defaults
+    (ntemperatures = max(10, p + q), one chain for p = 1, nburnin = nsamples // 2, population-variance priors), all
+    curves in one carma_multi_pt_run launch.  Returns a SurveySample."""
+    if not p > q:
+        raise ValueError("Order of AR polynomial, p, must be larger than order of MA polynomial, q.")
+    if ntemperatures is None:
+        ntemperatures = max(10, p + q)
+    if nburnin is None:
+        nburnin = nsamples // 2
+    if seed is None:
+        seed = int(np.random.SeedSequence().generate_state(1, dtype=np.uint64)[0])
+    if p == 1:
+        ntemperatures = 1  # run_mcmc_car1 has a single chain (carmcmc.cpp:30-77)
+    kind = _kind_for(p, q)
+    if priors is None:
+        priors = ms.default_priors(population_var=True)  # carmcmc.cpp:85-89
+    res = ms.pt_run(kind, p, q, int(nsamples), int(nburnin), thin=int(nthin), ntemps=int(ntemperatures),
+                    n_ensembles=int(n_ensembles), seed=seed, priors=priors)
+    nc, d = ms.ncurves, model_dim(kind, p, q)
+    sample = SurveySample(res["samples"].reshape(nc, -1, d), res["logposts"].reshape(nc, -1), p, q, kind=kind,
+                          priors=priors, stats=ms.curve_stats(), multi_series=ms)
+    sample.accept_rates = res["accept_rates"]
+    sample.exchange_rates = res["exchange_rates"]
+    return sample
+
+
+class SurveySample(object):
+    """The posterior samples of every curve of a survey (MultiSeries.run_mcmc): what CarmaSample / Car1Sample give for
+    one curve, as per-curve arrays.  trace (ncurves, nsamples, d) with the ensembles of a curve one after the other, as
+    CarmaModel.run_mcmc concatenates them; logpost (ncurves, nsamples).  Derived parameters come from one device launch
+    over the whole trace, made when one is first asked for; the power-spectrum band and the effective sample sizes run
+    on the device without the per-sample arrays crossing PCIe.  stats: MultiSeries.curve_stats() (the default frequency
+    grid); priors: PRIOR_DTYPE per curve; multi_series: the survey the trace came from (for curve())."""
+
+    _DERIVED = ("ar_roots", "psd_width", "psd_centroid", "ar_coefs", "ma_coefs", "sigma")
+
+    def __init__(self, trace, logpost, p, q, kind=None, priors=None, stats=None, multi_series=None):
+        self.trace = np.asarray(trace, dtype=float)
+        self.logpost = np.asarray(logpost, dtype=float)
+        if self.trace.ndim != 3 or self.logpost.shape != self.trace.shape[:2]:
+            raise ValueError("trace must be (ncurves, nsamples, d) and logpost (ncurves, nsamples)")
+        self.p, self.q = p, q
+        self.kind = _kind_for(p, q) if kind is None else kind
+        if self.trace.shape[2] != model_dim(self.kind, p, q):
+            raise ValueError("trace rows must have %d entries for this model" % model_dim(self.kind, p, q))
+        self.ncurves, self.nsamples = self.trace.shape[:2]
+        self.priors, self.stats, self.multi_series = priors, stats, multi_series
+        self._derived = None
+
+    def _prior_struct(self, c):
+        return None if self.priors is None else _lib.Prior(*[float(v) for v in self.priors[c]])
+
+    def _derive(self):
+        if self._derived is None:
+            if self.kind == KIND_ZCARMA:
+                raise ValueError("derived parameters of a ZCARMA survey need per-curve kappa bounds; use curve()")
+            der = _lib.derived_params(self.kind, self.p, self.q, self.trace.reshape(-1, self.trace.shape[2]))
+            shape = (self.ncurves, self.nsamples)
+            self._derived = {k: v.reshape(shape + v.shape[1:]) for k, v in der.items()}
+            self._derived["ma_coefs"] = self._derived["ma_coefs"][:, :, :self.q + 1]
+        return self._derived
+
+    def get_samples(self, name):
+        """The CarmaSample / Car1Sample entry `name` of every curve: (ncurves, nsamples) for scalars, (ncurves,
+        nsamples, k) for vectors."""
+        th = self.trace
+        if name == "var":
+            return th[:, :, 0] ** 2
+        if name == "measerr_scale":
+            return th[:, :, 1].copy()
+        if name == "mu":
+            return th[:, :, 2].copy()
+        if name in ("loglik", "logpost"):
+            return self.logpost.copy()
+        if name == "loglik_only":
+            return self.logpost - CarmaSample.log_prior(th.reshape(-1, th.shape[2])).reshape(self.logpost.shape)
+        if self.p == 1 and self.kind == KIND_CAR1:
+            if name == "log_omega":
+                return th[:, :, 3].copy()
+            if name == "sigma":   # Car1Sample: sqrt(2 omega var)
+                return np.sqrt(2.0 * np.exp(th[:, :, 3]) * th[:, :, 0] ** 2)
+        elif name == "quad_coefs":
+            return np.exp(th[:, :, 3:3 + self.p])
+        if name in self._DERIVED and not (self.kind == KIND_CAR1 and name in ("ar_coefs", "ma_coefs")):
+            return self._derive()[name].copy()
+        raise KeyError(name)
+
+    def best_index(self):
+        """Index of the largest log-posterior of every curve (ncurves,): CarmaSample.best_index per curve."""
+        return np.argmax(self.logpost, axis=1)
+
+    def map_theta(self):
+        """The maximum-a-posteriori theta row of every curve (ncurves, d), the input of MultiSeries.predict /
+        kalman_filter / conditional_simulate."""
+        return self.trace[np.arange(self.ncurves), self.best_index()].copy()
+
+    def DIC(self):
+        """CarmaSample.DIC of every curve (ncurves,) (carma_pack.py:808-828)."""
+        ll = self.logpost
+        return -2.0 * ll.mean(axis=1) + 2.0 * np.var(-2.0 * ll, axis=1) / 2.0
+
+    def effective_samples(self, name):
+        """MCMCSample.effective_samples of `name` (a real-valued entry) for every curve, on the device: (ncurves, k)."""
+        x = np.asarray(self.get_samples(name))
+        if np.iscomplexobj(x):
+            raise ValueError("effective_samples needs a real-valued entry, %r is complex" % name)
+        if x.ndim == 2:
+            x = x[:, :, None]
+        return _lib.effective_samples(x)
+
+    def default_freq(self):
+        """CarmaSample's frequency grid of every curve (ncurves, 200): 200 log-spaced points from 1 / tspan to
+        0.5 / min_dt."""
+        if self.stats is None:
+            raise ValueError("the default frequency grid needs the curve statistics (MultiSeries.curve_stats())")
+        lo = np.log10(1.0 / np.asarray(self.stats["tspan"], dtype=float))
+        hi = np.log10(0.5 / np.asarray(self.stats["min_dt"], dtype=float))
+        return np.stack([np.logspace(a, b, 200) for a, b in zip(lo, hi)])
+
+    def psd_credible_band(self, percentile=68.0, freq=None):
+        """CarmaSample.psd_credible_band of every curve over all its samples (slice the trace for a subset), on the
+        device (carma_psd_quantiles).  freq: None (CarmaSample's grid per curve), (nfreq,) or (ncurves, nfreq).
+        Returns (psd_lo, psd_hi, psd_mid, freq), each (ncurves, nfreq)."""
+        freq = self.default_freq() if freq is None else np.asarray(freq, dtype=float)
+        lo, hi = (100.0 - percentile) / 2.0, 100.0 - (100.0 - percentile) / 2.0
+        out = _lib.psd_quantiles(self.kind, self.p, self.q, self.trace, freq, [lo, hi, 50.0], priors=self.priors)
+        freq = np.broadcast_to(freq, (self.ncurves, freq.shape[-1])).copy()
+        return out[:, 0], out[:, 1], out[:, 2], freq
+
+    def curve(self, c):
+        """The CarmaSample (Car1Sample for p = 1) of curve c, built from the same arrays: the bridge to per-curve code."""
+        if self.multi_series is None:
+            raise ValueError("curve() needs the multi-series the samples came from")
+        t, y, e = self.multi_series.curve(c)
+        if self.kind == KIND_CAR1:
+            return Car1Sample(t, y, e, trace=self.trace[c], logpost=self.logpost[c], prior=self._prior_struct(c))
+        return CarmaSample(t, y, e, trace=self.trace[c], logpost=self.logpost[c], p=self.p, q=self.q,
+                           prior=self._prior_struct(c))
+
+
 class MCMCSample(object):
     """Dictionary of traces (subset of src/carmcmc/samplers.py:13-408 without the plots)."""
 

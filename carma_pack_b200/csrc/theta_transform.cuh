@@ -598,4 +598,69 @@ __host__ __device__ __forceinline__ int explicit_constants(const ExplicitModel& 
     return st;
 }
 
+// One theta row -> AR roots w, MA coefficients ma (beta_0 = 1, zero beyond q; ZCARMA: binomial / kappa^i) and sigma^2 of
+// the driving noise, with the formulas of CarmaSample._ar_roots / _ma_coefs / _sigma_noise (Car1Sample for CAR(1):
+// sigma^2 = 2 omega var) and IEEE division throughout.  pr: only the kappa bounds are read (ZCARMA).  AR_POLY: also the
+// AR polynomial prod (x - w_k), highest power first (numpy.poly), into ac[P + 1].  Shared by derived_params_kernel
+// (loglik.cu) and the PSD kernels (posterior.cu).
+template <int P, bool AR_POLY = false>
+__device__ __forceinline__ double derive_row(int kind, int q, const carma_prior_t& pr, const double* th, cxd* w, double* ma,
+                                             cxd* ac = nullptr) {
+    if (kind == CARMA_KIND_CAR1) w[0] = cx(-exp(th[3]), 0.0);
+    else quad_roots_dev<P>(th + 3, P, w);
+    if (AR_POLY) {
+        ac[0] = cx(1.0, 0.0);
+#pragma unroll
+        for (int i = 1; i <= P; i++) ac[i] = cx(0.0, 0.0);
+#pragma unroll
+        for (int i = 0; i < P; i++)
+#pragma unroll
+            for (int j = P; j >= 1; j--)
+                if (j <= i + 1) ac[j] = ac[j] - w[i] * ac[j - 1];
+    }
+    // MA coefficients (carpack.cpp:522-580, 687-698)
+#pragma unroll
+    for (int i = 0; i < P; i++) ma[i] = (i == 0) ? 1.0 : 0.0;
+    if (kind == CARMA_KIND_CARMA && q > 0) {
+        cxd rt[P], cf[P];
+#pragma unroll
+        for (int i = 0; i < P; i++) { rt[i] = cx(0, 0); cf[i] = cx(0, 0); }
+        quad_roots_dev<P>(th + 3 + P, q, rt);
+        cf[0] = cx(1.0, 0.0);
+        for (int i = 0; i < q; i++)
+            for (int j = i + 1; j >= 1; j--) cf[j] = cf[j] - rt[i] * cf[j - 1];
+        const double norm = cf[q].re;
+        for (int i = 0; i <= q; i++) ma[i] = cf[q - i].re / norm;
+    } else if (kind == CARMA_KIND_ZCARMA) {
+        const double x = th[3 + P];
+        const double kn = exp(x) / (1.0 + exp(x));
+        const double kappa = (pr.kappa_high - pr.kappa_low) * kn + pr.kappa_low;
+        double binom = 1.0;
+#pragma unroll
+        for (int i = 1; i < P; i++) {
+            binom = binom * (double)(P - i) / (double)i;
+            ma[i] = rint(binom) / pow(kappa, (double)i);
+        }
+    }
+    // Variance(w, beta, sigma = 1) (carpack.cpp:377-409) -> sigma^2 = var / Variance
+    cxd var_acc = cx(0, 0);
+#pragma unroll
+    for (int k = 0; k < P; k++) {
+        cxd s1 = cx(ma[P - 1], 0), s2 = cx(ma[P - 1], 0);
+        const cxd mw = -w[k];
+#pragma unroll
+        for (int l = P - 2; l >= 0; l--) {
+            s1 = s1 * w[k] + cx(ma[l], 0);
+            s2 = s2 * mw + cx(ma[l], 0);
+        }
+        cxd dp = cx(1, 0);
+#pragma unroll
+        for (int l = 0; l < P; l++)
+            if (l != k) dp = dp * ((w[l] - w[k]) * (conj(w[l]) + w[k]));
+        var_acc = var_acc + cdiv(s1 * s2, (-2.0 * w[k].re) * dp);
+    }
+    const double ysigma = th[0];
+    return (kind == CARMA_KIND_CAR1) ? 2.0 * ysigma * ysigma * (-w[0].re) : ysigma * ysigma / var_acc.re;
+}
+
 }  // namespace carma

@@ -130,6 +130,33 @@ int carma_derived_params(int kind, int p, int q, const carma_prior_t* prior, siz
                          int device);
 int carma_derived_params_dev(int kind, int p, int q, const carma_prior_t* prior, size_t n, const double* d_theta,
                              double* d_out, void* stream);
+/* Pointwise percentiles of the CARMA power spectrum over the samples of each of ncurves groups (survey form of
+ * CarmaSample.psd_credible_band / plot_power_spectrum, carma_pack.py:548-612).  theta: ncurves*nsamples rows of d,
+ * curve-major.  freq: freq_rows (1 or ncurves) rows of nfreq frequencies.  pct: npct values in [0, 100].
+ *   PSD(f) = sigma^2 |sum_{k<=q} beta_k (2 pi i f)^k|^2 / prod_k |2 pi i f - w_k|^2
+ * with the roots w, MA coefficients beta and sigma of carma_derived_params (CAR1: sigma^2 = 2 omega var).
+ * out[(c*npct + j)*nfreq + f] = np.percentile(psd[c, :, f], pct[j]) (method "linear"), bitwise, of the values returned in
+ * psd_out (NULL, or ncurves*nsamples*nfreq: psd_out[(c*nsamples + s)*nfreq + f]).  A theta row whose PSD is not finite
+ * (NaN or inf in theta, a failed derivation) gives NaN there and NaN percentiles in its curve's columns.  An output
+ * depends only on its curve's theta rows, frequency row and prior.  priors: ncurves entries, only the kappa bounds read
+ * (required for ZCARMA, else may be NULL).  Columns of up to 16384 samples are sorted in shared memory; longer ones are
+ * selected by a radix select over a global scratch column (CARMA_PSD_GLOBAL_SELECT=1 forces that path).
+ * Curves go in chunks whose device footprint stays within 4 GiB: peak 8 B * (B * (nsamples * (d + 22 + nfreq * (1 +
+ * [psd_out])) + npct * nfreq + [freq_rows > 1] nfreq) + npct + nfreq) for a chunk of B curves.  _dev: device pointers, all
+ * curves in one pass with 8 B * ncurves * nsamples * (1 + 3p + [long columns] nfreq) of stream-ordered scratch; pct is
+ * not checked on the host there, and a percentile outside [0, 100] gives NaN. */
+int carma_psd_quantiles(int kind, int p, int q, const carma_prior_t* priors, size_t ncurves, size_t nsamples,
+                        const double* theta, const double* freq, size_t freq_rows, size_t nfreq,
+                        const double* pct, size_t npct, double* out, double* psd_out, int device);
+int carma_psd_quantiles_dev(int kind, int p, int q, const carma_prior_t* d_priors, size_t ncurves, size_t nsamples,
+                            const double* d_theta, const double* d_freq, size_t freq_rows, size_t nfreq,
+                            const double* d_pct, size_t npct, double* d_out, double* d_psd_out, void* stream);
+/* MCMCSample.effective_samples for every column of every series: x (nseries, n, k) row-major, ess (nseries, k).
+ * r = x - mean, ac[j] = sum_i r_i r_{i+j} / max(sum r^2, 1e-300), tau = 1 + 2 sum ac[j] while ac[j] > 0.05,
+ * ess = n / tau; lags are computed one at a time up to the cutoff, in a fixed summation order.  A column whose values
+ * are all equal gets ess = n (its residuals are zero). */
+int carma_effective_samples(size_t nseries, size_t n, size_t k, const double* x, double* ess, int device);
+int carma_effective_samples_dev(size_t nseries, size_t n, size_t k, const double* d_x, double* d_ess, void* stream);
 
 /* ---- maximum-likelihood fits from many starts ----------------------------------------------
  * Replaces the ntrials scipy L-BFGS-B runs of CarmaModel.get_mle / _get_mle_single / _carma_loglik
