@@ -55,7 +55,7 @@ EXPORTED_SYMBOLS = [
     "carma_mle_grid_device", "carma_multi_series_curve_stats", "carma_multi_mle_grid_device",
     "carma_multi_filter_dev", "carma_multi_filter", "carma_multi_assess_fit", "carma_multi_predict",
     "carma_multi_simulate", "carma_psd_quantiles", "carma_psd_quantiles_dev", "carma_effective_samples",
-    "carma_effective_samples_dev",
+    "carma_effective_samples_dev", "carma_multi_smooth",
 ]
 
 
@@ -172,6 +172,8 @@ def _load():
                                       _vp, _vp]
     L.carma_multi_simulate.argtypes = [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp, _vp, _sz, ctypes.c_uint, _vp,
                                        _vp, _sz, ctypes.c_uint64, ctypes.c_uint32, _vp]
+    L.carma_multi_smooth.argtypes = [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp, _vp, ctypes.c_uint, _vp, _vp, _vp,
+                                     _vp, _vp, _vp, _vp, _vp, _vp]
     L.carma_filter.argtypes = [_vp, ctypes.c_double, _dp, _dp, ctypes.c_int, ctypes.c_double, ctypes.c_double, _dp, _dp]
     L.carma_predict.argtypes = [_vp, ctypes.c_double, _dp, _dp, ctypes.c_int, ctypes.c_double, ctypes.c_double,
                                 _dp, _sz, _dp, _dp]
@@ -792,6 +794,47 @@ class MultiSeries:
                                        t.ctypes.data, npaths, int(seed), int(curve_offset), out.ctypes.data),
               "carma_multi_simulate")
         return out
+
+    def smooth(self, kind, p, q, theta, tq=None, q_offsets=None, priors=None, flags=None, points=True):
+        """Kalman smoother of every curve given all of its data (carma_multi_smooth): one pass forward and one backward,
+        O(ny + nq) steps per curve.  theta, priors and flags as kalman_filter (flags None = the survey fits' rule).
+        tq / q_offsets (optional, together): absolute query times as in predict.  Returns an OptimizeResult-style dict:
+          mean, var          the noise-free process at every data point given the curve's data (flat, CSR, mu included);
+          loo_mean, loo_var  the law of each y given every other point of its curve (mu and measurement noise included):
+                             (y - loo_mean) / sqrt(loo_var) is the standardised deleted residual, for flagging outliers;
+          loglik             per curve, bitwise MultiSeries.loglik;
+          qmean, qvar        the smoothed process at tq, in the order of tq (only when tq is given).
+        points=False leaves out the four per-point arrays (nothing but loglik and the queries crosses PCIe), for a caller
+        who only wants the curves on a grid.  A row outside the prior gives NaN for its curve and -inf loglik."""
+        from .carma_pack import OptimizeResult
+        th, priors = self._rows(kind, p, q, theta, priors)
+        if (tq is None) != (q_offsets is None):
+            raise ValueError("tq and q_offsets must be given together")
+        qo = t = None
+        if tq is not None:
+            t = _c(np.atleast_1d(tq))
+            qo = np.ascontiguousarray(q_offsets, dtype=np.int64)
+            if qo.shape != (self.ncurves + 1,) or qo[0] != 0 or qo[-1] != t.size:
+                raise ValueError("q_offsets must have %d entries from 0 to len(tq) = %d" % (self.ncurves + 1, t.size))
+        total = int(self.offsets[-1]) if points else 0
+        mean, var, lm, lv, ll = np.empty(total), np.empty(total), np.empty(total), np.empty(total), np.empty(self.ncurves)
+        ptr = (lambda a: a.ctypes.data) if points else (lambda a: None)
+        qm = qv = None
+        if t is not None:
+            qm, qv = np.empty(t.size), np.empty(t.size)
+        check(lib.carma_multi_smooth(self.handle, kind, p, q, None if priors is None else priors.ctypes.data, th.ctypes.data,
+                                     self._default_flags(p, flags), ptr(mean), ptr(var), ptr(lm), ptr(lv), ll.ctypes.data,
+                                     None if qo is None else qo.ctypes.data,
+                                     None if t is None else t.ctypes.data, None if qm is None else qm.ctypes.data,
+                                     None if qv is None else qv.ctypes.data), "carma_multi_smooth")
+        res = OptimizeResult(loglik=ll)
+        if points:
+            mu = np.repeat(th[:, 2], np.diff(self.offsets))
+            res.update(mean=mean + mu, var=var, loo_mean=lm + mu, loo_var=lv)
+        if t is not None:
+            res.qmean = qm + np.repeat(th[:, 2], np.diff(qo))
+            res.qvar = qv
+        return res
 
 
 def lbfgs_batch(fun_batch, x0, lower, upper, maxiter=1000, history=8, gtol=1e-5, ftol=2.2e-9, fd_eps=1e-8):

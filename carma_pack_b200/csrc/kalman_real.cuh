@@ -200,6 +200,77 @@ struct KalmanReal {
         var = vv;
         mean = m;
     }
+
+    // ---- the smoother's adjoint recursion (multi_smooth_kernel, survey.cu): lambda (P) and the symmetric Lambda (upper
+    // triangle, D's layout) run backwards through the transposed transitions.
+    // v <- Phi^T v: the blocks of Phi^T are [[A, B],[sB, A]], Phi's with B and sB swapped
+    static CARMA_HD void propagate_vec_t(const double* fa, const double* fb, const double* fsb, double fo, double* v) {
+        propagate_vec(fa, fsb, fb, fo, v);
+    }
+    // M <- Phi^T M Phi for a symmetric M: the covariance part of propagate with B and sB swapped
+    static CARMA_HD void congruence_t(double* M, const double* fa, const double* fb, const double* fsb, double fo) {
+#pragma unroll
+        for (int a = 0; a < NS; a++) {
+            const int i = 2 * a;
+            const double A = fa[a], B = fsb[a], SB = fb[a];
+            {
+                const double d00 = M[idx(i, i)], d01 = M[idx(i, i + 1)], d11 = M[idx(i + 1, i + 1)];
+                const double m00 = fma(A, d00, SB * d01), m01 = fma(A, d01, SB * d11);
+                const double m10 = fma(B, d00, A * d01), m11 = fma(B, d01, A * d11);
+                M[idx(i, i)] = fma(m00, A, m01 * SB);
+                M[idx(i, i + 1)] = fma(m00, B, m01 * A);
+                M[idx(i + 1, i + 1)] = fma(m10, B, m11 * A);
+            }
+#pragma unroll
+            for (int b = a + 1; b < NS; b++) {
+                const int j = 2 * b;
+                const double A2 = fa[b], B2 = fsb[b], SB2 = fb[b];
+                const double d00 = M[idx(i, j)], d01 = M[idx(i, j + 1)], d10 = M[idx(i + 1, j)], d11 = M[idx(i + 1, j + 1)];
+                const double m00 = fma(A, d00, SB * d10), m01 = fma(A, d01, SB * d11);
+                const double m10 = fma(B, d00, A * d10), m11 = fma(B, d01, A * d11);
+                M[idx(i, j)] = fma(m00, A2, m01 * SB2);
+                M[idx(i, j + 1)] = fma(m00, B2, m01 * A2);
+                M[idx(i + 1, j)] = fma(m10, A2, m11 * SB2);
+                M[idx(i + 1, j + 1)] = fma(m10, B2, m11 * A2);
+            }
+            if (ODD) {
+                const double d0 = M[idx(i, P - 1)] * fo, d1 = M[idx(i + 1, P - 1)] * fo;
+                M[idx(i, P - 1)] = fma(A, d0, SB * d1);
+                M[idx(i + 1, P - 1)] = fma(B, d0, A * d1);
+            }
+        }
+        if (ODD) M[idx(P - 1, P - 1)] *= fo * fo;
+    }
+    // out = M v for a symmetric M
+    static CARMA_HD void sym_mul(const double* M, const double* v, double* out) {
+#pragma unroll
+        for (int i = 0; i < P; i++) {
+            double acc = 0.0;
+#pragma unroll
+            for (int j = 0; j < P; j++) acc = fma(M[(i <= j) ? idx(i, j) : idx(j, i)], v[j], acc);
+            out[i] = acc;
+        }
+    }
+    static CARMA_HD double dot(const double* a, const double* b) {
+        double s = 0.0;
+#pragma unroll
+        for (int i = 0; i < P; i++) s = fma(a[i], b[i], s);
+        return s;
+    }
+    // Lambda <- c c^T / S + (I - K c)^T Lambda (I - K c) = Lambda - c u^T - u c^T + dk c c^T, given u = Lambda K and
+    // dk = 1/S + K^T u: a symmetric update of rank two along the fixed observation row, O(P^2)
+    static CARMA_HD void info_update(double* M, const double* u, double dk) {
+#pragma unroll
+        for (int i = 0; i < P; i++)
+#pragma unroll
+            for (int j = i; j < P; j++) {
+                double v = M[idx(i, j)];
+                if ((i & 1) == 0) v -= u[j];
+                if ((j & 1) == 0) v -= u[i];
+                if ((i & 1) == 0 && (j & 1) == 0) v += dk;
+                M[idx(i, j)] = v;
+            }
+    }
 };
 
 // Running sum of -1/2 log(var_i) - 1/2 innov_i^2 / var_i with the logs folded into one log of a product of
@@ -566,6 +637,131 @@ __host__ __device__ __noinline__ double loglik_exact_slow(const RealParams<P>& p
         if (i + 1 < ny) kf.template advance<false>(prm, tb, innov, 1.0 / kf.var, dt_i, e_i);
     }
     return ll;
+}
+
+// ---- Kalman smoother of one curve (Bryson-Frazier adjoint form; the survey's multi_smooth_kernel, DESIGN.md K-smooth).
+// Records, field-major: field f of point i at rp[f * ps + i] -- g[P] = P^- c, the predictive mean (without mu), the
+// predictive variance S -- and field f of the curve's sorted query k at rq[f * qs + k - k0] -- w[P] = Phi(t[ip] - t*) g*,
+// mean^-(t*), v^-(t*), ip (number of data times strictly before t*, as a double).  Queries are on the curve's own axis
+// (running sum of dt from 0), sorted; qmean / qvar are written at perm[k].
+//
+// Forward: K4's steps in K4's order (the log-density is bitwise K4's: renormalising LogLikAcc at other points only
+// rescales its mantissa product by powers of two), the point records, and for each query the state filtered at point
+// ip - 1 moved to t* without noise (predict_resume's first half); forecasts (ip = ny) are final here.
+template <int P, bool ALLC, class Tab>
+CARMA_HD void smooth_forward(KalmanReal<P>& kf, LogLikAcc& acc, const RealParams<P>& prm, const Tab& tb, const double* dt,
+                             const double* y, const double* E, int ny, double* rp, size_t ps, long long k, long long k1,
+                             const double* qtq, double* rq, size_t qs, const long long* perm, double* qmean, double* qvar) {
+    constexpr int NS = P / 2;
+    double fa[NS > 0 ? NS : 1], fb[NS > 0 ? NS : 1], fsb[NS > 0 ? NS : 1], fo;
+    double t = 0.0;
+    for (; k < k1 && !(qtq[k] > t); k++) {   // at or before the first point (ip = 0): the stationary law, g* = h
+        double w[P];
+#pragma unroll
+        for (int j = 0; j < P; j++) w[j] = prm.h[j];
+        KalmanReal<P>::template transition<false>(prm, tb, t - qtq[k], fa, fb, fsb, &fo);
+        KalmanReal<P>::propagate_vec(fa, fb, fsb, fo, w);
+#pragma unroll
+        for (int j = 0; j < P; j++) rq[j * qs] = w[j];
+        rq[P * qs] = 0.0;
+        rq[(P + 1) * qs] = prm.v0;
+        rq[(P + 2) * qs] = 0.0;
+        rq++;
+    }
+    int since = 0;
+    for (int i = 0; i < ny; i++) {
+        const bool last = i + 1 == ny;
+        const double dt_i = last ? 0.0 : dt[i];
+        const double tn = t + dt_i;
+        const double innov = (y[i] - prm.mu) - kf.mean;
+        const double inv = rcp_fast(kf.var);
+        acc.add(kf.var, innov, inv);
+#pragma unroll
+        for (int j = 0; j < P; j++) rp[j * ps + i] = kf.g[j];
+        rp[P * ps + i] = kf.mean;
+        rp[(P + 1) * ps + i] = kf.var;
+        for (; k < k1 && (last || !(qtq[k] > tn)); k++) {   // t[i] < t* <= t[i+1], or past the last point: ip = i + 1
+            KalmanReal<P> kq = kf;
+            kq.template advance<false>(prm, tb, innov, 1.0 / kf.var, qtq[k] - t, 0.0);   // no noise at t*
+            if (last) {
+                qmean[perm[k]] = kq.mean;
+                qvar[perm[k]] = kq.var;
+            } else {
+                KalmanReal<P>::template transition<false>(prm, tb, tn - qtq[k], fa, fb, fsb, &fo);
+                KalmanReal<P>::propagate_vec(fa, fb, fsb, fo, kq.g);
+#pragma unroll
+                for (int j = 0; j < P; j++) rq[j * qs] = kq.g[j];
+                rq[P * qs] = kq.mean;
+                rq[(P + 1) * qs] = kq.var;
+            }
+            rq[(P + 2) * qs] = (double)(i + 1);
+            rq++;
+        }
+        if (last) break;
+        kf.template advance<ALLC>(prm, tb, innov, inv, dt_i, E[i + 1]);
+        if (++since == RENORM_EVERY) { acc.renorm(since); since = 0; }
+        t = tn;
+    }
+    acc.renorm(since + 1);
+}
+
+// Backward, from the last point with lambda = Lambda = 0 (K_i = g_i / S_i):
+//   lambda^_i = Phi_i^T lambda_{i+1},  Lambda^_i = Phi_i^T Lambda_{i+1} Phi_i
+//   u_i = e_i / S_i - K_i^T lambda^_i,  d_i = 1 / S_i + K_i^T Lambda^_i K_i
+//   loo: y_i - mu given the rest has mean (y_i - mu) - u_i / d_i and variance 1 / d_i
+//   lambda_i = c u_i + lambda^_i,  Lambda_i = c c^T / S_i + (I - K_i c)^T Lambda^_i (I - K_i c)
+//   smoothed f(t_i): mean_i + g_i^T lambda_i, c.g_i - g_i^T Lambda_i g_i;  query with ip = i: mean^- + w^T lambda_i,
+//   v^- - w^T Lambda_i w.  Outputs (the curve's own slices) without mu.
+template <int P, class Tab>
+CARMA_HD void smooth_backward(const RealParams<P>& prm, const Tab& tb, const double* dt, const double* y, int ny,
+                              const double* rp, size_t ps, long long k0, long long k1, const double* rq, size_t qs,
+                              const long long* perm, double* mean, double* var, double* loo_mean, double* loo_var,
+                              double* qmean, double* qvar) {
+    using KR = KalmanReal<P>;
+    constexpr int NS = P / 2, NT = KR::NT;
+    double lam[P], Lam[NT];
+#pragma unroll
+    for (int j = 0; j < P; j++) lam[j] = 0.0;
+#pragma unroll
+    for (int j = 0; j < NT; j++) Lam[j] = 0.0;
+    const double* qip = rq + (P + 2) * qs - k0;
+    long long k = k1 - 1;
+    while (k >= k0 && qip[k] == (double)ny) k--;   // forecasts are done
+    double fa[NS > 0 ? NS : 1], fb[NS > 0 ? NS : 1], fsb[NS > 0 ? NS : 1], fo;
+    for (int i = ny - 1; i >= 0; i--) {
+        if (i + 1 < ny) {
+            KR::template transition<false>(prm, tb, dt[i], fa, fb, fsb, &fo);
+            KR::propagate_vec_t(fa, fb, fsb, fo, lam);
+            KR::congruence_t(Lam, fa, fb, fsb, fo);
+        }
+        double g[P], K[P], u[P];
+#pragma unroll
+        for (int j = 0; j < P; j++) g[j] = rp[j * ps + i];
+        const double m = rp[P * ps + i], S = rp[(P + 1) * ps + i];
+        const double inv = 1.0 / S, yc = y[i] - prm.mu;
+#pragma unroll
+        for (int j = 0; j < P; j++) K[j] = g[j] * inv;
+        KR::sym_mul(Lam, K, u);
+        const double ui = (yc - m) * inv - KR::dot(K, lam);
+        const double di = inv + KR::dot(K, u);
+        loo_var[i] = 1.0 / di;
+        loo_mean[i] = yc - ui / di;
+#pragma unroll
+        for (int j = 0; j < P; j += 2) lam[j] += ui;
+        KR::info_update(Lam, u, di);
+        double Lg[P];
+        KR::sym_mul(Lam, g, Lg);
+        mean[i] = m + KR::dot(g, lam);
+        var[i] = KR::observe_vec(g) - KR::dot(g, Lg);
+        for (; k >= k0 && qip[k] == (double)i; k--) {
+            double w[P], Lw[P];
+#pragma unroll
+            for (int j = 0; j < P; j++) w[j] = rq[j * qs + (k - k0)];
+            KR::sym_mul(Lam, w, Lw);
+            qmean[perm[k]] = rq[P * qs + (k - k0)] + KR::dot(w, lam);
+            qvar[perm[k]] = rq[(P + 1) * qs + (k - k0)] - KR::dot(w, Lw);
+        }
+    }
 }
 
 }  // namespace carma

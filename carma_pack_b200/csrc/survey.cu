@@ -8,7 +8,10 @@
 //   predict_query_kernel<P>    queries, parking the state in front of each; then one thread = one query resumes from it
 //                              (predict_resume, shared with the single-series predict_real_kernel);
 //   condsim_prior_kernel<P>    one thread = one (curve, path): the prior draw of conditional simulation (Matheron's rule,
-//                              as carma_simulate); the two predict kernels then run on every path's residual data.
+//                              as carma_simulate); the two predict kernels then run on every path's residual data;
+//   multi_smooth_kernel<P>     one thread = one curve: K4's recursion forward, storing per-point and per-query records,
+//                              then the adjoint (Bryson-Frazier) recursion backward: smoothed values, leave-one-out laws
+//                              and queries in O(ny + nq) steps.
 #include <algorithm>
 #include <cmath>
 #include <cstdlib>
@@ -372,6 +375,67 @@ condsim_prior_kernel(const double* __restrict__ dt, const double* __restrict__ y
     }
 }
 
+// Smoother: one thread = one curve of a chunk of curves (smooth_forward / smooth_backward, kalman_real.cuh).  The
+// records live in scratch, field-major: a curve's point records at rp + (o0 - pbase), aligned like its dt / y / e2 arrays
+// (pbase: the chunk's first point rounded down to a multiple of 4, stride pstride), its query records at
+// rq + (qoff[c] - qbase) (stride qstride).  Outputs without mu at the curve's CSR positions; a row the transform rejects
+// gives NaN everywhere and -inf loglik.
+struct SmoothChunk {
+    size_t c0 = 0, nc = 0;
+    long long pbase = 0, qbase = 0;
+    size_t pstride = 0, qstride = 0;
+};
+
+template <int P>
+__global__ void __launch_bounds__(SF_BLOCK, P <= 3 ? 8 : 1)   // K4's bounds
+multi_smooth_kernel(const double* __restrict__ dt, const double* __restrict__ y, const double* __restrict__ e2,
+                    const long long* __restrict__ off, SmoothChunk ch, double dt_max, int kind, int q, int d,
+                    unsigned flags, const carma_prior_t* __restrict__ priors, const double* __restrict__ theta,
+                    const long long* __restrict__ qoff, const double* __restrict__ qtq, const long long* __restrict__ perm,
+                    double* __restrict__ rp, double* __restrict__ rq, double* __restrict__ mean, double* __restrict__ var,
+                    double* __restrict__ loo_mean, double* __restrict__ loo_var, double* __restrict__ loglik,
+                    double* __restrict__ qmean, double* __restrict__ qvar) {
+    MathTab tb;
+    tb.load();
+    const size_t tid = (size_t)blockIdx.x * SF_BLOCK + threadIdx.x;
+    if (tid >= ch.nc) return;
+    const size_t c = ch.c0 + tid;
+    const long long o0 = off[c];
+    const int ny = (int)(off[c + 1] - o0);
+    const long long k0 = qoff[c], k1 = qoff[c + 1];
+    double th[MAX_D];
+#pragma unroll
+    for (int j = 0; j < MAX_D; j++) th[j] = (j < d) ? theta[c * (size_t)d + j] : 0.0;
+    RealParams<P> prm;
+    carma_prior_t pr = priors[c];
+    if (transform_theta<P>(kind, q, flags, pr, th, dt_max, prm) != TT_OK) {
+        for (int i = 0; i < ny; i++) { mean[o0 + i] = NAN; var[o0 + i] = NAN; loo_mean[o0 + i] = NAN; loo_var[o0 + i] = NAN; }
+        for (long long k = k0; k < k1; k++) { qmean[perm[k]] = NAN; qvar[perm[k]] = NAN; }
+        loglik[c] = -INFINITY;
+        return;
+    }
+    const double *cdt = dt + o0, *cy = y + o0, *cE = e2 + o0;
+    double* crp = rp + (o0 - ch.pbase);
+    double* crq = rq + (k0 - ch.qbase);
+    {
+        KalmanReal<P> kf;
+        LogLikAcc acc;
+        kf.reset(prm, cE[0]);
+        acc.init();
+        constexpr unsigned ALL = (P / 2 > 0) ? ((1u << (P / 2)) - 1u) : 0u;
+        if (__all_sync(__activemask(), prm.cmask == ALL))   // warp-uniform, as filter_span_blocks_any
+            smooth_forward<P, true>(kf, acc, prm, tb, cdt, cy, cE, ny, crp, ch.pstride, k0, k1, qtq, crq, ch.qstride,
+                                    perm, qmean, qvar);
+        else
+            smooth_forward<P, false>(kf, acc, prm, tb, cdt, cy, cE, ny, crp, ch.pstride, k0, k1, qtq, crq, ch.qstride,
+                                     perm, qmean, qvar);
+        const SeriesPtr src{cdt, cy, cE + 1};
+        loglik[c] = (acc.bad() ? loglik_exact_slow<P>(prm, tb, src, ny, cE[0]) : acc.value()) + prm.logprior;
+    }
+    smooth_backward<P>(prm, tb, cdt, cy, ny, crp, ch.pstride, k0, k1, crq, ch.qstride, perm, mean + o0, var + o0,
+                       loo_mean + o0, loo_var + o0, qmean, qvar);
+}
+
 // ---- launchers ---------------------------------------------------------------------------------------------------
 static bool alike32(const void* a, const void* b) { return (((size_t)a ^ (size_t)b) & 31u) == 0; }
 
@@ -479,6 +543,18 @@ static double sort_queries(const carma_multi_series* m, const int64_t* q_offsets
 }
 
 static size_t round32(size_t n) { return (n + 31) & ~(size_t)31; }   // doubles: keeps 256-byte alignment
+
+template <int P>
+static cudaError_t launch_smooth_p(const carma_multi_series* m, int kind, int q, unsigned flags, double dt_max,
+                                   const carma_prior_t* d_priors, const double* d_theta, const long long* d_qoff,
+                                   const double* d_qtq, const long long* d_perm, const SmoothChunk& ch, double* d_rp,
+                                   double* d_rq, double* const* d_pt, double* d_ll, double* d_qm, double* d_qv,
+                                   cudaStream_t st) {
+    multi_smooth_kernel<P><<<(unsigned)((ch.nc + SF_BLOCK - 1) / SF_BLOCK), SF_BLOCK, 0, st>>>(
+        m->d_dt, m->d_y, m->d_e2, m->d_off, ch, dt_max, kind, q, model_dim(kind, P, q), flags, d_priors, d_theta, d_qoff,
+        d_qtq, d_perm, d_rp, d_rq, d_pt[0], d_pt[1], d_pt[2], d_pt[3], d_ll, d_qm, d_qv);
+    return cudaGetLastError();
+}
 
 }  // namespace carma
 
@@ -708,6 +784,112 @@ int carma_multi_simulate(carma_multi_series_t m, int kind, int p, int q, const c
             return CARMA_ERR_CUDA;
     }
     if (!cuda_ok(cudaStreamSynchronize(st), "multi_simulate sync")) return CARMA_ERR_CUDA;
+    return CARMA_OK;
+}
+
+int carma_multi_smooth(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* priors, const double* theta,
+                       unsigned flags, double* mean, double* var, double* loo_mean, double* loo_var, double* loglik,
+                       const int64_t* q_offsets, const double* tq, double* qmean, double* qvar) {
+    if (q_offsets && q_offsets[0] != 0) { set_error("carma_multi_smooth: q_offsets must start at 0"); return CARMA_ERR_ARG; }
+    if (!m || !theta) { set_error("carma_multi_smooth: null argument"); return CARMA_ERR_ARG; }
+    if (!valid_model(kind, p, q)) { set_error("carma_multi_smooth: invalid (kind,p,q)"); return CARMA_ERR_ARG; }
+    const size_t nc = m->ncurves;
+    std::vector<int64_t> no_queries;
+    if (!q_offsets) {
+        no_queries.assign(nc + 1, 0);
+        q_offsets = no_queries.data();
+    }
+    for (size_t c = 0; c < nc; c++)
+        if (q_offsets[c + 1] < q_offsets[c]) { set_error("carma_multi_smooth: q_offsets must be non-decreasing"); return CARMA_ERR_ARG; }
+    const size_t nq = (size_t)q_offsets[nc];
+    if (nq > 0 && !tq) { set_error("carma_multi_smooth: null argument (tq)"); return CARMA_ERR_ARG; }
+    for (size_t k = 0; k < nq; k++)
+        if (!std::isfinite(tq[k])) { set_error("carma_multi_smooth: non-finite query time"); return CARMA_ERR_ARG; }
+    std::vector<long long> perm;
+    std::vector<double> qtq;
+    std::vector<int> qcurve;
+    const double dt_max = sort_queries(m, q_offsets, tq, perm, qtq, qcurve);
+    if (!cuda_ok(cudaSetDevice(m->device), "cudaSetDevice")) return CARMA_ERR_CUDA;
+    cudaStream_t st = 0;
+    int rc = upload_rows(m, kind, p, q, priors, theta, nc, st);
+    if (rc) return rc;
+    // Curves go in chunks whose records fit the budget (CARMA_MULTI_SMOOTH_BUDGET bytes, read at every call so that a
+    // test can force several chunks).  Every output depends only on its curve, so chunking changes no bit.
+    const size_t PF = (size_t)p + 2, QF = (size_t)p + 3;
+    size_t budget = (size_t)4 << 30;
+    if (const char* env = getenv("CARMA_MULTI_SMOOTH_BUDGET")) budget = (size_t)std::strtoull(env, nullptr, 10);
+    std::vector<SmoothChunk> chunks;
+    size_t rec_max = 0;   // doubles of the largest chunk's records
+    for (size_t c = 0; c < nc;) {
+        SmoothChunk ch;
+        ch.c0 = c;
+        ch.pbase = m->off[c] & ~3ll;
+        ch.qbase = q_offsets[c];
+        size_t need = 0;
+        for (size_t e = c + 1; e <= nc; e++) {
+            const size_t ps = round32((size_t)(m->off[e] - ch.pbase)), qs = round32((size_t)(q_offsets[e] - ch.qbase));
+            const size_t n = PF * ps + QF * qs;
+            if (e > c + 1 && n * sizeof(double) > budget) break;
+            ch.nc = e - c;
+            ch.pstride = ps;
+            ch.qstride = qs;
+            need = n;
+        }
+        rec_max = std::max(rec_max, need);
+        chunks.push_back(ch);
+        c += ch.nc;
+    }
+    // scratch_pts: mean | var | loo_mean | loo_var (total each); scratch_misc: one chunk's point and query records;
+    // scratch_q: qm | qv | qtq | perm | qoff; scratch_out: loglik
+    const size_t b_pt = round32(m->total), b_q = round32(nq), b_off = round32(nc + 1);
+    if (!m->scratch_pts.reserve(4 * b_pt * sizeof(double)) || !m->scratch_misc.reserve(std::max<size_t>(rec_max, 1) * sizeof(double)) ||
+        !m->scratch_q.reserve((4 * b_q + b_off) * sizeof(double)) || !m->scratch_out.reserve(nc * sizeof(double)))
+        return CARMA_ERR_CUDA;
+    double* d_pt[4];
+    for (int j = 0; j < 4; j++) d_pt[j] = (double*)m->scratch_pts.p + j * b_pt;
+    double* d_qm = (double*)m->scratch_q.p;
+    double* d_qv = d_qm + b_q;
+    double* d_qtq = d_qv + b_q;
+    long long* d_perm = (long long*)(d_qtq + b_q);
+    long long* d_qoff = (long long*)((double*)d_perm + b_q);
+    double* d_ll = (double*)m->scratch_out.p;
+    bool ok = cuda_ok(cudaMemcpyAsync(d_qoff, q_offsets, (nc + 1) * sizeof(long long), cudaMemcpyHostToDevice, st), "H2D q_offsets");
+    if (ok && nq > 0)
+        ok = cuda_ok(cudaMemcpyAsync(d_qtq, qtq.data(), nq * sizeof(double), cudaMemcpyHostToDevice, st), "H2D tq") &&
+             cuda_ok(cudaMemcpyAsync(d_perm, perm.data(), nq * sizeof(long long), cudaMemcpyHostToDevice, st), "H2D perm");
+    if (!ok) return CARMA_ERR_CUDA;
+    const carma_prior_t* d_pr = (const carma_prior_t*)m->scratch_pr.p;
+    const double* d_th = (const double*)m->scratch_in.p;
+    for (const SmoothChunk& ch : chunks) {
+        double* d_rp = (double*)m->scratch_misc.p;
+        double* d_rq = d_rp + PF * ch.pstride;
+        cudaError_t e;
+#define LAUNCH_SM(PP) e = launch_smooth_p<PP>(m, kind, q, flags, dt_max, d_pr, d_th, d_qoff, d_qtq, d_perm, ch, d_rp, d_rq, \
+                                              d_pt, d_ll, d_qm, d_qv, st)
+        switch (p) {
+            case 1: LAUNCH_SM(1); break;
+            case 2: LAUNCH_SM(2); break;
+            case 3: LAUNCH_SM(3); break;
+            case 4: LAUNCH_SM(4); break;
+            case 5: LAUNCH_SM(5); break;
+            case 6: LAUNCH_SM(6); break;
+            default: LAUNCH_SM(7); break;
+        }
+#undef LAUNCH_SM
+        if (!cuda_ok(e, "multi_smooth_kernel launch")) return CARMA_ERR_CUDA;
+    }
+    double* const host_pt[4] = {mean, var, loo_mean, loo_var};
+    const char* what[4] = {"D2H mean", "D2H var", "D2H loo_mean", "D2H loo_var"};
+    for (int j = 0; j < 4; j++)
+        if (host_pt[j] && !cuda_ok(cudaMemcpyAsync(host_pt[j], d_pt[j], m->total * sizeof(double), cudaMemcpyDeviceToHost, st), what[j]))
+            return CARMA_ERR_CUDA;
+    if (loglik && !cuda_ok(cudaMemcpyAsync(loglik, d_ll, nc * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H loglik"))
+        return CARMA_ERR_CUDA;
+    if (nq > 0 && qmean && !cuda_ok(cudaMemcpyAsync(qmean, d_qm, nq * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H qmean"))
+        return CARMA_ERR_CUDA;
+    if (nq > 0 && qvar && !cuda_ok(cudaMemcpyAsync(qvar, d_qv, nq * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H qvar"))
+        return CARMA_ERR_CUDA;
+    if (!cuda_ok(cudaStreamSynchronize(st), "multi_smooth sync")) return CARMA_ERR_CUDA;
     return CARMA_OK;
 }
 

@@ -298,6 +298,24 @@ int carma_multi_predict(carma_multi_series_t m, int kind, int p, int q, const ca
 int carma_multi_simulate(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* priors,
                          const double* theta, size_t theta_rows, unsigned flags, const int64_t* s_offsets,
                          const double* tsim, size_t npaths, uint64_t seed, uint32_t curve_offset, double* ysim);
+/* Kalman smoother (Bryson-Frazier adjoint form, an extension: the reference has none) of every curve in one pass forward
+ * and one backward, O(ny + nq) steps per curve.  theta, priors and flags as carma_multi_filter.  Per point, in the CSR
+ * order of the multi-series (total entries each), means without mu:
+ *   mean / var:         E[f(t_i) | y] and Var[f(t_i) | y] of the noise-free process given all of the curve's data;
+ *   loo_mean / loo_var: the law of y_i given every other point of its curve (measurement noise included), so that
+ *                       (y_i - mu - loo_mean) / sqrt(loo_var) is the standardised deleted residual.
+ * loglik (ncurves): bitwise what carma_multi_loglik returns for the same arguments.  q_offsets / tq as carma_multi_predict
+ * (absolute times, any order; qmean / qvar in the caller's order), or both NULL for no queries: the smoothed process at
+ * each query time (a data time gives that point's smoothed value, a time past the last point the forecast).  Any output
+ * pointer may be NULL.  A row the transform rejects gives NaN outputs for its curve and -inf loglik.  Blocking; uses the
+ * multi-series' scratch (one call per handle at a time).  Curves run in chunks whose records stay within 4 GiB: peak
+ * scratch 32 round32(total) + 32 round32(nq) + 8 round32(ncurves + 1) + 8 ncurves bytes for the outputs and sorted
+ * queries, plus the records of
+ * the largest chunk, 8 ((p + 2) ny + (p + 3) nq) bytes summed over its curves (one curve's records even when they
+ * exceed the budget), plus the theta rows and priors. */
+int carma_multi_smooth(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* priors, const double* theta,
+                       unsigned flags, double* mean, double* var, double* loo_mean, double* loo_var, double* loglik,
+                       const int64_t* q_offsets, const double* tq, double* qmean, double* qvar);
 
 /* ---- one very long light curve: temporally parallel (associative-scan) form of the same LogDensity ----
  * Replaces the strictly sequential Filter() loop (src/include/kfilter.hpp:126-132) when there is a single
