@@ -37,6 +37,9 @@ _point_at_bundled_nccl()
 KIND_CAR1, KIND_CARP, KIND_CARMA, KIND_ZCAR, KIND_ZCARMA = 0, 1, 2, 3, 4
 IGNORE_BOUNDS, LOGLIK_ONLY = 1, 2
 MAX_P = 7
+# status of MultiSeries.hessian per curve (CARMA_HESS_*), and its default relative step 2^-13
+HESS_OK, HESS_REJECTED, HESS_NONFINITE, HESS_NOT_NEGDEF = 0, 1, 2, 3
+HESS_REL_STEP = 2.0 ** -13
 
 EXPORTED_SYMBOLS = [
     "carma_last_error", "carma_abi_version", "carma_device_count",
@@ -55,7 +58,7 @@ EXPORTED_SYMBOLS = [
     "carma_mle_grid_device", "carma_multi_series_curve_stats", "carma_multi_mle_grid_device",
     "carma_multi_filter_dev", "carma_multi_filter", "carma_multi_assess_fit", "carma_multi_predict",
     "carma_multi_simulate", "carma_psd_quantiles", "carma_psd_quantiles_dev", "carma_effective_samples",
-    "carma_effective_samples_dev", "carma_multi_smooth",
+    "carma_effective_samples_dev", "carma_multi_smooth", "carma_multi_hessian",
 ]
 
 
@@ -174,6 +177,8 @@ def _load():
                                        _vp, _sz, ctypes.c_uint64, ctypes.c_uint32, _vp]
     L.carma_multi_smooth.argtypes = [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp, _vp, ctypes.c_uint, _vp, _vp, _vp,
                                      _vp, _vp, _vp, _vp, _vp, _vp]
+    L.carma_multi_hessian.argtypes = [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp, _vp, ctypes.c_uint,
+                                      ctypes.c_double, _vp, _vp, _vp, _vp, _vp]
     L.carma_filter.argtypes = [_vp, ctypes.c_double, _dp, _dp, ctypes.c_int, ctypes.c_double, ctypes.c_double, _dp, _dp]
     L.carma_predict.argtypes = [_vp, ctypes.c_double, _dp, _dp, ctypes.c_int, ctypes.c_double, ctypes.c_double,
                                 _dp, _sz, _dp, _dp]
@@ -835,6 +840,44 @@ class MultiSeries:
             res.qmean = qm + np.repeat(th[:, 2], np.diff(qo))
             res.qvar = qv
         return res
+
+    def hessian(self, kind, p, q, theta, priors=None, flags=None, rel_step=None):
+        """Gradient, Hessian and Laplace covariance of every curve's log-density at its theta row
+        (carma_multi_hessian): central finite differences, d^2 + d + 1 evaluations per curve in one launch.  The
+        function is exactly MultiSeries.loglik with the same priors and flags (None = the survey fits' rule), so at a
+        fit, hessian(kind, p, q, fit.x).loglik is -fit.fun.  Steps h_i = rel_step * (theta_0, theta_1, theta_0, 1, ...)_i
+        (rel_step None or <= 0: HESS_REL_STEP = 2^-13).  Returns an OptimizeResult-style dict:
+          loglik (nc,), grad (nc, d), hessian (nc, d, d), cov (nc, d, d) = (-hessian)^-1,
+          stderr (nc, d) = sqrt(diag(cov)), NaN unless status is HESS_OK,
+          status (nc,) one of HESS_OK, HESS_REJECTED (loglik -inf, the rest NaN), HESS_NONFINITE (a stencil value is
+          not finite: grad / hessian / cov NaN), HESS_NOT_NEGDEF (-hessian not positive definite: cov NaN),
+          step (nc, d) the h used."""
+        from .carma_pack import OptimizeResult
+        th, priors = self._rows(kind, p, q, theta, priors)
+        rs = HESS_REL_STEP if rel_step is None else float(rel_step)
+        if not np.isfinite(rs):
+            raise ValueError("rel_step must be finite")
+        if rs <= 0.0:
+            rs = HESS_REL_STEP
+        nc, d = self.ncurves, th.shape[1]
+        ll, g, h, cov = np.empty(nc), np.empty((nc, d)), np.empty((nc, d, d)), np.empty((nc, d, d))
+        st = np.empty(nc, dtype=np.intc)
+        check(lib.carma_multi_hessian(self.handle, kind, p, q, None if priors is None else priors.ctypes.data,
+                                      th.ctypes.data, self._default_flags(p, flags), rs, ll.ctypes.data, g.ctypes.data,
+                                      h.ctypes.data, cov.ctypes.data, st.ctypes.data), "carma_multi_hessian")
+        stderr = np.sqrt(np.diagonal(cov, axis1=1, axis2=2))
+        stderr = np.where((st == HESS_OK)[:, None], stderr, np.nan)
+        return OptimizeResult(loglik=ll, grad=g, hessian=h, cov=cov, stderr=stderr, status=st.astype(np.int64),
+                              step=hessian_steps(th, rs))
+
+
+def hessian_steps(theta, rel_step=HESS_REL_STEP):
+    """The finite-difference steps of carma_multi_hessian for theta rows (n, d): rel_step * (theta_0, theta_1, theta_0,
+    1, 1, ...), each one rounded product."""
+    th = np.atleast_2d(np.asarray(theta, dtype=np.float64))
+    s = np.ones_like(th)
+    s[:, 0], s[:, 1], s[:, 2] = th[:, 0], th[:, 1], th[:, 0]
+    return rel_step * s
 
 
 def lbfgs_batch(fun_batch, x0, lower, upper, maxiter=1000, history=8, gtol=1e-5, ftol=2.2e-9, fd_eps=1e-8):

@@ -315,6 +315,19 @@ class CarmaModel(object):
             raise ValueError("optimizer must be 'device', 'native' or 'python'")
         return self._mle_result(x, f, nit, nfev)
 
+    def hessian(self, theta, p=None, q=None, rel_step=None):
+        """Gradient, Hessian and Laplace covariance of the log-density at theta (e.g. get_mle(...).x), with get_mle's
+        model kind, population-variance prior and flags: MultiSeries.hessian on this curve alone, so it equals a survey
+        row bit for bit.  Returns loglik (scalar), grad (d,), hessian (d, d), cov (d, d), stderr (d,), status, step (d,)."""
+        p = self.p if p is None else p
+        q = self.q if q is None else q
+        ms = _lib.MultiSeries(self.time, self.y, self.ysig, [0, self.time.size], device=self.device)
+        try:
+            res = ms.hessian(_kind_for(p, q), p, q, np.asarray(theta, dtype=np.float64)[None, :], rel_step=rel_step)
+        finally:
+            ms.close()
+        return OptimizeResult({k: (v[0].item() if v.ndim == 1 else v[0]) for k, v in res.items()})
+
     @staticmethod
     def _mle_result(x, f, nit, nfev):
         best = int(np.argmin(f))

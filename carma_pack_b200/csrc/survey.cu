@@ -11,7 +11,9 @@
 //                              as carma_simulate); the two predict kernels then run on every path's residual data;
 //   multi_smooth_kernel<P>     one thread = one curve: K4's recursion forward, storing per-point and per-query records,
 //                              then the adjoint (Bryson-Frazier) recursion backward: smoothed values, leave-one-out laws
-//                              and queries in O(ny + nq) steps.
+//                              and queries in O(ny + nq) steps;
+//   multi_hessian_eval_kernel<P>  one thread = one (curve, stencil point): K4's body on a finite-difference row;
+//   multi_hessian_assemble_kernel one thread = one curve: gradient, Hessian and covariance from its stencil values.
 #include <algorithm>
 #include <cmath>
 #include <cstdlib>
@@ -20,6 +22,7 @@
 #include <string>
 #include <vector>
 
+#include "hessian.cuh"
 #include "kalman_real.cuh"
 #include "series.h"
 
@@ -436,6 +439,73 @@ multi_smooth_kernel(const double* __restrict__ dt, const double* __restrict__ y,
                        loo_mean + o0, loo_var + o0, qmean, qvar);
 }
 
+// Hessian, evaluation: one thread per (curve, stencil point) of the curves c0 .. c0 + nc - 1, stencil-minor (thread u:
+// curve c0 + u / npts, point u % npts; hessian.cuh), so the lanes of a warp walk the same curve: each 32-byte block of it
+// is fetched once per warp and its length does not diverge inside the warp.  The step is one rounded product and the
+// row one rounded add or subtract (no contraction), as numpy forms them.  After the row, the body is
+// multi_loglik_kernel's (same transform and rate clamp, block loads, slow fallback, log-prior), so fval[u] is what
+// carma_multi_loglik returns for that row.
+template <int P>
+__global__ void __launch_bounds__(SF_BLOCK, P <= 3 ? 8 : 1)   // K4's bounds
+multi_hessian_eval_kernel(const double* __restrict__ dt, const double* __restrict__ y, const double* __restrict__ e2,
+                          const long long* __restrict__ off, size_t c0, size_t nc, int npts, double dt_max, int kind,
+                          int q, int d, unsigned flags, const carma_prior_t* __restrict__ priors,
+                          const double* __restrict__ theta, double rel_step, double* __restrict__ fval) {
+    MathTab tb;
+    tb.load();
+    const size_t u = (size_t)blockIdx.x * SF_BLOCK + threadIdx.x;
+    if (u >= nc * npts) return;
+    const size_t cl = u / npts;
+    const int k = (int)(u - cl * npts);
+    const size_t c = c0 + cl;
+    const long long o0 = off[c], o1 = off[c + 1];
+    const int ny = (int)(o1 - o0);
+    const double* row = theta + c * (size_t)d;
+    const double th0 = row[0], th1 = row[1];
+    int a, b;
+    double sa, sb;
+    hess_point_dirs(k, d, &a, &sa, &b, &sb);
+    double th[MAX_D];
+#pragma unroll
+    for (int j = 0; j < MAX_D; j++) {
+        const double v = (j < d) ? row[j] : 0.0;
+        const double h = __dmul_rn(rel_step, hess_scale(th0, th1, j));
+        const double s = (j == a) ? sa : (j == b) ? sb : 0.0;
+        th[j] = (s > 0.0) ? __dadd_rn(v, h) : (s < 0.0) ? __dsub_rn(v, h) : v;
+    }
+    RealParams<P> prm;
+    carma_prior_t pr = priors[c];
+    if (transform_theta<P>(kind, q, flags, pr, th, dt_max, prm) != TT_OK) {
+        fval[u] = -INFINITY;
+        return;
+    }
+    KalmanReal<P> kf;
+    LogLikAcc acc;
+    kf.reset(prm, e2[o0]);
+    acc.init();
+    const SeriesPtr src{dt + o0, y + o0, e2 + o0 + 1};
+    filter_span_blocks_any<P>(kf, acc, prm, tb, dt + o0, y + o0, e2 + o0, ny);
+    fval[u] = (acc.bad() ? loglik_exact_slow<P>(prm, tb, src, ny, e2[o0]) : acc.value()) + prm.logprior;
+}
+
+// Hessian, assembly: one thread per curve of the chunk, hess_assemble on its npts stencil values; outputs at the curve's
+// global index.
+__global__ void __launch_bounds__(SF_BLOCK)
+multi_hessian_assemble_kernel(const double* __restrict__ fval, size_t c0, size_t nc, int d,
+                              const double* __restrict__ theta, double rel_step, double* __restrict__ loglik,
+                              double* __restrict__ grad, double* __restrict__ hess, double* __restrict__ cov,
+                              int* __restrict__ status) {
+    const size_t cl = (size_t)blockIdx.x * SF_BLOCK + threadIdx.x;
+    if (cl >= nc) return;
+    const size_t c = c0 + cl;
+    const double* row = theta + c * (size_t)d;
+    double h[MAX_D];
+    for (int i = 0; i < d; i++) h[i] = __dmul_rn(rel_step, hess_scale(row[0], row[1], i));
+    const double* f = fval + cl * (size_t)hess_points(d);
+    loglik[c] = f[0];
+    status[c] = hess_assemble(d, f, h, grad + c * d, hess + c * d * d, cov + c * d * d);
+}
+
 // ---- launchers ---------------------------------------------------------------------------------------------------
 static bool alike32(const void* a, const void* b) { return (((size_t)a ^ (size_t)b) & 31u) == 0; }
 
@@ -553,6 +623,16 @@ static cudaError_t launch_smooth_p(const carma_multi_series* m, int kind, int q,
     multi_smooth_kernel<P><<<(unsigned)((ch.nc + SF_BLOCK - 1) / SF_BLOCK), SF_BLOCK, 0, st>>>(
         m->d_dt, m->d_y, m->d_e2, m->d_off, ch, dt_max, kind, q, model_dim(kind, P, q), flags, d_priors, d_theta, d_qoff,
         d_qtq, d_perm, d_rp, d_rq, d_pt[0], d_pt[1], d_pt[2], d_pt[3], d_ll, d_qm, d_qv);
+    return cudaGetLastError();
+}
+
+template <int P>
+static cudaError_t launch_hessian_eval_p(const carma_multi_series* m, int kind, int q, unsigned flags,
+                                         const carma_prior_t* d_priors, const double* d_theta, double rel_step,
+                                         size_t c0, size_t nc, double* d_f, cudaStream_t st) {
+    const int d = model_dim(kind, P, q), npts = hess_points(d);
+    multi_hessian_eval_kernel<P><<<(unsigned)((nc * npts + SF_BLOCK - 1) / SF_BLOCK), SF_BLOCK, 0, st>>>(
+        m->d_dt, m->d_y, m->d_e2, m->d_off, c0, nc, npts, m->dt_max, kind, q, d, flags, d_priors, d_theta, rel_step, d_f);
     return cudaGetLastError();
 }
 
@@ -890,6 +970,66 @@ int carma_multi_smooth(carma_multi_series_t m, int kind, int p, int q, const car
     if (nq > 0 && qvar && !cuda_ok(cudaMemcpyAsync(qvar, d_qv, nq * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H qvar"))
         return CARMA_ERR_CUDA;
     if (!cuda_ok(cudaStreamSynchronize(st), "multi_smooth sync")) return CARMA_ERR_CUDA;
+    return CARMA_OK;
+}
+
+int carma_multi_hessian(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* priors, const double* theta,
+                        unsigned flags, double rel_step, double* loglik, double* grad, double* hess, double* cov,
+                        int* status) {
+    if (!std::isfinite(rel_step)) { set_error("carma_multi_hessian: rel_step must be finite"); return CARMA_ERR_ARG; }
+    if (!valid_model(kind, p, q)) { set_error("carma_multi_hessian: invalid (kind,p,q)"); return CARMA_ERR_ARG; }
+    if (!m || !theta) { set_error("carma_multi_hessian: null argument"); return CARMA_ERR_ARG; }
+    if (rel_step <= 0.0) rel_step = CARMA_HESS_DEFAULT_REL_STEP;
+    if (!alike32(m->d_dt, m->d_y) || !alike32(m->d_dt, m->d_e2)) { set_error("carma_multi_hessian: curve arrays not sector-aligned"); return CARMA_ERR_ARG; }
+    const size_t nc = m->ncurves, d = (size_t)model_dim(kind, p, q), npts = (size_t)hess_points((int)d);
+    if (!cuda_ok(cudaSetDevice(m->device), "cudaSetDevice")) return CARMA_ERR_CUDA;
+    cudaStream_t st = 0;
+    int rc = upload_rows(m, kind, p, q, priors, theta, nc, st);
+    if (rc) return rc;
+    // Curves go in chunks of B whose stencil values fit the budget (CARMA_MULTI_HESSIAN_BUDGET bytes, read at every call
+    // so that a test can force several chunks).  Every output depends only on its curve, so chunking changes no bit.
+    size_t budget = (size_t)4 << 30;
+    if (const char* env = getenv("CARMA_MULTI_HESSIAN_BUDGET")) budget = (size_t)std::strtoull(env, nullptr, 10);
+    const size_t B = std::max<size_t>(1, std::min(nc, budget / (npts * sizeof(double))));
+    // scratch_misc: one chunk's stencil values; scratch_pts: loglik | grad | hess | cov | status
+    const size_t b_ll = round32(nc), b_g = round32(nc * d), b_h = round32(nc * d * d), b_st = round32((nc + 1) / 2);
+    if (!m->scratch_misc.reserve(B * npts * sizeof(double)) ||
+        !m->scratch_pts.reserve((b_ll + b_g + 2 * b_h + b_st) * sizeof(double)))
+        return CARMA_ERR_CUDA;
+    double* d_f = (double*)m->scratch_misc.p;
+    double* d_ll = (double*)m->scratch_pts.p;
+    double* d_g = d_ll + b_ll;
+    double* d_h = d_g + b_g;
+    double* d_cov = d_h + b_h;
+    int* d_st = (int*)(d_cov + b_h);
+    const carma_prior_t* d_pr = (const carma_prior_t*)m->scratch_pr.p;
+    const double* d_th = (const double*)m->scratch_in.p;
+    for (size_t c0 = 0; c0 < nc; c0 += B) {
+        const size_t n = std::min(B, nc - c0);
+        cudaError_t e;
+#define LAUNCH_HE(PP) e = launch_hessian_eval_p<PP>(m, kind, q, flags, d_pr, d_th, rel_step, c0, n, d_f, st)
+        switch (p) {
+            case 1: LAUNCH_HE(1); break;
+            case 2: LAUNCH_HE(2); break;
+            case 3: LAUNCH_HE(3); break;
+            case 4: LAUNCH_HE(4); break;
+            case 5: LAUNCH_HE(5); break;
+            case 6: LAUNCH_HE(6); break;
+            default: LAUNCH_HE(7); break;
+        }
+#undef LAUNCH_HE
+        if (!cuda_ok(e, "multi_hessian_eval_kernel launch")) return CARMA_ERR_CUDA;
+        multi_hessian_assemble_kernel<<<(unsigned)((n + SF_BLOCK - 1) / SF_BLOCK), SF_BLOCK, 0, st>>>(
+            d_f, c0, n, (int)d, d_th, rel_step, d_ll, d_g, d_h, d_cov, d_st);
+        if (!cuda_ok(cudaGetLastError(), "multi_hessian_assemble_kernel launch")) return CARMA_ERR_CUDA;
+    }
+    struct Out { void* host; const void* dev; size_t bytes; const char* what; };
+    const Out outs[5] = {{loglik, d_ll, nc * sizeof(double), "D2H loglik"}, {grad, d_g, nc * d * sizeof(double), "D2H grad"},
+                         {hess, d_h, nc * d * d * sizeof(double), "D2H hess"}, {cov, d_cov, nc * d * d * sizeof(double), "D2H cov"},
+                         {status, d_st, nc * sizeof(int), "D2H status"}};
+    for (const Out& o : outs)
+        if (o.host && !cuda_ok(cudaMemcpyAsync(o.host, o.dev, o.bytes, cudaMemcpyDeviceToHost, st), o.what)) return CARMA_ERR_CUDA;
+    if (!cuda_ok(cudaStreamSynchronize(st), "multi_hessian sync")) return CARMA_ERR_CUDA;
     return CARMA_OK;
 }
 

@@ -316,6 +316,39 @@ int carma_multi_simulate(carma_multi_series_t m, int kind, int p, int q, const c
 int carma_multi_smooth(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* priors, const double* theta,
                        unsigned flags, double* mean, double* var, double* loo_mean, double* loo_var, double* loglik,
                        const int64_t* q_offsets, const double* tq, double* qmean, double* qvar);
+/* Curvature of every curve's log-density at its theta row (an extension: the reference's get_mle returns at most scipy's
+ * approximate hess_inv), by central finite differences evaluated on the device.  The function is exactly the one
+ * carma_multi_loglik evaluates for the row, with the same kind, p, q, priors (NULL: defaults) and flags, log-prior term
+ * on measerr_scale included; with the survey fits' flags (0 for p == 1, else CARMA_IGNORE_BOUNDS) it is -fun of the fit.
+ *   Steps: h_i = rel_step * s_i, s = (theta_0, theta_1, theta_0, 1, 1, ...): sigma_y and measerr_scale relative, mu in
+ *   units of sigma_y, every coordinate from 3 on (log or logit) absolute.  rel_step <= 0 selects
+ *   CARMA_HESS_DEFAULT_REL_STEP = 2^-13 (about eps^(1/4)); a power of two makes h_i exact.  NaN or inf is rejected.
+ *   Stencil, d^2 + d + 1 points per curve: the centre f0, theta +- h_i e_i (f+i, f-i), and for i < j
+ *   theta + h_i e_i + h_j e_j (f+ij) and theta - h_i e_i - h_j e_j (f-ij).
+ *   Assembly: g_i = (f+i - f-i) / 2h_i;  H_ii = (f+i - 2 f0 + f-i) / h_i^2;
+ *   H_ij = (f+ij - f+i - f+j + 2 f0 - f-i - f-j + f-ij) / (2 h_i h_j), formed for i < j and mirrored;
+ *   cov = (-H)^-1 through a Cholesky factorisation of -H.
+ * Outputs (any may be NULL): loglik (ncurves) = f0, bitwise carma_multi_loglik's; grad (ncurves x d); hess and cov
+ * (ncurves x d x d, row-major); status (ncurves) one of CARMA_HESS_*:
+ *   OK          every output valid;
+ *   REJECTED    the centre row fails the transform or the prior bounds: loglik -inf, the rest NaN;
+ *   NONFINITE   a stencil value or a step is not finite or zero (e.g. CAR(1) on its prior's frequency bound): loglik
+ *               valid, grad / hess / cov NaN;
+ *   NOT_NEGDEF  the Cholesky factorisation of -H fails: grad and hess valid, cov NaN.
+ * There is no one-sided fallback at a bound: a fit on a bound has no interior curvature and the status says so.  An
+ * output depends only on its curve's data, theta row and prior.  Blocking; uses the multi-series' scratch (one call per
+ * handle at a time).  Curves run in chunks whose stencil values (8 (d^2 + d + 1) bytes per curve) stay within 4 GiB;
+ * outputs take 8 ncurves (2 d^2 + d + 2) bytes more, plus the theta rows and priors. */
+#define CARMA_HESS_DEFAULT_REL_STEP 1.220703125e-4   /* 2^-13 */
+enum {
+    CARMA_HESS_OK = 0,
+    CARMA_HESS_REJECTED = 1,
+    CARMA_HESS_NONFINITE = 2,
+    CARMA_HESS_NOT_NEGDEF = 3
+};
+int carma_multi_hessian(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* priors,
+                        const double* theta /* ncurves x d */, unsigned flags, double rel_step, double* loglik,
+                        double* grad, double* hess, double* cov, int* status);
 
 /* ---- one very long light curve: temporally parallel (associative-scan) form of the same LogDensity ----
  * Replaces the strictly sequential Filter() loop (src/include/kfilter.hpp:126-132) when there is a single
