@@ -23,7 +23,7 @@ CXX = os.environ.get("CXX_HOST") or shutil.which("g++") or "g++"
 
 CUDA_SOURCES = ["loglik.cu", "mcmc.cu", "scan.cu", "sim.cu", "mle.cu", "mle_dev.cu", "comm.cu", "survey.cu", "posterior.cu"]
 CUDA_HEADERS = ["device_math.cuh", "fast_math.cuh", "theta_transform.cuh", "kalman_real.cuh", "kalman_cplx.cuh", "series.h",
-                "hessian.cuh", os.path.join(ROOT, "include", "carma_b200.h")]
+                "hessian.cuh", "laplace.cuh", "select.cuh", os.path.join(ROOT, "include", "carma_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr", "-Xptxas", "-v"]
 

@@ -40,6 +40,9 @@ MAX_P = 7
 # status of MultiSeries.hessian per curve (CARMA_HESS_*), and its default relative step 2^-13
 HESS_OK, HESS_REJECTED, HESS_NONFINITE, HESS_NOT_NEGDEF = 0, 1, 2, 3
 HESS_REL_STEP = 2.0 ** -13
+# status of MultiSeries.laplace per curve (CARMA_LAPLACE_*), and the most draws per curve of one call
+LAPLACE_OK, LAPLACE_BAD_COV, LAPLACE_NO_WEIGHT = 0, 1, 2
+LAPLACE_MAX_DRAWS = 1 << 20
 
 EXPORTED_SYMBOLS = [
     "carma_last_error", "carma_abi_version", "carma_device_count",
@@ -58,7 +61,7 @@ EXPORTED_SYMBOLS = [
     "carma_mle_grid_device", "carma_multi_series_curve_stats", "carma_multi_mle_grid_device",
     "carma_multi_filter_dev", "carma_multi_filter", "carma_multi_assess_fit", "carma_multi_predict",
     "carma_multi_simulate", "carma_psd_quantiles", "carma_psd_quantiles_dev", "carma_effective_samples",
-    "carma_effective_samples_dev", "carma_multi_smooth", "carma_multi_hessian",
+    "carma_effective_samples_dev", "carma_multi_smooth", "carma_multi_hessian", "carma_multi_laplace",
 ]
 
 
@@ -179,6 +182,8 @@ def _load():
                                      _vp, _vp, _vp, _vp, _vp, _vp]
     L.carma_multi_hessian.argtypes = [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp, _vp, ctypes.c_uint,
                                       ctypes.c_double, _vp, _vp, _vp, _vp, _vp]
+    L.carma_multi_laplace.argtypes = [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, _vp, _vp, _vp, ctypes.c_uint, _sz,
+                                      ctypes.c_uint64, ctypes.c_uint32, _vp, _vp, _vp, _vp, _vp, _vp, _vp]
     L.carma_filter.argtypes = [_vp, ctypes.c_double, _dp, _dp, ctypes.c_int, ctypes.c_double, ctypes.c_double, _dp, _dp]
     L.carma_predict.argtypes = [_vp, ctypes.c_double, _dp, _dp, ctypes.c_int, ctypes.c_double, ctypes.c_double,
                                 _dp, _sz, _dp, _dp]
@@ -869,6 +874,75 @@ class MultiSeries:
         stderr = np.where((st == HESS_OK)[:, None], stderr, np.nan)
         return OptimizeResult(loglik=ll, grad=g, hessian=h, cov=cov, stderr=stderr, status=st.astype(np.int64),
                               step=hessian_steps(th, rs))
+
+    def laplace(self, kind, p, q, theta, cov, ndraws=1000, seed=None, curve_offset=0, priors=None, flags=0):
+        """Importance sampling of every curve's posterior from its Laplace approximation N(theta_c, cov_c)
+        (carma_multi_laplace): ndraws draws per curve, each draw's exact log-density, the Pareto k-hat of the weights and
+        an equally weighted resample, in one call.  The target is MultiSeries.loglik with these priors (None: the
+        population-variance defaults) and flags.  The defaults, flags 0 and those priors, are the posterior run_mcmc
+        samples, so that the weights target it; they differ from hessian's default (the survey fits' rule, which skips
+        the prior bounds for p > 1), because a fit's curvature and a posterior's draws answer different questions.
+        Draw j of curve c depends only on (seed, j, curve_offset + c, theta_c, cov_c).  Returns an OptimizeResult-style
+        dict:
+          draws (nc, ndraws, d), logpost (nc, ndraws) bitwise MultiSeries.loglik of the draws, logq (nc, ndraws) the
+          proposal's log-density, log_weights = logpost - logq (-inf where logpost is not finite; NaN for
+          every draw of a LAPLACE_BAD_COV curve, which has no draws),
+          ess (nc,) the weight ESS, khat (nc,) the Pareto k-hat (<= 0.7: the Gaussian answer is good; above: run MCMC),
+          resample (nc, ndraws) indices into draws of an equally weighted sample (-1 unless status is LAPLACE_OK),
+          status (nc,) one of LAPLACE_OK, LAPLACE_BAD_COV (cov or theta not finite, or not positive definite: NaN
+          draws), LAPLACE_NO_WEIGHT (no draw has a finite logpost)."""
+        from .carma_pack import OptimizeResult
+        th, priors = self._rows(kind, p, q, theta, priors)
+        nc, d = self.ncurves, th.shape[1]
+        cv = np.ascontiguousarray(cov, dtype=np.float64)
+        if cv.shape != (nc, d, d):
+            raise ValueError("cov must be (%d, %d, %d)" % (nc, d, d))
+        S = int(ndraws)
+        if not 1 <= S <= LAPLACE_MAX_DRAWS:
+            raise ValueError("ndraws must be in 1 .. %d" % LAPLACE_MAX_DRAWS)
+        curve_offset = int(curve_offset)
+        if curve_offset < 0 or curve_offset + nc > 2 ** 32:
+            raise ValueError("curve_offset must be >= 0 with curve_offset + ncurves <= 2^32")
+        if seed is None:
+            seed = int(np.random.SeedSequence().generate_state(1, dtype=np.uint64)[0] >> 1)
+        draws, lp, lq = np.empty((nc, S, d)), np.empty((nc, S)), np.empty((nc, S))
+        rs = np.empty((nc, S), dtype=np.int32)
+        ess, kh, st = np.empty(nc), np.empty(nc), np.empty(nc, dtype=np.intc)
+        check(lib.carma_multi_laplace(self.handle, kind, p, q, None if priors is None else priors.ctypes.data,
+                                      th.ctypes.data, cv.ctypes.data, int(flags), S, int(seed), curve_offset,
+                                      draws.ctypes.data, lp.ctypes.data, lq.ctypes.data, rs.ctypes.data, ess.ctypes.data,
+                                      kh.ctypes.data, st.ctypes.data), "carma_multi_laplace")
+        lw = np.where(np.isfinite(lp), lp - lq, -np.inf)
+        lw[st == LAPLACE_BAD_COV] = np.nan
+        return OptimizeResult(draws=draws, logpost=lp, logq=lq, log_weights=lw, ess=ess, khat=kh, resample=rs,
+                              status=st.astype(np.int64))
+
+    def laplace_sample(self, p, q, theta, cov=None, ndraws=1000, seed=None, curve_offset=0, priors=None):
+        """The posterior of every curve by importance sampling from its Laplace approximation at theta (e.g.
+        get_mle(p, q).x): laplace() with run_mcmc's posterior, resampled to an equally weighted sample.  cov None: the
+        covariance of hessian(kind, p, q, theta, priors=priors); a curve whose Hessian status is not HESS_OK comes back
+        LAPLACE_BAD_COV.  Returns a LaplaceSample (a SurveySample: derived parameters, psd_credible_band, map_theta, DIC
+        and curve(c) work as for run_mcmc's) with khat, ess, status and the raw laplace() result; the trace rows of a
+        curve whose status is not LAPLACE_OK are NaN, so its summaries are NaN."""
+        from .carma_pack import LaplaceSample, _kind_for
+        if not p > q:
+            raise ValueError("Order of AR polynomial, p, must be larger than order of MA polynomial, q.")
+        kind = _kind_for(p, q)
+        th, priors = self._rows(kind, p, q, theta, priors)
+        if cov is None:
+            h = self.hessian(kind, p, q, th, priors=priors)
+            cov = np.where((h.status == HESS_OK)[:, None, None], h.cov, np.nan)
+        r = self.laplace(kind, p, q, th, cov, ndraws=ndraws, seed=seed, curve_offset=curve_offset, priors=priors)
+        nc = self.ncurves
+        idx = np.maximum(r.resample, 0)
+        trace = r.draws[np.arange(nc)[:, None], idx]
+        lp = r.logpost[np.arange(nc)[:, None], idx]
+        bad = r.status != LAPLACE_OK
+        trace[bad] = np.nan
+        lp[bad] = np.nan
+        if priors is None:
+            priors = self.default_priors(population_var=True)
+        return LaplaceSample(trace, lp, p, q, r, kind=kind, priors=priors, stats=self.curve_stats(), multi_series=self)
 
 
 def hessian_steps(theta, rel_step=HESS_REL_STEP):

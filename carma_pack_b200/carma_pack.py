@@ -328,6 +328,32 @@ class CarmaModel(object):
             ms.close()
         return OptimizeResult({k: (v[0].item() if v.ndim == 1 else v[0]) for k, v in res.items()})
 
+    def laplace_sample(self, theta, p=None, q=None, cov=None, ndraws=1000, seed=None):
+        """The posterior by importance sampling from the Laplace approximation at theta (e.g. get_mle(...).x):
+        MultiSeries.laplace_sample on this curve alone (curve_offset 0), so it equals a one-curve survey call bit for bit.
+        cov None: the covariance of self.hessian(theta).  Returns a CarmaSample (Car1Sample for p = 1) of the resampled
+        draws, carrying khat, ess and status (k-hat above 0.7: the Gaussian proposal misses the posterior; run_mcmc)."""
+        p = self.p if p is None else p
+        q = self.q if q is None else q
+        if seed is None:
+            seed = int(np.random.SeedSequence().generate_state(1, dtype=np.uint64)[0] >> 1)
+        th = np.asarray(theta, dtype=np.float64)[None, :]
+        cv = None if cov is None else np.asarray(cov, dtype=np.float64)[None, :, :]
+        ms = _lib.MultiSeries(self.time, self.y, self.ysig, [0, self.time.size], device=self.device)
+        try:
+            ls = ms.laplace_sample(p, q, th, cov=cv, ndraws=ndraws, seed=seed)
+        finally:
+            ms.close()
+        prior = self.series.default_prior(population_var=True)
+        if p == 1:
+            sample = Car1Sample(self.time, self.y, self.ysig, trace=ls.trace[0], logpost=ls.logpost[0], series=self.series,
+                                prior=prior)
+        else:
+            sample = CarmaSample(self.time, self.y, self.ysig, trace=ls.trace[0], logpost=ls.logpost[0], p=p, q=q,
+                                 series=self.series, prior=prior)
+        sample.khat, sample.ess, sample.status = float(ls.khat[0]), float(ls.ess[0]), int(ls.status[0])
+        return sample
+
     @staticmethod
     def _mle_result(x, f, nit, nfev):
         best = int(np.argmin(f))
@@ -649,6 +675,24 @@ class SurveySample(object):
             return Car1Sample(t, y, e, trace=self.trace[c], logpost=self.logpost[c], prior=self._prior_struct(c))
         return CarmaSample(t, y, e, trace=self.trace[c], logpost=self.logpost[c], p=self.p, q=self.q,
                            prior=self._prior_struct(c))
+
+
+class LaplaceSample(SurveySample):
+    """The posterior samples of every curve of a survey by importance sampling from its Laplace approximation
+    (MultiSeries.laplace_sample): trace (ncurves, ndraws, d) the equally weighted resample of the draws, logpost their
+    log-posteriors; NaN rows for a curve whose status is not LAPLACE_OK.  khat (ncurves,): the Pareto k-hat of the
+    weights, the reliability of the sample (<= 0.7: use it; above: run MCMC on that curve); ess (ncurves,) the weight
+    ESS; status (ncurves,); laplace: the raw MultiSeries.laplace result (draws, weights, resample indices)."""
+
+    def __init__(self, trace, logpost, p, q, laplace, kind=None, priors=None, stats=None, multi_series=None):
+        super(LaplaceSample, self).__init__(trace, logpost, p, q, kind=kind, priors=priors, stats=stats,
+                                            multi_series=multi_series)
+        self.laplace = laplace
+        self.khat, self.ess, self.status = laplace.khat, laplace.ess, laplace.status
+
+    def effective_samples(self, name):
+        raise ValueError("the draws of a LaplaceSample are resampled, not a chain: autocorrelation ESS means nothing "
+                         "for them; .ess holds each curve's weight ESS")
 
 
 class MCMCSample(object):

@@ -13,7 +13,10 @@
 //                              then the adjoint (Bryson-Frazier) recursion backward: smoothed values, leave-one-out laws
 //                              and queries in O(ny + nq) steps;
 //   multi_hessian_eval_kernel<P>  one thread = one (curve, stencil point): K4's body on a finite-difference row;
-//   multi_hessian_assemble_kernel one thread = one curve: gradient, Hessian and covariance from its stencil values.
+//   multi_hessian_assemble_kernel one thread = one curve: gradient, Hessian and covariance from its stencil values;
+//   multi_laplace_factor_kernel   one thread = one curve: Cholesky factor of its proposal covariance (laplace.cuh);
+//   multi_laplace_eval_kernel<P>  one thread = one (curve, draw): the proposal draw, then K4's body on it;
+//   multi_laplace_summary_kernel  one block = one curve: weight ESS, Pareto k-hat and systematic resampling.
 #include <algorithm>
 #include <cmath>
 #include <cstdlib>
@@ -24,6 +27,8 @@
 
 #include "hessian.cuh"
 #include "kalman_real.cuh"
+#include "laplace.cuh"
+#include "select.cuh"
 #include "series.h"
 
 namespace carma {
@@ -506,6 +511,251 @@ multi_hessian_assemble_kernel(const double* __restrict__ fval, size_t c0, size_t
     status[c] = hess_assemble(d, f, h, grad + c * d, hess + c * d * d, cov + c * d * d);
 }
 
+// Laplace importance sampling, factor: one thread per curve of the chunk; L (d x d), log|L| and the CARMA_LAPLACE_OK /
+// BAD_COV status at the curve's chunk index.
+__global__ void __launch_bounds__(SF_BLOCK)
+multi_laplace_factor_kernel(const double* __restrict__ theta, const double* __restrict__ cov, size_t c0, size_t nc,
+                            int d, double* __restrict__ L, double* __restrict__ logdet, int* __restrict__ fstat) {
+    const size_t cl = (size_t)blockIdx.x * SF_BLOCK + threadIdx.x;
+    if (cl >= nc) return;
+    const size_t c = c0 + cl;
+    fstat[cl] = lap_cholesky(d, theta + c * d, cov + c * d * d, L + cl * d * d, logdet + cl);
+}
+
+// Laplace importance sampling, evaluation: one thread per (curve, draw) of the chunk, draw-minor (thread u: chunk curve
+// u / S, draw u % S), so the lanes of a warp walk the same curve with broadcast loads, as multi_hessian_eval_kernel.
+// The draw (Philox pairs, Box-Muller, the row theta + L z with every product and sum rounded on its own) and its
+// proposal log-density, then multi_loglik_kernel's body (same transform and rate clamp, block loads, slow fallback,
+// log-prior), so logpost[u] is what carma_multi_loglik returns for the row.  A BAD_COV curve gets NaN rows.
+template <int P>
+__global__ void __launch_bounds__(SF_BLOCK, P <= 3 ? 8 : 1)   // K4's bounds
+multi_laplace_eval_kernel(const double* __restrict__ dt, const double* __restrict__ y, const double* __restrict__ e2,
+                          const long long* __restrict__ off, size_t c0, size_t nc, size_t S, double dt_max, int kind,
+                          int q, int d, unsigned flags, const carma_prior_t* __restrict__ priors,
+                          const double* __restrict__ theta, const double* __restrict__ L,
+                          const double* __restrict__ logdet, const int* __restrict__ fstat, unsigned long long seed,
+                          uint32_t curve_offset, double* __restrict__ draws, double* __restrict__ logpost,
+                          double* __restrict__ logq) {
+    MathTab tb;
+    tb.load();
+    const size_t u = (size_t)blockIdx.x * SF_BLOCK + threadIdx.x;
+    if (u >= nc * S) return;
+    const size_t cl = u / S;
+    const uint32_t j = (uint32_t)(u - cl * S);
+    const size_t c = c0 + cl;
+    double* out = draws + u * d;
+    if (fstat[cl] != CARMA_LAPLACE_OK) {
+        for (int i = 0; i < d; i++) out[i] = NAN;
+        logpost[u] = NAN;
+        logq[u] = NAN;
+        return;
+    }
+    const uint32_t block = curve_offset + (uint32_t)c;
+    double z[MAX_D + 1];
+    double zz = 0.0;
+#pragma unroll
+    for (int k = 0; k < MAX_D; k += 2) {
+        z[k] = z[k + 1] = 0.0;
+        if (k < d) {
+            double u0, u1, sn, cs;
+            uniforms2(seed, j, STREAM_LAPLACE, (uint32_t)(k / 2), block, &u0, &u1);
+            const double r = sqrt(-2.0 * log(u0));
+            sincos(6.283185307179586476925286766559 * u1, &sn, &cs);
+            z[k] = __dmul_rn(r, cs);
+            z[k + 1] = __dmul_rn(r, sn);
+            zz = __dadd_rn(zz, __dmul_rn(z[k], z[k]));
+            if (k + 1 < d) zz = __dadd_rn(zz, __dmul_rn(z[k + 1], z[k + 1]));
+        }
+    }
+    logq[u] = -0.5 * zz - logdet[cl] - 0.5 * d * LAP_LOG_2PI;
+    const double* Lc = L + cl * d * d;
+    const double* row = theta + c * (size_t)d;
+    double th[MAX_D];
+#pragma unroll
+    for (int i = 0; i < MAX_D; i++) {
+        th[i] = 0.0;
+        if (i < d) {
+            double s = 0.0;
+#pragma unroll
+            for (int k = 0; k <= i; k++) s = __dadd_rn(s, __dmul_rn(Lc[i * d + k], z[k]));
+            th[i] = __dadd_rn(row[i], s);
+            out[i] = th[i];
+        }
+    }
+    RealParams<P> prm;
+    carma_prior_t pr = priors[c];
+    if (transform_theta<P>(kind, q, flags, pr, th, dt_max, prm) != TT_OK) {
+        logpost[u] = -INFINITY;
+        return;
+    }
+    const long long o0 = off[c], o1 = off[c + 1];   // read here rather than first: P = 5 then spills half as much
+    const int ny = (int)(o1 - o0);
+    KalmanReal<P> kf;
+    LogLikAcc acc;
+    kf.reset(prm, e2[o0]);
+    acc.init();
+    const SeriesPtr src{dt + o0, y + o0, e2 + o0 + 1};
+    filter_span_blocks_any<P>(kf, acc, prm, tb, dt + o0, y + o0, e2 + o0, ny);
+    logpost[u] = (acc.bad() ? loglik_exact_slow<P>(prm, tb, src, ny, e2[o0]) : acc.value()) + prm.logprior;
+}
+
+// Fixed-order block reductions of LAP_THREADS threads (xor butterflies, then warp 0 over the warp partials): the same
+// inputs give the same bits on every run.
+constexpr int LAP_THREADS = 256;
+constexpr int LAP_TAIL_MAX = 4096;   // >= psis_tail_len(CARMA_LAPLACE_MAX_DRAWS) = 3072; a power of two for the sort
+static_assert(3 * 1024 <= LAP_TAIL_MAX, "the Pareto tail must fit the shared sort");
+
+template <bool MAX>
+__device__ __forceinline__ double lap_block_reduce(double v, double* sh) {
+#pragma unroll
+    for (int k = 16; k >= 1; k >>= 1) {
+        const double o = __shfl_xor_sync(0xffffffffu, v, k);
+        v = MAX ? fmax(v, o) : v + o;
+    }
+    const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    __syncthreads();   // sh is free
+    if (lane == 0) sh[w] = v;
+    __syncthreads();
+    if (w == 0) {
+        v = lane < LAP_THREADS / 32 ? sh[lane] : (MAX ? -INFINITY : 0.0);
+#pragma unroll
+        for (int k = 16; k >= 1; k >>= 1) {
+            const double o = __shfl_xor_sync(0xffffffffu, v, k);
+            v = MAX ? fmax(v, o) : v + o;
+        }
+        if (lane == 0) sh[LAP_THREADS / 32] = v;
+    }
+    __syncthreads();
+    return sh[LAP_THREADS / 32];
+}
+
+// Laplace importance sampling, summary: one block per curve of the chunk.  W (S doubles per curve) holds the log
+// weights lw, then exp(lw - max), then their running sums.  The cut a_(S-M-1) comes from the radix select of select.cuh
+// on lw (a = lw - max is monotone in lw), the tail (at most M <= 3072 values) is sorted in shared memory, and the
+// generalised-Pareto fit spreads its trial b_i over the warps.  Outputs at the curve's chunk index.
+__global__ void __launch_bounds__(LAP_THREADS)
+multi_laplace_summary_kernel(size_t c0, size_t S, const int* __restrict__ fstat, const double* __restrict__ logpost,
+                             const double* __restrict__ logq, double* __restrict__ W, unsigned long long seed,
+                             uint32_t curve_offset, int32_t* __restrict__ resample, double* __restrict__ ess,
+                             double* __restrict__ khat, int* __restrict__ status) {
+    __shared__ double tail[LAP_TAIL_MAX];
+    __shared__ double red[LAP_THREADS / 32 + 1];
+    __shared__ double gb[128], gl[128], gw[128];
+    __shared__ SelectSmem sm;
+    __shared__ unsigned ntail;
+    const size_t cl = blockIdx.x;
+    const int tid = threadIdx.x;
+    const double* lp = logpost + cl * S;
+    const double* lq = logq + cl * S;
+    double* w = W + cl * S;
+    int32_t* rs = resample + cl * S;
+    auto reject = [&](int st) {
+        for (size_t i = tid; i < S; i += LAP_THREADS) rs[i] = -1;
+        if (tid == 0) { ess[cl] = 0.0; khat[cl] = NAN; status[cl] = st; }
+    };
+    if (fstat[cl] != CARMA_LAPLACE_OK) { reject(CARMA_LAPLACE_BAD_COV); return; }
+    double mx = -INFINITY;
+    for (size_t i = tid; i < S; i += LAP_THREADS) {
+        const double a = lp[i];
+        const double v = isfinite(a) ? a - lq[i] : -INFINITY;
+        w[i] = v;
+        mx = fmax(mx, v);
+    }
+    mx = lap_block_reduce<true>(mx, red);
+    if (mx == -INFINITY) { reject(CARMA_LAPLACE_NO_WEIGHT); return; }
+    // weight ESS
+    double s1 = 0.0, s2 = 0.0;
+    for (size_t i = tid; i < S; i += LAP_THREADS) {
+        const double e = exp(w[i] - mx);
+        s1 += e;
+        s2 += e * e;
+    }
+    s1 = lap_block_reduce<false>(s1, red);
+    s2 = lap_block_reduce<false>(s2, red);
+    // k-hat
+    double kh = INFINITY;
+    if (S >= 2) {
+        const size_t M = psis_tail_len(S);
+        unsigned long long ka, kb;
+        block_select_pair(w, S, S - M - 1, sm, &ka, &kb);
+        const double cut = fmax(key_value(ka) - mx, LAP_LOG_DBL_MIN), ecut = exp(cut);
+        if (tid == 0) ntail = 0;
+        __syncthreads();
+        for (size_t i = tid; i < S; i += LAP_THREADS) {
+            const double a = w[i] - mx;
+            if (a > cut) {
+                const unsigned k = atomicAdd(&ntail, 1u);
+                if (k < LAP_TAIL_MAX) tail[k] = exp(a) - ecut;
+            }
+        }
+        __syncthreads();
+        const int n = (int)min(ntail, (unsigned)LAP_TAIL_MAX);
+        if (n > 4) {
+            int n2 = 1;
+            while (n2 < n) n2 <<= 1;
+            for (int i = n + tid; i < n2; i += LAP_THREADS) tail[i] = INFINITY;
+            __syncthreads();
+            for (int k = 2; k <= n2; k <<= 1)   // bitonic sort, ascending
+                for (int jj = k >> 1; jj > 0; jj >>= 1) {
+                    for (int i = tid; i < n2; i += LAP_THREADS) {
+                        const int l = i ^ jj;
+                        if (l > i) {
+                            const double a = tail[i], b = tail[l];
+                            if (((i & k) == 0) == (a > b)) { tail[i] = b; tail[l] = a; }
+                        }
+                    }
+                    __syncthreads();
+                }
+            const int m = gpd_m(n), wp = tid >> 5, lane = tid & 31;
+            for (int i = wp; i < m; i += LAP_THREADS / 32) {   // warp wp: trial b_(i+1)
+                const double b = gpd_b(i + 1, m, tail, n);
+                double s = 0.0;
+                for (int t = lane; t < n; t += 32) s += log1p(-b * tail[t]);
+#pragma unroll
+                for (int k = 16; k >= 1; k >>= 1) s += __shfl_xor_sync(0xffffffffu, s, k);
+                if (lane == 0) { gb[i] = b; gl[i] = gpd_profile(n, b, s / n); }
+            }
+            __syncthreads();
+            for (int i = tid; i < m; i += LAP_THREADS) gw[i] = gpd_weight(i, m, gl);
+            __syncthreads();
+            const double bbar = gpd_bbar(m, gb, gw);   // every thread, same order
+            double s = 0.0;
+            for (int t = tid; t < n; t += LAP_THREADS) s += log1p(-bbar * tail[t]);
+            s = lap_block_reduce<false>(s, red);
+            kh = gpd_khat(n, s / n);
+        }
+    }
+    // systematic resampling: running sums of e over contiguous per-thread ranges, then the ranges' offsets in order
+    const size_t per = (S + LAP_THREADS - 1) / LAP_THREADS, i0 = min(S, tid * per), i1 = min(S, i0 + per);
+    double part = 0.0;
+    for (size_t i = i0; i < i1; i++) {
+        const double e = exp(w[i] - mx);
+        w[i] = e;
+        part += e;
+    }
+    __syncthreads();
+    tail[tid] = part;   // the tail is no longer needed
+    __syncthreads();
+    if (tid == 0)
+        for (int t = 1; t < LAP_THREADS; t++) tail[t] += tail[t - 1];
+    __syncthreads();
+    double run = tid == 0 ? 0.0 : tail[tid - 1];
+    for (size_t i = i0; i < i1; i++) {
+        run += w[i];
+        w[i] = run;
+    }
+    __syncthreads();
+    const double T = w[S - 1];
+    double u0, u1;
+    uniforms2(seed, 0u, STREAM_LAPLACE_RESAMPLE, 0u, curve_offset + (uint32_t)(c0 + cl), &u0, &u1);
+    for (size_t i = tid; i < S; i += LAP_THREADS) rs[i] = (int32_t)resample_find(w, S, resample_target(i, u0, S, T));
+    if (tid == 0) {
+        ess[cl] = s1 * s1 / s2;
+        khat[cl] = kh;
+        status[cl] = CARMA_LAPLACE_OK;
+    }
+}
+
 // ---- launchers ---------------------------------------------------------------------------------------------------
 static bool alike32(const void* a, const void* b) { return (((size_t)a ^ (size_t)b) & 31u) == 0; }
 
@@ -633,6 +883,24 @@ static cudaError_t launch_hessian_eval_p(const carma_multi_series* m, int kind, 
     const int d = model_dim(kind, P, q), npts = hess_points(d);
     multi_hessian_eval_kernel<P><<<(unsigned)((nc * npts + SF_BLOCK - 1) / SF_BLOCK), SF_BLOCK, 0, st>>>(
         m->d_dt, m->d_y, m->d_e2, m->d_off, c0, nc, npts, m->dt_max, kind, q, d, flags, d_priors, d_theta, rel_step, d_f);
+    return cudaGetLastError();
+}
+
+// one chunk of carma_multi_laplace's draws: curves c0 .. c0 + nc - 1, S draws each
+struct LaplaceChunk {
+    double *L, *logdet, *w, *draws, *logpost, *logq, *ess, *khat;
+    int *fstat, *status;
+    int32_t* resample;
+};
+
+template <int P>
+static cudaError_t launch_laplace_eval_p(const carma_multi_series* m, int kind, int q, unsigned flags,
+                                         const carma_prior_t* d_priors, const double* d_theta, size_t c0, size_t nc,
+                                         size_t S, unsigned long long seed, uint32_t curve_offset, const LaplaceChunk& ch,
+                                         cudaStream_t st) {
+    multi_laplace_eval_kernel<P><<<(unsigned)((nc * S + SF_BLOCK - 1) / SF_BLOCK), SF_BLOCK, 0, st>>>(
+        m->d_dt, m->d_y, m->d_e2, m->d_off, c0, nc, S, m->dt_max, kind, q, model_dim(kind, P, q), flags, d_priors,
+        d_theta, ch.L, ch.logdet, ch.fstat, seed, curve_offset, ch.draws, ch.logpost, ch.logq);
     return cudaGetLastError();
 }
 
@@ -1030,6 +1298,93 @@ int carma_multi_hessian(carma_multi_series_t m, int kind, int p, int q, const ca
     for (const Out& o : outs)
         if (o.host && !cuda_ok(cudaMemcpyAsync(o.host, o.dev, o.bytes, cudaMemcpyDeviceToHost, st), o.what)) return CARMA_ERR_CUDA;
     if (!cuda_ok(cudaStreamSynchronize(st), "multi_hessian sync")) return CARMA_ERR_CUDA;
+    return CARMA_OK;
+}
+
+int carma_multi_laplace(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* priors, const double* theta,
+                        const double* cov, unsigned flags, size_t ndraws, uint64_t seed, uint32_t curve_offset,
+                        double* draws, double* logpost, double* logq, int32_t* resample, double* ess, double* khat,
+                        int* status) {
+    if (!m || !theta || !cov) { set_error("carma_multi_laplace: null argument"); return CARMA_ERR_ARG; }
+    if (!valid_model(kind, p, q)) { set_error("carma_multi_laplace: invalid (kind,p,q)"); return CARMA_ERR_ARG; }
+    if (ndraws == 0 || ndraws > CARMA_LAPLACE_MAX_DRAWS) {
+        set_error("carma_multi_laplace: ndraws must be in 1 .. CARMA_LAPLACE_MAX_DRAWS (2^20)");
+        return CARMA_ERR_ARG;
+    }
+    if ((unsigned long long)curve_offset + m->ncurves > (1ull << 32)) {
+        set_error("carma_multi_laplace: curve_offset + ncurves exceeds 2^32");
+        return CARMA_ERR_ARG;
+    }
+    if (!alike32(m->d_dt, m->d_y) || !alike32(m->d_dt, m->d_e2)) { set_error("carma_multi_laplace: curve arrays not sector-aligned"); return CARMA_ERR_ARG; }
+    const size_t nc = m->ncurves, d = (size_t)model_dim(kind, p, q), S = ndraws;
+    if (!cuda_ok(cudaSetDevice(m->device), "cudaSetDevice")) return CARMA_ERR_CUDA;
+    cudaStream_t st = 0;
+    int rc = upload_rows(m, kind, p, q, priors, theta, nc, st);
+    if (rc) return rc;
+    if (!m->scratch_pts.reserve(nc * d * d * sizeof(double)) ||
+        !cuda_ok(cudaMemcpyAsync(m->scratch_pts.p, cov, nc * d * d * sizeof(double), cudaMemcpyHostToDevice, st), "H2D cov"))
+        return CARMA_ERR_CUDA;
+    // Curves go in chunks of B whose scratch fits the budget (CARMA_MULTI_LAPLACE_BUDGET bytes, read at every call so
+    // that a test can force several chunks), and whose threads fit one grid.  Every output depends only on its curve, so
+    // chunking changes no bit.
+    size_t budget = (size_t)4 << 30;
+    if (const char* env = getenv("CARMA_MULTI_LAPLACE_BUDGET")) budget = (size_t)std::strtoull(env, nullptr, 10);
+    const size_t per_curve = 8 * S * (d + 3) + 4 * S + 8 * d * d + 32;
+    const size_t B = std::max<size_t>(1, std::min(std::min(nc, budget / per_curve), ((size_t)1 << 36) / S));
+    // scratch_misc: L | logdet | ess | khat | w | draws | logpost | logq | fstat | status | resample
+    const size_t b_L = round32(B * d * d), b_1 = round32(B), b_S = round32(B * S), b_i = round32((B + 1) / 2);
+    const size_t b_D = round32(B * S * d), b_r = round32((B * S + 1) / 2);
+    if (!m->scratch_misc.reserve((b_L + 3 * b_1 + 3 * b_S + b_D + 2 * b_i + b_r) * sizeof(double))) return CARMA_ERR_CUDA;
+    LaplaceChunk ch;
+    ch.L = (double*)m->scratch_misc.p;
+    ch.logdet = ch.L + b_L;
+    ch.ess = ch.logdet + b_1;
+    ch.khat = ch.ess + b_1;
+    ch.w = ch.khat + b_1;
+    ch.draws = ch.w + b_S;
+    ch.logpost = ch.draws + b_D;
+    ch.logq = ch.logpost + b_S;
+    ch.fstat = (int*)(ch.logq + b_S);
+    ch.status = (int*)((double*)ch.fstat + b_i);
+    ch.resample = (int32_t*)((double*)ch.status + b_i);
+    const carma_prior_t* d_pr = (const carma_prior_t*)m->scratch_pr.p;
+    const double* d_th = (const double*)m->scratch_in.p;
+    const double* d_cov = (const double*)m->scratch_pts.p;
+    for (size_t c0 = 0; c0 < nc; c0 += B) {
+        const size_t n = std::min(B, nc - c0);
+        multi_laplace_factor_kernel<<<(unsigned)((n + SF_BLOCK - 1) / SF_BLOCK), SF_BLOCK, 0, st>>>(
+            d_th, d_cov, c0, n, (int)d, ch.L, ch.logdet, ch.fstat);
+        if (!cuda_ok(cudaGetLastError(), "multi_laplace_factor_kernel launch")) return CARMA_ERR_CUDA;
+        cudaError_t e;
+#define LAUNCH_LE(PP) e = launch_laplace_eval_p<PP>(m, kind, q, flags, d_pr, d_th, c0, n, S, seed, curve_offset, ch, st)
+        switch (p) {
+            case 1: LAUNCH_LE(1); break;
+            case 2: LAUNCH_LE(2); break;
+            case 3: LAUNCH_LE(3); break;
+            case 4: LAUNCH_LE(4); break;
+            case 5: LAUNCH_LE(5); break;
+            case 6: LAUNCH_LE(6); break;
+            default: LAUNCH_LE(7); break;
+        }
+#undef LAUNCH_LE
+        if (!cuda_ok(e, "multi_laplace_eval_kernel launch")) return CARMA_ERR_CUDA;
+        multi_laplace_summary_kernel<<<(unsigned)n, LAP_THREADS, 0, st>>>(
+            c0, S, ch.fstat, ch.logpost, ch.logq, ch.w, seed, curve_offset, ch.resample, ch.ess, ch.khat, ch.status);
+        if (!cuda_ok(cudaGetLastError(), "multi_laplace_summary_kernel launch")) return CARMA_ERR_CUDA;
+        struct Out { void* host; const void* dev; size_t bytes; const char* what; };
+        const Out outs[7] = {
+            {draws ? draws + c0 * S * d : nullptr, ch.draws, n * S * d * sizeof(double), "D2H draws"},
+            {logpost ? logpost + c0 * S : nullptr, ch.logpost, n * S * sizeof(double), "D2H logpost"},
+            {logq ? logq + c0 * S : nullptr, ch.logq, n * S * sizeof(double), "D2H logq"},
+            {resample ? resample + c0 * S : nullptr, ch.resample, n * S * sizeof(int32_t), "D2H resample"},
+            {ess ? ess + c0 : nullptr, ch.ess, n * sizeof(double), "D2H ess"},
+            {khat ? khat + c0 : nullptr, ch.khat, n * sizeof(double), "D2H khat"},
+            {status ? status + c0 : nullptr, ch.status, n * sizeof(int), "D2H status"}};
+        for (const Out& o : outs)
+            if (o.host && !cuda_ok(cudaMemcpyAsync(o.host, o.dev, o.bytes, cudaMemcpyDeviceToHost, st), o.what)) return CARMA_ERR_CUDA;
+        // the next chunk reuses the scratch: its outputs must have left
+        if (!cuda_ok(cudaStreamSynchronize(st), "multi_laplace sync")) return CARMA_ERR_CUDA;
+    }
     return CARMA_OK;
 }
 

@@ -349,6 +349,55 @@ enum {
 int carma_multi_hessian(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* priors,
                         const double* theta /* ncurves x d */, unsigned flags, double rel_step, double* loglik,
                         double* grad, double* hess, double* cov, int* status);
+/* Importance sampling of every curve's posterior from its Laplace approximation N(theta_c, cov_c) (an extension: the
+ * reference has only MCMC), with the Pareto k-hat reliability diagnostic and an equally weighted resample, so that a
+ * survey can keep the Gaussian answer where it is good and run MCMC only where k-hat says it is not.  S = ndraws.
+ *   Factor: the lower Cholesky factor L of cov_c, reading only its lower triangle (the upper one is never read), in
+ *   the fixed loop order s = cov_jj - sum_{k<j} L_jk^2, L_jj = sqrt(s), L_ij = (cov_ij - sum_{k<j} L_ik L_jk) / L_jj
+ *   (i > j, sums left to right, every product and difference rounded on its own); log|L| = sum_i log L_ii.
+ *   Draw j: coordinate pair k takes (u0, u1) = uniforms2(seed, j, STREAM_LAPLACE = 6, k, curve_offset + c) (Philox
+ *   counters laid out as carma_multi_simulate's (path, point, curve)); r = sqrt(-2 log u0), z_2k = r cos(2 pi u1),
+ *   z_2k+1 = r sin(2 pi u1) (the second is dropped when d is odd).  Row: s_i = sum_{k<=i} L_ik z_k accumulated left to
+ *   right from 0, theta_i = theta_c,i + s_i, each product and sum rounded on its own (no contraction).
+ *   logq = -1/2 sum_k z_k^2 - log|L| - (d/2) log(2 pi), the proposal's log-density of the row.
+ *   logpost is bitwise what carma_multi_loglik returns for the row with the same kind, p, q, priors (NULL: defaults)
+ *   and flags, log-prior included.
+ *   Weights: lw_j = logpost_j - logq_j where logpost_j is finite, else -inf; a_j = lw_j - max_j lw_j, e_j = exp(a_j).
+ *   ess = (sum e)^2 / sum e^2, the weight ESS of the raw weights.
+ *   khat, the generalised-Pareto shape of the largest weights (Vehtari et al., PSIS; ArviZ _psislw / _gpdfit, r_eff = 1):
+ *     M = ceil(min(0.2 S, 3 sqrt(S))); cut = max(a_(S-M-1), log DBL_MIN), a_(.) ascending and 0-based (S < 2: +inf);
+ *     the tail is {a_j > cut}, n members; n <= 4: khat = +inf;
+ *     else x = ascending(exp(a_j) - exp(cut)) over the tail, m = 30 + floor(sqrt(n)), and for i = 1 .. m
+ *       b_i = (1 - sqrt(m / (i - 1/2))) / (3 x[floor(n/4 + 1/2) - 1]) + 1 / x[n-1],
+ *       k_i = mean_t log1p(-b_i x_t),  L_i = n (log(-b_i / k_i) - k_i - 1),  w_i = 1 / sum_l exp(L_l - L_i);
+ *     the w_i < 10 DBL_EPSILON are dropped and the rest renormalised; bbar = sum_i w_i b_i, k = mean_t log1p(-bbar x_t);
+ *     khat = (n k + 5) / (n + 10).  khat <= 0.7: the importance sample is reliable; above, it is not (run MCMC).
+ *   resample (systematic, from the raw weights): u = the first uniform of uniforms2(seed, 0, STREAM_LAPLACE_RESAMPLE =
+ *   7, 0, curve_offset + c), C_j = e_0 + ... + e_j, T = C_{S-1}; resample[c, i] = the first j with C_j > ((i + u) / S) T,
+ *   capped at S - 1: draws[c, resample[c, i]] is an equally weighted sample of the posterior.
+ * Every reduction runs in a fixed order, so every output is deterministic.  A draw depends only on (seed, j,
+ * curve_offset + c, theta_c, cov_c): batch mates, ndraws (a call with fewer draws gives a prefix of draws / logpost /
+ * logq), chunking and curve subsets with a matching curve_offset change no bit.
+ * Outputs (any may be NULL): draws (ncurves x ndraws x d), logpost, logq, resample (ncurves x ndraws), ess, khat,
+ * status (ncurves) one of CARMA_LAPLACE_*, each curve's independent of the others':
+ *   OK         every output valid;
+ *   BAD_COV    theta_c or the lower triangle of cov_c is not finite, or the factorisation fails (s <= 0): draws,
+ *              logpost, logq and khat NaN, ess 0, resample -1;
+ *   NO_WEIGHT  no draw has a finite logpost (e.g. the proposal lies outside the prior): draws and logq valid, logpost
+ *              as evaluated, ess 0, khat NaN, resample -1.
+ * CARMA_ERR_ARG before any CUDA call: m, theta or cov NULL, an invalid (kind, p, q), ndraws 0 or above
+ * CARMA_LAPLACE_MAX_DRAWS, curve_offset + ncurves > 2^32.  Blocking; uses the multi-series' scratch (one call per handle
+ * at a time).  Curves run in chunks whose scratch, 8 S (d + 3) + 4 S + 8 d^2 + 32 bytes per curve, stays within 4 GiB
+ * (CARMA_MULTI_LAPLACE_BUDGET bytes, read at every call); theta, cov and the priors of all curves take 8 ncurves
+ * (d^2 + d) bytes and the priors more. */
+#define CARMA_LAPLACE_MAX_DRAWS (1u << 20)
+enum { CARMA_LAPLACE_OK = 0, CARMA_LAPLACE_BAD_COV = 1, CARMA_LAPLACE_NO_WEIGHT = 2 };
+int carma_multi_laplace(carma_multi_series_t m, int kind, int p, int q, const carma_prior_t* priors /* NULL: defaults */,
+                        const double* theta /* ncurves x d: centres */, const double* cov /* ncurves x d x d */,
+                        unsigned flags, size_t ndraws, uint64_t seed, uint32_t curve_offset,
+                        double* draws /* ncurves x ndraws x d */, double* logpost /* ncurves x ndraws */,
+                        double* logq /* ncurves x ndraws */, int32_t* resample /* ncurves x ndraws */,
+                        double* ess /* ncurves */, double* khat /* ncurves */, int* status /* ncurves */);
 
 /* ---- one very long light curve: temporally parallel (associative-scan) form of the same LogDensity ----
  * Replaces the strictly sequential Filter() loop (src/include/kfilter.hpp:126-132) when there is a single
